@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- PDHG iterations/s on ROF-TV 4096^2 (BASELINE.json metric) with roofline evidence.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one PDHG iteration (BackendPDHG::PerformIteration, backend_pdhg.cu:311-381) on the
 metric config of SURVEY.md section 8(d): ROF 4096 x 4096 gray, BlockGradient2D + 1d:square +
@@ -342,6 +342,43 @@ def iterate_hash(env, be, part, n_planes_x, n_planes_y):
     return {"x": f"{hx:016x}", "y": f"{hy:016x}"}
 
 
+DUMP_SAMPLE = 1 << 21       # positions drawn per array: at most 4 arrays x 8 MB of float32
+
+
+def dump_outputs(env, be, part, out_dir):
+    """x, z, y, w as the backend returns them to a caller after the timed iterations, written by rank 0 as
+    out_dir/<name>.npy (float32).  Each array is sampled at the same sorted positions on every run (seed 0), a
+    position being plane * NX * NY + column * NY + row of the whole image, so that dumps of two builds, or of runs
+    on different numbers of GPUs, can be compared element for element."""
+    import numpy as np
+    x, z, y, w = be.current_solution()
+    rng = np.random.default_rng(0)
+    where = {}                           # sampled positions: plane, column, row
+    vals = {}                            # this rank's values at the positions in its columns, in position order
+    for name, arr, planes in (("x", x, 1), ("z", z, 2), ("y", y, 2), ("w", w, 1)):
+        pos = np.unique(rng.integers(0, planes * NX * NY, DUMP_SAMPLE))
+        where[name] = (pos // (NX * NY), pos % (NX * NY) // NY, pos % NY)
+        p, c, r = where[name]
+        x0, x1 = part.range(env.rank)
+        mine = (c >= x0) & (c < x1)
+        vals[name] = arr[p[mine] * ((x1 - x0) * NY) + (c[mine] - x0) * NY + r[mine]]
+    if env.world > 1:
+        parts = [None] * env.world
+        env.dist.all_gather_object(parts, vals)
+    else:
+        parts = [vals]
+    if env.rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    for name in ("x", "z", "y", "w"):
+        _, c, _ = where[name]
+        out = np.full(c.size, np.nan, dtype=np.float32)
+        for rank, rank_vals in enumerate(parts):
+            x0, x1 = part.range(rank)
+            out[(c >= x0) & (c < x1)] = rank_vals[name]
+        np.save(os.path.join(out_dir, f"{name}.npy"), out)
+
+
 def aux_workload(env, name, steps, warmup):
     """BASELINE configs 2-4 at full size on the same GPUs: iterations/s (device-timed, max over ranks) and the
     fraction of the HBM roofline on the algorithmic bytes of SURVEY.md 8(d)."""
@@ -481,6 +518,8 @@ def run_ours(args):
     value = args.steps / (ms * 1e-3)
     # slab parity carried by the run itself: checksum of the iterates after W + K iterations
     hashes = iterate_hash(env, be, part, 1, 2)
+    if args.dump_outputs:
+        dump_outputs(env, be, part, args.dump_outputs)
 
     # ---------------- per-kernel timing for the roofline --------------------------------------------
     # CUDA events around every launch, recorded back to back and read after ONE synchronisation at the end
@@ -634,11 +673,15 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-workloads", action="store_true", help="skip BASELINE configs 2-4")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write a fixed sample of x, z, y, w to DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs needs --impl ours")
         run_reference_arm(args, rank, world)
         return
     run_ours(args)
