@@ -106,7 +106,7 @@ class Backend {
   virtual bool is_fused() const { return false; }
   virtual unsigned long long one_pass_iterations() const { return 0; }
   virtual void device_iterates(float** d_x, float** d_y) = 0;
-  // iterations between two residual refreshes (for the solver loop's chunking)
+  // iterations between two residual refreshes
   virtual int residual_iter() const = 0;
   // does the iteration that starts with iteration() == it_before refresh the residuals?  PDHG checks
   // before iteration_++ (backend_pdhg.cu:389, size_t % int), ADMM after it (backend_admm.cu:525-529).
@@ -114,9 +114,6 @@ class Backend {
     const unsigned long long mod = static_cast<unsigned long long>(static_cast<long long>(residual_iter()));
     return it_before == 0 || (it_before % mod) == 0;
   }
-  // may iterate(n) put several iterations into one launch?  (the solver loop then enqueues whole stretches
-  // between two observable events with one call)
-  virtual bool batches_iterations() const { return false; }
   // slab decomposition (pb_comm.cuh); must be called before initialize()
   virtual void set_slab(class Comm*) { fail(PB_ERR_UNSUPPORTED, "this backend has no slab decomposition"); }
 

@@ -53,9 +53,6 @@ struct Context {
   // kernels return without touching memory.  Lets a device-resident loop (the CGLS projection of
   // BackendADMM, pb_admm.cu) stop early without a host round trip per inner iteration.
   const int* skip_flag = nullptr;
-  // > 0: CTAs per SM for the identity-row dual pass (stencil_dual_identity_launch) while it runs beside the
-  // gradient-row pass on a second stream (BackendPDHG, pb_pdhg.cu); 0: the kernel takes the whole GPU
-  int identity_ctas_per_sm = 0;
   // two pinned staging buffers for copies to / from pageable host memory (pb_hostio.cu), allocated on
   // first use and released by pb_context_destroy
   void* stage[2] = {nullptr, nullptr};

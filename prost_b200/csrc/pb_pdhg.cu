@@ -193,13 +193,6 @@ __global__ void __launch_bounds__(kBlock) z_variable_kernel(float* __restrict__ 
 
 // ---- backend -------------------------------------------------------------------------------------
 
-// default number of iterations per persistent-ring launch (0: one launch per iteration).  Multi-iteration
-// launches (RingMulti) are bit-identical but measured SLOWER on 1 and 2 GPUs (profiles/r02_scaling.md): the
-// per-tile release fences sit on the tile pipeline's critical path; PB_RING_ITERS=n enables them for experiments.
-constexpr int kRingItersDefault = 0;
-
-constexpr int kOverlapIdentityDefault = 0;
-
 class BackendPDHG : public Backend {
  public:
   BackendPDHG(Context* ctx, std::shared_ptr<Problem> prob, const pb_pdhg_options& opts,
@@ -208,12 +201,6 @@ class BackendPDHG : public Backend {
     if (opts_.residual_iter == 0) fail(PB_ERR_INVALID, "residual_iter must not be 0");
     if (opts_.stepsize_variant < PB_PDHG_ALG1 || opts_.stepsize_variant > PB_PDHG_BOYD)
       fail(PB_ERR_INVALID, "unknown PDHG step size variant");
-  }
-
-  ~BackendPDHG() override {
-    if (fork_ev_) cudaEventDestroy(fork_ev_);
-    if (join_ev_) cudaEventDestroy(join_ev_);
-    if (side_stream_) cudaStreamDestroy(side_stream_);
   }
 
   void initialize(const float* h_x0, size_t nx0, const float* h_y0, size_t ny0) override;
@@ -233,7 +220,6 @@ class BackendPDHG : public Backend {
   unsigned long long one_pass_iterations() const override { return tile_iterations_; }
   void device_iterates(float** d_x, float** d_y) override { *d_x = x_.data(); *d_y = y_.data(); }
   int residual_iter() const override { return opts_.residual_iter; }
-  bool batches_iterations() const override { return fused_ && tile_ok_ && ring_iters_ > 1; }
   void set_slab(Comm* comm) override { comm_ = comm; }
 
  private:
@@ -241,18 +227,8 @@ class BackendPDHG : public Backend {
   void slab_primal_halo(unsigned xs);
   void slab_dual_halo(unsigned xs, unsigned ys);
   RingHalo slab_ring_halo();           // advances x_seq / y_seq: one-pass iteration on a slab
-  // experimental (PB_RING_ITERS > 1): up to ring_iters_ consecutive non-refresh iterations in one launch
-  bool is_check_at(unsigned long long it) const {
-    const unsigned long long mod = static_cast<unsigned long long>(static_cast<long long>(opts_.residual_iter));
-    return it == 0 || (it % mod) == 0;
-  }
-  bool multi_iteration_launch(int n_it);
-  int ring_iters_ = 0;
-  unsigned ring_base_ = 0;
-  DeviceBuffer<unsigned> ring_done_, ring_edge_counters_;
   DeviceBuffer<unsigned> fin_ticket_;        // RingFinish: CTAs of the running residual-refresh launch that are done
   RingFinish ring_finish();
-  DeviceBuffer<int> ring_error_;
   void slab_apply(float* d_res, const float* d_rhs, const float* d_halo, bool adjoint);
   Comm* comm_ = nullptr;
   bool halo_in_ll_ = false;            // the newest halo columns live in the ring kernel's flag-in-data slots only
@@ -265,10 +241,6 @@ class BackendPDHG : public Backend {
   bool plan_fused();
   void iteration_fused();
   cudaEvent_t* prof_ev_ = nullptr;     // 4 events when profiling, else null
-  // identity-row dual pass beside the gradient-row pass (0 = off, else CTAs per SM for the identity pass)
-  int overlap_identity_ = 0;
-  cudaStream_t side_stream_ = nullptr;
-  cudaEvent_t fork_ev_ = nullptr, join_ev_ = nullptr;
   void iteration_unfused();
   PdhgState fetch_state();
   unsigned sgrid(size_t n) const { return (unsigned)std::min<size_t>(grid_for(n), (size_t)ctx_->num_sms * 32); }
@@ -343,16 +315,6 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
 
   iteration_ = 0;
   halo_in_ll_ = false;
-  {
-    // PB_OVERLAP_IDENTITY: CTAs per SM of the identity-row pass while it runs beside the gradient-row pass (0: off)
-    static const int want = [] { const char* e = getenv("PB_OVERLAP_IDENTITY"); return e ? atoi(e) : kOverlapIdentityDefault; }();
-    overlap_identity_ = want > 0 ? want : 0;
-    if (overlap_identity_ && !side_stream_) {
-      PB_CUDA(cudaStreamCreateWithFlags(&side_stream_, cudaStreamNonBlocking));
-      PB_CUDA(cudaEventCreateWithFlags(&fork_ev_, cudaEventDisableTiming));
-      PB_CUDA(cudaEventCreateWithFlags(&join_ev_, cudaEventDisableTiming));
-    }
-  }
   PdhgState st{};
   st.tau = static_cast<float>(opts_.tau0);
   st.sigma = static_cast<float>(opts_.sigma0);
@@ -428,25 +390,17 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
   vote(!(ny0 > 0 && ny0 != m), PB_ERR_INVALID, "Initial dual solution has wrong size.");
 
   { PB_TRACE_SCOPE("  plan_fused"); fused_ = plan_fused(); }
+  // one-pass iterations run the ring kernel only: its dry run decides here, a launch that fails later is an error
   tile_ok_ = fused_ && opts_.fuse == 1 &&
-             tile_iteration_supported(stencil_, g_descs_, f_descs_, problem_->right_ref(), problem_->left_ref());
+             tile_iteration_supported(stencil_, g_descs_, f_descs_, problem_->right_ref(), problem_->left_ref()) &&
+             tile_ring_available(ctx_, stencil_, g_descs_[0], f_descs_[0], comm_ != nullptr);
   // slabs: the one-pass kernel stores its edge columns straight into the neighbours' memory, so it
-  // needs the peer-to-peer halo blocks and the persistent-ring variant (PB_SLAB_TILE=0: two passes)
+  // needs the peer-to-peer halo blocks (PB_SLAB_TILE=0: two passes)
   if (comm_) {
     static const bool slab_tile = [] { const char* e = getenv("PB_SLAB_TILE"); return !e || atoi(e) != 0; }();
-    tile_ok_ = tile_ok_ && slab_tile && tile_ring_available() && stencil_.geom.nx >= 2;
+    tile_ok_ = tile_ok_ && slab_tile && stencil_.geom.nx >= 2;
   }
   tile_iterations_ = 0;
-  {
-    // Iterations per launch of the persistent ring (RingMulti); PB_RING_ITERS overrides the default.
-    static const int ring_iters = [] { const char* e = getenv("PB_RING_ITERS"); return e ? atoi(e) : -1; }();
-    const int dflt = kRingItersDefault;
-    ring_iters_ = std::min(ring_iters >= 0 ? ring_iters : dflt, 32);
-    // one GPU only: bit-identical to single launches there (tests/test_gpu_ring_multi.py); on column slabs the
-    // multi-iteration launch did not complete in bring-up (profiles/r02_scaling.md), so slabs always take one
-    // iteration per launch
-    if (comm_) ring_iters_ = 0;
-  }
   if (comm_) {
     // the halo protocol lives in the specialised stencil passes: one planar gradient operator
     // (+ identity rows), one prox_g over all columns, Norm2 on the gradient rows
@@ -483,16 +437,6 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
     try {
       x_.resize(n); x_prev_.resize(n); y_.resize(m); y_prev_.resize(m);
       if (tile_ok_) y_stage_.resize(m);
-      if (tile_ok_ && ring_iters_ > 1) {
-        const unsigned n_tiles = tile_ring_tile_count(stencil_);
-        ring_done_.resize(std::max(n_tiles, 1024u));
-        ring_done_.zero(s);
-        ring_edge_counters_.resize(64);
-        ring_edge_counters_.zero(s);
-        ring_error_.resize(1);
-        ring_error_.zero(s);
-        ring_base_ = 0;
-      }
       if (!fused_) {
         temp_.resize(std::max(m, n));
         kx_.resize(m); kx_prev_.resize(m); kty_.resize(n); kty_prev_.resize(n);
@@ -557,7 +501,6 @@ void BackendPDHG::iteration_fused() {
   const PdhgState* st = d_state_.data();
 
   unsigned nd = 0, np = 0;
-  unsigned tiled_check = 0;
   RingHalo ring_halo;
   const bool tiled = tile_ok_ && iteration_ > 0;
   if (tiled && comm_) ring_halo = slab_ring_halo();
@@ -566,22 +509,15 @@ void BackendPDHG::iteration_fused() {
   // itself (RingFinish) unless the halos travel through NCCL staging buffers (no peer-mapped slots then)
   bool finished_in_kernel = false;
   if (tiled && check) {
-    static const bool in_kernel = [] { const char* e = getenv("PB_RING_FINISH"); return !e || atoi(e) != 0; }();
-    const bool can_finish = in_kernel && (!comm_ || comm_->world() == 1 || comm_->reduce_p2p());
+    const bool can_finish = !comm_ || comm_->world() == 1 || comm_->reduce_p2p();
     RingFinish fin;
     if (can_finish) fin = ring_finish();
-    tiled_check = tile_check_iteration_launch(ctx_, stencil_, g_descs_[0], f_descs_[0], x_.data(), y_.data(),
-                                              y_prev_.data(), T, S, st, iteration_ <= 1, part_d_.data(),
-                                              part_p_.data(), x_prev_.data(), y_prev_staging(), false, rh,
-                                              can_finish ? &fin : nullptr);
-    if (!tiled_check && comm_)
-      fail(PB_ERR_CUDA, "slab decomposition: the one-pass ring kernel could not be launched");
-    finished_in_kernel = tiled_check && can_finish;
-  }
-  if (tiled_check) {
     // residual-refresh iteration in one pass: x_prev_ <- x^{k+1}; y^{k+1} cannot overwrite y_prev_ (the
     // pass reads y^{k-1} from it), so it goes to a third buffer that then takes y_prev_'s place
-    nd = np = tiled_check;
+    nd = np = tile_check_iteration_launch(ctx_, stencil_, g_descs_[0], f_descs_[0], x_.data(), y_.data(),
+                                          y_prev_.data(), T, S, st, iteration_ <= 1, part_d_.data(), part_p_.data(),
+                                          x_prev_.data(), y_prev_staging(), rh, can_finish ? &fin : nullptr);
+    finished_in_kernel = can_finish;
     tile_check_iterations_++;
     x_.swap(x_prev_);
     y_prev_.swap(y_stage_);      // y_prev_ now holds y^{k+1}, y_stage_ the dead y^{k-1}
@@ -591,7 +527,7 @@ void BackendPDHG::iteration_fused() {
       PB_CUDA(cudaEventRecord(prof_ev_[1], ctx_->stream));
       PB_CUDA(cudaEventRecord(prof_ev_[2], ctx_->stream));
     }
-  } else if (tile_ok_ && !check && iteration_ > 0) {
+  } else if (tiled) {
     // whole iteration in one pass over HBM (pb_tile.cu): x_prev_ <- x^{k+1}, y_prev_ <- y^{k+1}
     tile_iteration_launch(ctx_, stencil_, g_descs_[0], f_descs_[0], x_.data(), y_.data(), T, S, st,
                           x_prev_.data(), y_prev_.data(), rh);
@@ -624,32 +560,7 @@ void BackendPDHG::iteration_fused() {
     if (prof_ev_) PB_CUDA(cudaEventRecord(prof_ev_[1], ctx_->stream));
 
     // dual pass: y_prev_ <- prox_f*(y_ + sigma S K(2x^{k+1} - x^k)) (theta-extrapolated), then swap
-    // Gradient rows + identity rows (the lifting config): the identity-row pass is bound by the arithmetic of its
-    // prox (epigraph projection), the gradient-row pass by HBM; they write disjoint rows of y.  On plain iterations
-    // the identity pass goes first, on a second stream with a few CTAs per SM, and the gradient pass fills the rest
-    // of every SM: the two run side by side instead of back to back (profiles/r02_lifting.md).
     off = 0;
-    const bool side_by_side = overlap_identity_ && !check && !prof_ev_ && f_descs_.size() == 2 && stencil_.ok &&
-                              stencil_.geom.has_id && f_descs_[1].index == stencil_.geom.id_row;
-    if (side_by_side) {
-      cudaStream_t main = ctx_->stream;
-      PB_CUDA(cudaEventRecord(fork_ev_, main));
-      PB_CUDA(cudaStreamWaitEvent(side_stream_, fork_ev_, 0));
-      ctx_->stream = side_stream_;
-      ctx_->identity_ctas_per_sm = overlap_identity_;
-      const unsigned gi = stencil_dual_launch(ctx_, stencil_, f_descs_[1], y_.data(), x_.data(), x_prev_.data(),
-                                              f_scale_[1], st, iteration_ == 0, false, part_p_.data(), y_prev_.data());
-      ctx_->identity_ctas_per_sm = 0;
-      ctx_->stream = main;
-      if (gi == 0) fail(PB_ERR_UNSUPPORTED, "identity-row pass not launched");
-      PB_CUDA(cudaEventRecord(join_ev_, side_stream_));
-      const unsigned gg = stencil_dual_launch(ctx_, stencil_, f_descs_[0], y_.data(), x_.data(), x_prev_.data(),
-                                              f_scale_[0], st, iteration_ == 0, false, part_p_.data(), y_prev_.data());
-      if (gg == 0)
-        fused_dual_launch(ctx_, f_descs_[0], blocks_, y_.data(), x_.data(), x_prev_.data(), f_scale_[0], st,
-                          iteration_ == 0, false, part_p_.data(), y_prev_.data());
-      PB_CUDA(cudaStreamWaitEvent(main, join_ev_, 0));
-    } else
     for (size_t i = 0; i < f_descs_.size(); ++i) {
       const ProxDesc& d = f_descs_[i];
       const ScaleRef Sd = f_scale_[i];
@@ -892,64 +803,16 @@ void BackendPDHG::profile_detail(int n_iters, float out[8]) {
 
 void BackendPDHG::iterate(int n_iters) {
   ctx_->bind();
-  for (int i = 0; i < n_iters;) {
-    if (fused_ && tile_ok_ && ring_iters_ > 1 && iteration_ > 0 && !prof_ev_ &&
-        opts_.stepsize_variant != PB_PDHG_ALG2) {
-      // stretch of iterations that neither refresh the residuals nor change the step sizes
-      int r = 0;
-      while (i + r < n_iters && r < ring_iters_ && !is_check_at(iteration_ + r)) ++r;
-      if (r >= 2 && multi_iteration_launch(r)) { i += r; continue; }
-    }
+  for (int i = 0; i < n_iters; ++i) {
     if (fused_) iteration_fused();
     else iteration_unfused();
-    ++i;
   }
-}
-
-// n_it >= 2 non-refresh iterations in one launch of the persistent ring kernel (pb_tile.cu, RingMulti)
-bool BackendPDHG::multi_iteration_launch(int n_it) {
-  if (ring_done_.size() == 0) return false;
-  const ScaleRef T = problem_->right_ref(), S = problem_->left_ref();
-  RingMulti mi;
-  mi.n_it = n_it;
-  mi.base = ring_base_;
-  mi.done = ring_done_.data();
-  mi.error = ring_error_.data();
-  {
-    static const int coarse = [] { const char* e = getenv("PB_RING_COARSE"); return e ? atoi(e) : 0; }();
-    static const int debug = [] { const char* e = getenv("PB_RING_DEBUG"); return e ? atoi(e) : 0; }();
-    mi.coarse = coarse;
-    mi.debug = debug;
-  }
-  mi.x_io[0] = x_.data(); mi.x_io[1] = x_prev_.data();
-  mi.y_io[0] = y_.data(); mi.y_io[1] = y_prev_.data();
-  RingHalo h;
-  const unsigned xs0 = comm_ ? comm_->x_seq : 0, ys0 = comm_ ? comm_->y_seq : 0;
-  if (comm_) {
-    h = slab_ring_halo();                       // sequence numbers of the launch's first iteration
-  }
-  const unsigned grid = tile_multi_iteration_launch(ctx_, stencil_, g_descs_[0], f_descs_[0], x_.data(), y_.data(),
-                                                    x_prev_.data(), y_prev_.data(), T, S, d_state_.data(), mi,
-                                                    comm_ ? &h : nullptr);
-  if (!grid) {
-    if (comm_) { comm_->x_seq = xs0; comm_->y_seq = ys0; }     // nothing ran: take the sequence numbers back
-    return false;
-  }
-  if (comm_) { comm_->x_seq = xs0 + n_it; comm_->y_seq = ys0 + n_it; }
-  ring_base_ += static_cast<unsigned>(n_it);
-  if (n_it & 1) { x_.swap(x_prev_); y_.swap(y_prev_); }        // the newest iterate is in set (n_it & 1)
-  iteration_ += n_it;
-  tile_iterations_ += n_it;
-  return true;
 }
 
 PdhgState BackendPDHG::fetch_state() {
   if (fused_) {
     d_state_.download(&h_state_, 1, ctx_->stream);
-    int ring_err = 0;
-    if (ring_error_.size()) ring_error_.download(&ring_err, 1, ctx_->stream);
     PB_CUDA(cudaStreamSynchronize(ctx_->stream));
-    if (ring_err) fail(PB_ERR_CUDA, "multi-iteration ring kernel: a tile dependency wait timed out");
   }
   return h_state_;
 }

@@ -501,8 +501,7 @@ unsigned stencil_dual_identity_launch(Context* ctx, const GradGeom& g, const Pro
                                       bool dry_run) {
   const int cap = dim_cap(d.dim, d.kind);
   if (cap == 0 || cap > 8) return 0;
-  const size_t per_sm = ctx->identity_ctas_per_sm > 0 && !check ? (size_t)ctx->identity_ctas_per_sm : 16;
-  const unsigned grid = (unsigned)std::min<size_t>(grid_for(d.count), (size_t)ctx->num_sms * per_sm);
+  const unsigned grid = (unsigned)std::min<size_t>(grid_for(d.count), (size_t)ctx->num_sms * 16);
   if (dry_run || d.count == 0) return d.count ? grid : 0;
 #define PB_ARGS ctx, grid, g, d, y, x_new, x_old, S, st, kxprev_zero, check, partials, y_out
   switch (cap) {

@@ -86,30 +86,6 @@ struct RingHalo {
   int* error = nullptr;                // set when a wait times out
 };
 
-// Several consecutive non-refresh iterations in ONE launch of the persistent ring kernel (experimental,
-// PB_RING_ITERS > 1): the CTAs stay resident and a tile of iteration it+1 starts as soon as its 3 x 3 tile
-// neighbourhood has finished iteration it (per-tile counters in global memory, release / acquire at gpu scope,
-// fence.proxy.async before the TMA loads), so the kernel boundary -- launch latency, pipeline prologue and
-// tail -- is paid once per launch instead of once per iteration.  Iterates ping-pong between the two buffer
-// sets io[0] (input of even iterations) and io[1].
-struct RingMulti {
-  int n_it = 1;
-  unsigned base = 0;                   // value of every done[] counter when the launch starts
-  unsigned* done = nullptr;            // per tile: iterations completed (monotonic across launches)
-  int* error = nullptr;                // set when a dependency wait times out
-  float* x_io[2] = {nullptr, nullptr};
-  float* y_io[2] = {nullptr, nullptr};
-  // dependency granularity: 0 = per tile (one release per tile, 3 x 3 tile neighbourhood probed per work item),
-  // 1 = per CTA and iteration (one release per CTA and iteration: done[cta] counts the iterations the CTA has
-  // finished; a work item waits for the CTAs that own its neighbour tiles)
-  int coarse = 0;
-  int debug = 0;                       // timing experiments only: bit 0 skips the release, bit 1 the probe
-  // PB_RING_TRACE: per launch {first CTA start, last CTA end, longest left-edge halo wait, longest right-edge halo
-  // wait} in globaltimer ns (atomicMin / atomicMax), slot = launch number modulo the buffer length
-  unsigned long long* trace = nullptr;
-  unsigned trace_slot = 0;
-};
-
 // Residual-refresh launches of the ring kernel finish the iteration themselves: the last CTA to arrive (ticket)
 // folds the per-CTA partial sums in index order, on slabs combines them across ranks through peer-mapped slots
 // (cross_rank_sum4, pb_crosssum.cuh: identical bits on all ranks), and runs the step-size state machine
@@ -728,23 +704,20 @@ unsigned stencil_dual_launch(Context* ctx, const StencilPlan& plan, const ProxDe
 // ---- whole iteration as one tiled pass (pb_tile.cu) ---------------------------------------------
 bool tile_iteration_supported(const StencilPlan& plan, const std::vector<ProxDesc>& gd,
                               const std::vector<ProxDesc>& fd, ScaleRef T, ScaleRef S);
+// can the ring kernel run this plan, plain and residual-refresh launch alike (slab: the halo variants)?
+bool tile_ring_available(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf, bool slab);
+// plain iteration as one tiled pass; raises PB_ERR_CUDA if the ring kernel cannot be launched
 void tile_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
                            const float* x, const float* y, ScaleRef T, ScaleRef S, const PdhgState* st,
                            float* x_out, float* y_out, const RingHalo* halo = nullptr);
-// slab mode: is the persistent ring (the only one-pass variant that speaks the halo protocol) available?
-bool tile_ring_available();
-unsigned tile_ring_trace_read(unsigned long long* h_out, unsigned n);      // PB_RING_TRACE experiments
-// several consecutive non-refresh iterations in one launch (RingMulti; experimental, PB_RING_ITERS > 1)
-unsigned tile_ring_tile_count(const StencilPlan& plan);
-unsigned tile_multi_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
-                                     float* x_a, float* y_a, float* x_b, float* y_b, ScaleRef T, ScaleRef S,
-                                     const PdhgState* st, const RingMulti& multi, const RingHalo* halo);
 // residual-refresh iteration as one tiled pass; returns the number of (a, b) partial pairs written to each of
-// part_d (dual residual sums) and part_p (primal residual sums), 0 if the two-pass kernels have to run
+// part_d (dual residual sums) and part_p (primal residual sums); raises PB_ERR_CUDA if the ring kernel cannot
+// be launched
 unsigned tile_check_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
                                      const float* x, const float* y, const float* y_prev, ScaleRef T, ScaleRef S,
                                      const PdhgState* st, bool ktyprev_zero, double* part_d, double* part_p,
-                                     float* x_out, float* y_out, bool dry_run = false,
-                                     const RingHalo* halo = nullptr, const RingFinish* finish = nullptr);
+                                     float* x_out, float* y_out, const RingHalo* halo = nullptr,
+                                     const RingFinish* finish = nullptr);
+unsigned tile_ring_trace_read(unsigned long long* h_out, unsigned n);      // PB_RING_TRACE experiments
 
 }  // namespace pb

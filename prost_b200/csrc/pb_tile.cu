@@ -1,17 +1,17 @@
 // pb_tile.cu -- one whole PDHG iteration in ONE pass over HBM for planar 2-D gradient operators.
 //
 // The two-pass schedule (pb_stencil.cuh) moves 44 B per pixel and iteration for ROF: the dual pass
-// re-reads x+, x and y that the primal pass had in registers a moment earlier.  Here a CTA owns a
-// TX x TY tile of the image:
+// re-reads x+, x and y that the primal pass had in registers a moment earlier.  Here an owned tile of
+// TX x TY pixels is computed in two phases:
 //   phase A  x+ = prox_g(x - tau T K^T y) on the tile PLUS one halo column (x = cx+TX) and one
-//            halo row (y = cy+TY): the forward differences of the dual step need x+ there.  x+ and
+//            halo row vector (y = cy+TY): the forward differences of the dual step need x+ there.  x+ and
 //            x of the extended tile go to shared memory; the tile's own x+ is written to HBM.
 //   phase B  y+ = prox_f*(y + sigma S ((1+theta) K x+ - theta K x)) on the tile, with K x+ and K x
 //            taken from shared memory.
 // HBM traffic per pixel: read y (2), x, f; write x+, y+ (2) = 7 floats = 28 B instead of 44 B; the
-// halo re-computation costs (TX+1)(TY+1)/(TX TY) - 1 = 3.9 % extra arithmetic and loads that hit L2
-// (they are a neighbouring tile's primary loads).  The halo values of x+ are recomputed with exactly
-// the same instructions as in the tile that owns them, so the result is bit-identical to the
+// halo re-computation costs (TX+1)(TY+4)/(TX TY) - 1 = 6.6 % extra arithmetic (TX = 31, TY = 124) and loads
+// that hit L2 (they are a neighbouring tile's primary loads).  The halo values of x+ are recomputed with
+// exactly the same instructions as in the tile that owns them, so the result is bit-identical to the
 // two-pass kernels, which in turn follow the reference operation by operation
 // (backend_pdhg.cu:38-70, 311-381; block_gradient2d.cu:25-139).
 //
@@ -31,210 +31,6 @@ namespace pb {
 
 namespace {
 
-constexpr int kTileThreads = 256;
-// Tile shape: TX columns x TY rows (y is the contiguous direction).  TY/4 threads cover one column
-// with 128-bit accesses, the CTA sweeps kTileThreads/(TY/4) columns at a time.  Shared row pitch
-// TY + 4 floats: tile + halo row, 16-byte aligned.
-
-// prox_g on VEC lanes: ProxElemOperation<ElemOperation1D<FN>> with scalar weights and an optional
-// per-pixel b (same code path as grad_primal_body's scalar-weight branch)
-template <int VEC, int FN>
-__device__ __forceinline__ void elem1d_lanes(const ProxDesc& p, const Coeffs7& c0, const bool simple,
-                                             const float tau, const float Tval, const uint32_t e,
-                                             float (&arg)[VEC]) {
-  float bv[VEC];
-  if (p.coeffs.ptr[1]) {
-    VecIO<VEC>::ld(p.coeffs.ptr[1] + e, bv);
-  } else {
-#pragma unroll
-    for (int j = 0; j < VEC; ++j) bv[j] = c0.v[1];
-  }
-  const int fn = FN >= 0 ? FN : p.fn;
-  if (simple) {
-    const float tau_eff = effective_tau(tau, Tval, false);
-#pragma unroll
-    for (int j = 0; j < VEC; ++j)
-      arg[j] = scaled_fun_prox_simple(fn, arg[j], tau_eff, bv[j], c0.v[2], c0.v[5], c0.v[6]);
-  } else {
-    Coeffs7 c = c0;
-#pragma unroll
-    for (int j = 0; j < VEC; ++j) {
-      c.v[1] = bv[j];
-      arg[j] = elem1d_apply(fn, arg[j], tau, Tval, false, c);
-    }
-  }
-}
-
-// x+ at VEC consecutive y of column gx (label plane l); returns x (old) in xo and x+ in xn
-template <int VEC, int FN>
-__device__ __forceinline__ void primal_point(const GradGeom& g, const ProxDesc& pg, const Coeffs7& cg,
-                                             const bool simple, const float* __restrict__ x,
-                                             const float* __restrict__ y, const float tau, const float Tval,
-                                             const uint32_t gx, const uint32_t gy, const uint32_t l,
-                                             float (&xo)[VEC], float (&xn)[VEC]) {
-  const uint32_t idx = gy + gx * g.ny + l * g.nxny;
-  float k[VEC];
-  VecIO<VEC>::ld(x + idx, xo);
-  grad_adj<VEC, false, false, false>(g, y, nullptr, idx, gx, gy, l, k);
-#pragma unroll
-  for (int j = 0; j < VEC; ++j) xn[j] = primal_prox_arg(xo[j], tau, Tval, k[j]);
-  elem1d_lanes<VEC, FN>(pg, cg, simple, tau, Tval, idx, xn);
-}
-
-template <int kTX, int kTY, int FN_G, int FN_F>
-__global__ void __launch_bounds__(kTileThreads, 3) grad2d_iteration_tile_kernel(
-    const GradGeom g, const ProxDesc pg, const ProxDesc pf, const float* __restrict__ x,
-    const float* __restrict__ y, const float Tval, const float Sval, const PdhgState* __restrict__ st,
-    const uint32_t tiles_y, float* __restrict__ x_out, float* __restrict__ y_out) {
-  constexpr int kSRow = kTY + 4;
-  constexpr int kLanesY = kTY / 4;                    // threads per column
-  constexpr int kColsPerSweep = kTileThreads / kLanesY;
-  constexpr int kSweeps = kTX / kColsPerSweep;
-  static_assert(kTX % kColsPerSweep == 0 && kTX <= 32 && kLanesY <= kTileThreads - 32, "tile shape");
-  __shared__ __align__(16) float sxn[kTX + 1][kSRow];
-  __shared__ __align__(16) float sxo[kTX + 1][kSRow];
-
-  const float tau = st->tau, sigma = st->sigma, theta = st->theta;
-  const uint32_t tile = blockIdx.x;
-  const uint32_t tx = tile / tiles_y, ty = tile - tx * tiles_y;
-  const uint32_t cx = tx * kTX, cy = ty * kTY;
-  const uint32_t l = blockIdx.y;
-  const uint32_t lane = threadIdx.x & 31;
-  const uint32_t tcol = threadIdx.x / kLanesY;        // column of this thread within a sweep
-  const uint32_t ly = (threadIdx.x % kLanesY) * 4, gy = cy + ly;
-
-  Coeffs7 cg, cf;
-#pragma unroll
-  for (int k = 0; k < 7; ++k) { cg.v[k] = pg.coeffs.val[k]; cf.v[k] = pf.coeffs.val[k]; }
-  const bool g_simple = coeffs_simple(cg) && cg.v[2] != 0.f;
-
-  // ---- phase A: x+ on the extended tile ---------------------------------------------------------
-#pragma unroll
-  for (int s = 0; s < kSweeps; ++s) {
-    const uint32_t col = tcol + kColsPerSweep * s, gx = cx + col;
-    if (gx < g.nx && gy < g.ny) {
-      float xo[4], xn[4];
-      primal_point<4, FN_G>(g, pg, cg, g_simple, x, y, tau, Tval, gx, gy, l, xo, xn);
-      VecIO<4>::st(x_out + gy + gx * g.ny + l * g.nxny, xn);
-      VecIO<4>::st(&sxn[col][ly], xn);
-      VecIO<4>::st(&sxo[col][ly], xo);
-    }
-  }
-  if (threadIdx.x < kLanesY) {           // halo column x = cx + TX (owned by the tile to the right)
-    const uint32_t gx = cx + kTX;
-    if (gx < g.nx && gy < g.ny) {
-      float xo[4], xn[4];
-      primal_point<4, FN_G>(g, pg, cg, g_simple, x, y, tau, Tval, gx, gy, l, xo, xn);
-      VecIO<4>::st(&sxn[kTX][ly], xn);
-      VecIO<4>::st(&sxo[kTX][ly], xo);
-    }
-  } else if (threadIdx.x >= kTileThreads - 32) {   // halo row y = cy + TY (owned by the tile below)
-    const uint32_t gx = cx + lane, hy = cy + kTY;
-    if (lane < kTX && gx < g.nx && hy < g.ny) {
-      float xo[1], xn[1];
-      primal_point<1, FN_G>(g, pg, cg, g_simple, x, y, tau, Tval, gx, hy, l, xo, xn);
-      sxn[lane][kTY] = xn[0];
-      sxo[lane][kTY] = xo[0];
-    }
-  }
-  __syncthreads();
-
-  // ---- phase B: y+ on the tile --------------------------------------------------------------------
-  const int fn_f = FN_F >= 0 ? FN_F : pf.fn;
-  const float tau_f = effective_tau(sigma, Sval, false);
-  const bool f_simple = coeffs_simple(cf);
-#pragma unroll
-  for (int s = 0; s < kSweeps; ++s) {
-    const uint32_t col = tcol + kColsPerSweep * s, gx = cx + col;
-    if (gx < g.nx && gy < g.ny) {
-      const uint32_t idx = gy + gx * g.ny + l * g.nxny;
-      float arg[2][4];
-      float cn[4], co[4], rn[4], ro[4];
-      VecIO<4>::ld(&sxn[col][ly], cn);
-      VecIO<4>::ld(&sxo[col][ly], co);
-      float k1x[4], k0x[4], k1y[4], k0y[4];
-      if (gx < g.nx - 1) {               // grad_fwd: gx = u[idx+ny] - u[idx], 0 on the last column
-        VecIO<4>::ld(&sxn[col + 1][ly], rn);
-        VecIO<4>::ld(&sxo[col + 1][ly], ro);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { k1x[j] = rn[j] - cn[j]; k0x[j] = ro[j] - co[j]; }
-      } else {
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { k1x[j] = 0.f; k0x[j] = 0.f; }
-      }
-#pragma unroll
-      for (int j = 0; j < 3; ++j) { k1y[j] = cn[j + 1] - cn[j]; k0y[j] = co[j + 1] - co[j]; }
-      if (gy + 4 < g.ny) {               // gy = u[idx+1] - u[idx], 0 on the last row
-        k1y[3] = sxn[col][ly + 4] - cn[3];
-        k0y[3] = sxo[col][ly + 4] - co[3];
-      } else {
-        k1y[3] = 0.f;
-        k0y[3] = 0.f;
-      }
-      float y1[4], y2[4];
-      VecIO<4>::ld(y + idx, y1);
-      VecIO<4>::ld(y + g.plane + idx, y2);
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        arg[0][j] = dual_prox_arg(y1[j], sigma, Sval, dual_extrapolate(theta, k1x[j], k0x[j]));
-        arg[1][j] = dual_prox_arg(y2[j], sigma, Sval, dual_extrapolate(theta, k1y[j], k0y[j]));
-      }
-      if (f_simple) norm2_lanes<4, 2, true>(fn_f, arg, cf, tau_f);
-      else norm2_lanes<4, 2, false>(fn_f, arg, cf, tau_f);
-      VecIO<4>::st(y_out + idx, arg[0]);
-      VecIO<4>::st(y_out + g.plane + idx, arg[1]);
-    }
-  }
-}
-
-template <int TX, int TY, int FN_G>
-void tile_launch_f(Context* ctx, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf, const float* x,
-                   const float* y, float Tval, float Sval, const PdhgState* st, float* x_out, float* y_out) {
-  const uint32_t tiles_x = (g.nx + TX - 1) / TX, tiles_y = (g.ny + TY - 1) / TY;
-  const dim3 grid(tiles_x * tiles_y, g.L, 1);
-  if (pf.fn == PB_FUN_IND_LEQ0)
-    grad2d_iteration_tile_kernel<TX, TY, FN_G, PB_FUN_IND_LEQ0><<<grid, kTileThreads, 0, ctx->stream>>>(
-        g, pg, pf, x, y, Tval, Sval, st, tiles_y, x_out, y_out);
-  else
-    grad2d_iteration_tile_kernel<TX, TY, FN_G, -1><<<grid, kTileThreads, 0, ctx->stream>>>(
-        g, pg, pf, x, y, Tval, Sval, st, tiles_y, x_out, y_out);
-}
-
-template <int TX, int TY>
-void tile_launch_g(Context* ctx, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf, const float* x,
-                   const float* y, float Tval, float Sval, const PdhgState* st, float* x_out, float* y_out) {
-  if (pg.fn == PB_FUN_SQUARE) tile_launch_f<TX, TY, PB_FUN_SQUARE>(ctx, g, pg, pf, x, y, Tval, Sval, st, x_out, y_out);
-  else if (pg.fn == PB_FUN_ABS) tile_launch_f<TX, TY, PB_FUN_ABS>(ctx, g, pg, pf, x, y, Tval, Sval, st, x_out, y_out);
-  else tile_launch_f<TX, TY, -1>(ctx, g, pg, pf, x, y, Tval, Sval, st, x_out, y_out);
-}
-
-
-// ---- TMA variant ------------------------------------------------------------------------------------
-// Same arithmetic, but every operand tile (with its halos) is brought into shared memory by four
-// cp.async.bulk.tensor (TMA) loads issued by one thread; the SM issues no global-load instructions at
-// all and the whole tile's bytes are in flight at once (the plain variant above is latency bound:
-// ncu long-scoreboard stalls, profiles/r01_tile.md).  Image borders come for free: out-of-range box
-// elements are zero-filled, which is exactly the K^T boundary rule for x = -1 and y = -1; the
-// x = nx-1 / y = ny-1 rules are applied in registers like in grad_adj / grad_fwd.
-//   box   origin (row, col)       extent (cols x rows)   used for
-//   p1    (cy,   cx-1)            (TX+2) x (TY+4)        gx component of y incl. left neighbour column
-//   p2    (cy-4, cx)              (TX+1) x (TY+8)        gy component of y incl. row cy-1 (16 B aligned)
-//   x, f  (cy,   cx)              (TX+1) x (TY+4)        primal iterate and data term incl. halo col / row
-constexpr int kTmaTX = 32, kTmaTY = 128;
-constexpr int kTmaR = kTmaTY + 4;          // rows per column in the p1 / x / f / x+ tiles
-constexpr int kTmaR2 = kTmaTY + 8;         // rows per column in the p2 tile (starts 4 rows early)
-constexpr int kTmaP1Bytes = (kTmaTX + 2) * kTmaR * 4;
-constexpr int kTmaP2Bytes = (kTmaTX + 1) * kTmaR2 * 4;
-constexpr int kTmaXBytes = (kTmaTX + 1) * kTmaR * 4;
-constexpr int align128(int v) { return (v + 127) / 128 * 128; }
-constexpr int kTmaOffP1 = 0;
-constexpr int kTmaOffP2 = kTmaOffP1 + align128(kTmaP1Bytes);
-constexpr int kTmaOffX = kTmaOffP2 + align128(kTmaP2Bytes);
-constexpr int kTmaOffF = kTmaOffX + align128(kTmaXBytes);
-constexpr int kTmaOffXn = kTmaOffF + align128(kTmaXBytes);
-constexpr int kTmaOffBar = kTmaOffXn + align128(kTmaXBytes);
-constexpr int kTmaSmemBytes = kTmaOffBar + 128;
-
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }
@@ -243,163 +39,6 @@ __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, v
       "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
       ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
       : "memory");
-}
-
-template <int FN_G, int FN_F>
-__global__ void __launch_bounds__(kTileThreads, 2) grad2d_iteration_tma_kernel(
-    const __grid_constant__ CUtensorMap map_p1, const __grid_constant__ CUtensorMap map_p2,
-    const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_f, const GradGeom g,
-    const ProxDesc pg, const ProxDesc pf, const float Tval, const float Sval,
-    const PdhgState* __restrict__ st, const uint32_t tiles_y, float* __restrict__ x_out,
-    float* __restrict__ y_out) {
-  extern __shared__ __align__(128) unsigned char smem[];
-  float (*s_p1)[kTmaR] = reinterpret_cast<float (*)[kTmaR]>(smem + kTmaOffP1);
-  float (*s_p2)[kTmaR2] = reinterpret_cast<float (*)[kTmaR2]>(smem + kTmaOffP2);
-  float (*s_x)[kTmaR] = reinterpret_cast<float (*)[kTmaR]>(smem + kTmaOffX);
-  float (*s_f)[kTmaR] = reinterpret_cast<float (*)[kTmaR]>(smem + kTmaOffF);
-  float (*s_xn)[kTmaR] = reinterpret_cast<float (*)[kTmaR]>(smem + kTmaOffXn);
-  uint64_t* bar = reinterpret_cast<uint64_t*>(smem + kTmaOffBar);
-
-  const uint32_t tile = blockIdx.x;
-  const uint32_t tx = tile / tiles_y, ty = tile - tx * tiles_y;
-  const int cx = tx * kTmaTX, cy = ty * kTmaTY;
-  const int l = blockIdx.y;
-  const bool f_vec = pg.coeffs.ptr[1] != nullptr;
-
-  if (threadIdx.x == 0) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(bar)));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const uint32_t bytes = kTmaP1Bytes + kTmaP2Bytes + kTmaXBytes + (f_vec ? kTmaXBytes : 0);
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-    tma_load_3d(s_p1, &map_p1, bar, cy, cx - 1, l);
-    tma_load_3d(s_p2, &map_p2, bar, cy - 4, cx, (int)g.L + l);
-    tma_load_3d(s_x, &map_x, bar, cy, cx, l);
-    if (f_vec) tma_load_3d(s_f, &map_f, bar, cy, cx, l);
-  }
-
-  const float tau = st->tau, sigma = st->sigma, theta = st->theta;
-  Coeffs7 cg, cf;
-#pragma unroll
-  for (int k = 0; k < 7; ++k) { cg.v[k] = pg.coeffs.val[k]; cf.v[k] = pf.coeffs.val[k]; }
-  const bool g_simple = coeffs_simple(cg) && cg.v[2] != 0.f;
-  const int fn_g = FN_G >= 0 ? FN_G : pg.fn;
-  const float tau_g = effective_tau(tau, Tval, false);
-
-  {  // wait for the four boxes (phase 0 of the one-shot barrier)
-    uint32_t done = 0;
-    while (!done) {
-      asm volatile(
-          "{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
-          : "=r"(done) : "r"(smem_u32(bar)), "r"(0u) : "memory");
-    }
-  }
-
-  // ---- phase A: x+ on (TX+1) columns x (TY+4) rows ---------------------------------------------------
-  constexpr int kVecA = kTmaR / 4;                       // 33 row vectors per column
-  for (int it = threadIdx.x; it < (kTmaTX + 1) * kVecA; it += kTileThreads) {
-    const int col = it / kVecA, v = it - col * kVecA;
-    const int r0 = 4 * v;
-    const uint32_t gx = cx + col, gy = cy + r0;
-    if (gx >= g.nx) continue;
-    float xo[4], divx[4], o[4], a[4], xn[4];
-    VecIO<4>::ld(&s_x[col][r0], xo);
-    if (gx < g.nx - 1) {
-      VecIO<4>::ld(&s_p1[col + 1][r0], divx);
-    } else {
-#pragma unroll
-      for (int j = 0; j < 4; ++j) divx[j] = 0.f;
-    }
-    if (gx > 0) {
-      VecIO<4>::ld(&s_p1[col][r0], a);
-#pragma unroll
-      for (int j = 0; j < 4; ++j) divx[j] -= a[j];
-    }
-    VecIO<4>::ld(&s_p2[col][4 + r0], o);
-    float divy[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) divy[j] = (gy + j == g.ny - 1) ? 0.f : o[j];
-#pragma unroll
-    for (int j = 1; j < 4; ++j) divy[j] -= o[j - 1];
-    if (gy > 0) divy[0] -= s_p2[col][4 + r0 - 1];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) xn[j] = primal_prox_arg(xo[j], tau, Tval, -(divx[j] + divy[j]));
-    float bv[4];
-    if (f_vec) {
-      VecIO<4>::ld(&s_f[col][r0], bv);
-    } else {
-#pragma unroll
-      for (int j = 0; j < 4; ++j) bv[j] = cg.v[1];
-    }
-    if (g_simple) {
-#pragma unroll
-      for (int j = 0; j < 4; ++j) xn[j] = scaled_fun_prox_simple(fn_g, xn[j], tau_g, bv[j], cg.v[2], cg.v[5], cg.v[6]);
-    } else {
-      Coeffs7 c = cg;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        c.v[1] = bv[j];
-        xn[j] = elem1d_apply(fn_g, xn[j], tau, Tval, false, c);
-      }
-    }
-    VecIO<4>::st(&s_xn[col][r0], xn);
-    if (col < kTmaTX && v < kTmaTY / 4 && gy < g.ny)
-      VecIO<4>::st(x_out + gy + gx * g.ny + (uint32_t)l * g.nxny, xn);
-  }
-  __syncthreads();
-
-  // ---- phase B: y+ on the TX x TY tile -----------------------------------------------------------------
-  const int fn_f = FN_F >= 0 ? FN_F : pf.fn;
-  const float tau_f = effective_tau(sigma, Sval, false);
-  const bool f_simple = coeffs_simple(cf);
-  constexpr int kVecB = kTmaTY / 4;
-#pragma unroll
-  for (int s = 0; s < kTmaTX * kVecB / kTileThreads; ++s) {
-    const int it = threadIdx.x + s * kTileThreads;
-    const int col = it / kVecB, v = it - col * kVecB;
-    const int r0 = 4 * v;
-    const uint32_t gx = cx + col, gy = cy + r0;
-    if (gx < g.nx && gy < g.ny) {
-      const uint32_t idx = gy + gx * g.ny + (uint32_t)l * g.nxny;
-      float arg[2][4];
-      float cn[4], co[4], rn[4], ro[4];
-      VecIO<4>::ld(&s_xn[col][r0], cn);
-      VecIO<4>::ld(&s_x[col][r0], co);
-      float k1x[4], k0x[4], k1y[4], k0y[4];
-      if (gx < g.nx - 1) {
-        VecIO<4>::ld(&s_xn[col + 1][r0], rn);
-        VecIO<4>::ld(&s_x[col + 1][r0], ro);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { k1x[j] = rn[j] - cn[j]; k0x[j] = ro[j] - co[j]; }
-      } else {
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { k1x[j] = 0.f; k0x[j] = 0.f; }
-      }
-#pragma unroll
-      for (int j = 0; j < 3; ++j) { k1y[j] = cn[j + 1] - cn[j]; k0y[j] = co[j + 1] - co[j]; }
-      if (gy + 4 < g.ny) {
-        k1y[3] = s_xn[col][r0 + 4] - cn[3];
-        k0y[3] = s_x[col][r0 + 4] - co[3];
-      } else {
-        k1y[3] = 0.f;
-        k0y[3] = 0.f;
-      }
-      float y1[4], y2[4];
-      VecIO<4>::ld(&s_p1[col + 1][r0], y1);
-      VecIO<4>::ld(&s_p2[col][4 + r0], y2);
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        arg[0][j] = dual_prox_arg(y1[j], sigma, Sval, dual_extrapolate(theta, k1x[j], k0x[j]));
-        arg[1][j] = dual_prox_arg(y2[j], sigma, Sval, dual_extrapolate(theta, k1y[j], k0y[j]));
-      }
-      if (f_simple) norm2_lanes<4, 2, true>(fn_f, arg, cf, tau_f);
-      else norm2_lanes<4, 2, false>(fn_f, arg, cf, tau_f);
-      VecIO<4>::st(y_out + idx, arg[0]);
-      VecIO<4>::st(y_out + g.plane + idx, arg[1]);
-    }
-  }
 }
 
 // ---- tensor maps (host) ------------------------------------------------------------------------------
@@ -447,50 +86,20 @@ bool tensor_map_for(const float* base, uint32_t ny, uint32_t nx, uint32_t planes
   return true;
 }
 
-template <int FN_G, int FN_F>
-bool tma_launch_fn(Context* ctx, const CUtensorMap& mp1, const CUtensorMap& mp2, const CUtensorMap& mx,
-                   const CUtensorMap& mf, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf, float Tval,
-                   float Sval, const PdhgState* st, float* x_out, float* y_out) {
-  auto kernel = grad2d_iteration_tma_kernel<FN_G, FN_F>;
-  static bool configured = false, ok = false;
-  if (!configured) {
-    configured = true;
-    ok = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTmaSmemBytes) == cudaSuccess;
-    cudaGetLastError();
-  }
-  if (!ok) return false;
-  const uint32_t tiles_x = (g.nx + kTmaTX - 1) / kTmaTX, tiles_y = (g.ny + kTmaTY - 1) / kTmaTY;
-  const dim3 grid(tiles_x * tiles_y, g.L, 1);
-  kernel<<<grid, kTileThreads, kTmaSmemBytes, ctx->stream>>>(mp1, mp2, mx, mf, g, pg, pf, Tval, Sval, st, tiles_y,
-                                                             x_out, y_out);
-  return true;
-}
-
-bool tma_launch(Context* ctx, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf, const float* x,
-                const float* y, float Tval, float Sval, const PdhgState* st, float* x_out, float* y_out) {
-  CUtensorMap mp1, mp2, mx, mf;
-  if (!tensor_map_for(y, g.ny, g.nx, 2 * g.L, kTmaR, kTmaTX + 2, mp1)) return false;
-  if (!tensor_map_for(y, g.ny, g.nx, 2 * g.L, kTmaR2, kTmaTX + 1, mp2)) return false;
-  if (!tensor_map_for(x, g.ny, g.nx, g.L, kTmaR, kTmaTX + 1, mx)) return false;
-  const float* f = pg.coeffs.ptr[1] ? pg.coeffs.ptr[1] : x;      // unused when b is a scalar
-  if (!tensor_map_for(f, g.ny, g.nx, g.L, kTmaR, kTmaTX + 1, mf)) return false;
-#define PB_ARGS ctx, mp1, mp2, mx, mf, g, pg, pf, Tval, Sval, st, x_out, y_out
-  const bool leq0 = pf.fn == PB_FUN_IND_LEQ0;
-  if (pg.fn == PB_FUN_SQUARE) return leq0 ? tma_launch_fn<PB_FUN_SQUARE, PB_FUN_IND_LEQ0>(PB_ARGS) : tma_launch_fn<PB_FUN_SQUARE, -1>(PB_ARGS);
-  if (pg.fn == PB_FUN_ABS) return leq0 ? tma_launch_fn<PB_FUN_ABS, PB_FUN_IND_LEQ0>(PB_ARGS) : tma_launch_fn<PB_FUN_ABS, -1>(PB_ARGS);
-  return leq0 ? tma_launch_fn<-1, PB_FUN_IND_LEQ0>(PB_ARGS) : tma_launch_fn<-1, -1>(PB_ARGS);
-#undef PB_ARGS
-}
-
-
 // ---- persistent TMA ring ------------------------------------------------------------------------------
-// The one-shot kernels above alternate between waiting for memory and computing: ncu shows DRAM
-// ~50 % busy and the issue slots ~50 % busy, i.e. the two phases serialise (profiles/r01_tile.md).
-// Here ONE CTA of 1024 threads stays resident per SM and walks over tiles; the operand boxes of the
-// next two tiles are always in flight (two shared-memory stages filled by TMA, completion signalled on
-// mbarriers), so HBM streams continuously while the 32 warps compute the current tile.
+// A kernel that loads one tile, computes it and exits alternates between waiting for memory and computing:
+// with plain loads or one-shot TMA boxes such kernels reached 72 % / 68 % of HBM bandwidth, against 84 %
+// for this one (profiles/r01_tile.md).  Here ONE CTA of 1024 threads stays resident per SM and walks over
+// tiles; the operand boxes of the next two tiles are always in flight (two shared-memory stages filled by
+// TMA, completion signalled on mbarriers), so HBM streams continuously while the 32 warps compute the
+// current tile.
 //   computed x+ region 32 columns x 128 rows = 1024 row vectors = exactly one per thread;
 //   owned tile         31 columns x 124 rows (the last column / 4 rows are the halo of the neighbours).
+// Operand boxes per tile at owned-tile origin (cy, cx); out-of-image elements are zero-filled by TMA,
+// which is exactly the K^T boundary rule for x = -1 and y = -1:
+//   p1    (cy,   cx-1)   33 columns x 128 rows   gx component of y incl. the left neighbour column
+//   p2    (cy-4, cx)     32 columns x 132 rows   gy component of y incl. row cy-1 (16-byte aligned)
+//   x, f  (cy,   cx)     32 columns x 128 rows   primal iterate and data term
 // There is no CTA-wide barrier in the loop: warp w computes column w; its dual step only needs the
 // x+ of columns w and w+1, so it waits on column w+1's mbarrier; a stage is recycled when all 32
 // warps have arrived on its `empty` barrier, which warp 31 (it owns the halo column and has no dual
@@ -581,32 +190,18 @@ __device__ __forceinline__ void ll_store4(uint4* p, const float (&v)[4], unsigne
                "r"(__float_as_uint(v[3])), "r"(seq) : "memory");
 }
 
-// RingMulti: wait until a tile's iteration counter has reached `want` (acquire, gpu scope).  Non-blocking mode
-// returns false at once; blocking mode gives up after ~2 s and raises the error word (no GPU hang).
-__device__ __forceinline__ bool ring_count_wait(const unsigned* flag, unsigned want, bool blocking, int* error) {
-  unsigned v;
-  unsigned long long t0 = 0;
-  for (unsigned spins = 0;; ++spins) {
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(flag) : "memory");
-    if ((int)(v - want) >= 0) return true;
-    if (!blocking) return false;
-    if (error && *reinterpret_cast<volatile int*>(error)) return true;
-    if ((spins & 1023u) == 1023u) {
-      unsigned long long now;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-      if (t0 == 0) t0 = now;
-      else if (now - t0 > 2000000000ull) { if (error) atomicExch(error, 1); return true; }
-    }
-  }
-}
+// PB_RING_TRACE: per launch {first CTA start, last CTA end, longest left-edge halo wait, longest right-edge halo
+// wait} in globaltimer ns (atomicMin / atomicMax) at buf[4 * slot]; slot = launch number modulo the buffer length
+struct RingTraceSlot {
+  unsigned long long* buf = nullptr;   // null: tracing off
+  unsigned slot = 0;
+};
 
 // CHECK: this iteration refreshes the residuals (backend_pdhg.cu:73-120, 383-436): the same pass also
 // gathers K^T y_prev from the previous dual iterate (map_q1 / map_q2) and accumulates the four residual
 // sums in double, one (a, b) pair per CTA for each of the two residuals.
 // SLAB: the image is a block of columns of a wider one (has_left / has_right neighbours, RingHalo).
-// MULTI: mi.n_it consecutive non-refresh iterations in one launch (RingMulti, pb_stencil.cuh); map_q1 / map_q2 /
-// map_xb are then the boxes over the second buffer set (odd iterations read it, even ones write it).
-template <int FN_G, int FN_F, bool CHECK, bool SLAB, bool MULTI = false>
+template <int FN_G, int FN_F, bool CHECK, bool SLAB>
 __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
     const __grid_constant__ CUtensorMap map_p1, const __grid_constant__ CUtensorMap map_p2,
     const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_f,
@@ -615,8 +210,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
     const PdhgState* __restrict__ st, const FastDiv div_per_plane, const FastDiv div_tiles_y,
     const uint32_t n_tiles, const int ktyprev_zero, double* __restrict__ part_d, double* __restrict__ part_p,
     float* __restrict__ x_out, float* __restrict__ y_out, const uint32_t tiles_x, const RingHalo h,
-    const __grid_constant__ CUtensorMap map_xb, const RingMulti mi, const RingFinish fin) {
-  static_assert(!(MULTI && CHECK), "residual-refresh iterations run one per launch");
+    const RingTraceSlot trace, const RingFinish fin) {
   extern __shared__ __align__(128) unsigned char smem[];
   // tile -> (label plane, tile column, tile row).  On a slab the left-edge tile column is walked first (its new x
   // column leaves at the start of the launch) and the right-edge one at the first position of the SECOND wave:
@@ -637,17 +231,16 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
   const uint32_t stage_tx = kRingP1Bytes + kRingP2Bytes + kRingXBytes +
                             (CHECK ? (q_boxes ? kRingP1Bytes + kRingP2Bytes : 0) : (f_vec ? kRingXBytes : 0));
 
-  auto issue = [&](uint32_t tile, int s, uint32_t iter) {           // producer lane only
+  auto issue = [&](uint32_t tile, int s) {           // producer lane only
     uint32_t l, tx, ty;
     decode(tile, l, tx, ty);
     const int cx = tx * kRingTX, cy = ty * kRingTY;
     unsigned char* base = smem + s * kRingStageBytes;
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&full[s])), "r"(stage_tx)
                  : "memory");
-    const bool odd = MULTI && (iter & 1u);       // odd iterations of a multi-iteration launch read buffer set 1
-    tma_load_3d(base, odd ? &map_q1 : &map_p1, &full[s], cy, cx - 1, (int)l);
-    tma_load_3d(base + kRingP1Bytes, odd ? &map_q2 : &map_p2, &full[s], cy - 4, cx, (int)(g.L + l));
-    tma_load_3d(base + kRingP1Bytes + kRingP2Bytes, odd ? &map_xb : &map_x, &full[s], cy, cx, (int)l);
+    tma_load_3d(base, &map_p1, &full[s], cy, cx - 1, (int)l);
+    tma_load_3d(base + kRingP1Bytes, &map_p2, &full[s], cy - 4, cx, (int)(g.L + l));
+    tma_load_3d(base + kRingP1Bytes + kRingP2Bytes, &map_x, &full[s], cy, cx, (int)l);
     if (CHECK) {
       if (q_boxes) {
         tma_load_3d(base + kRingP1Bytes + kRingP2Bytes + kRingXBytes, &map_q1, &full[s], cy, cx - 1, (int)l);
@@ -681,17 +274,17 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
   // launch may be scheduled right away: it blocks at the same point until THIS grid has completed and flushed.
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   asm volatile("griddepcontrol.wait;" ::: "memory");
-  if (mi.trace && threadIdx.x == 0) {
+  if (trace.buf && threadIdx.x == 0) {
     unsigned long long now;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-    atomicMin(mi.trace + 4 * mi.trace_slot, now);
+    atomicMin(trace.buf + 4 * trace.slot, now);
   }
   __syncthreads();
-  if (producer && !MULTI) {
+  if (producer) {
 #pragma unroll
     for (int s = 0; s < kRingStages; ++s) {
       const uint32_t t = blockIdx.x + s * gridDim.x;
-      if (t < n_tiles) issue(t, s, 0u);
+      if (t < n_tiles) issue(t, s);
     }
   }
 
@@ -716,70 +309,11 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
   const float sq_T = sqrtf(Tval), sq_S = sqrtf(Sval);
   const float inv_tau_sq = 1.f / (tau * sq_T), inv_sigma_sq = 1.f / (sigma * sq_S);
 
-  // ---- multi-iteration launches: work item k = (iteration, k-th tile of this CTA), issued by warp 31 -------------
-  const uint32_t n_work = MULTI ? ((n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x) * (uint32_t)mi.n_it : 0u;
-  uint32_t ki = 0, ki_it = 0, ki_tile = blockIdx.x;      // next work item to issue
-  // Whole warp 31.  The stage of work item ki must be free (bounded wait: the other warps need nothing from
-  // outside to leave it) and, from the second iteration on, the 3 x 3 tile neighbourhood must have finished the
-  // previous iteration: its outputs are this tile's TMA boxes, and it has read what this tile overwrites.
-  // Blocking mode is only used when this warp has nothing left to compute, so it cannot hold up a neighbour.
-  auto multi_issue = [&](bool blocking) -> bool {
-    if (!MULTI || ki >= n_work) return false;
-    const int si = ki % kRingStages;
-    if (ki_it > 0) {
-      // neighbourhood probe first: its loads overlap the wait for the stage below
-      uint32_t l, tx, ty;
-      decode(ki_tile, l, tx, ty);
-      const int lane = threadIdx.x & 31;
-      bool ready = true;
-      if (lane < 9 && lane != 4 && !(mi.debug & 2)) {
-        const int ntx = (int)tx + lane % 3 - 1, nty = (int)ty + lane / 3 - 1;
-        if (ntx >= 0 && ntx < (int)tiles_x && nty >= 0 && nty < (int)div_tiles_y.d) {
-          uint32_t slot = l * div_per_plane.d + (uint32_t)ntx * div_tiles_y.d + (uint32_t)nty;
-          if (mi.coarse) {
-            // owner CTA of the neighbour tile: position in the walk order (slabs walk the edge columns first)
-            const uint32_t wx = !SLAB ? (uint32_t)ntx
-                                : ((uint32_t)ntx == tiles_x - 1 ? right_pos
-                                                                : ((uint32_t)ntx < right_pos ? (uint32_t)ntx : (uint32_t)ntx + 1u));
-            slot = (l * div_per_plane.d + wx * div_tiles_y.d + (uint32_t)nty) % gridDim.x;
-            if (slot == blockIdx.x) slot = 0xffffffffu;        // own tiles: program order
-          }
-          if (slot != 0xffffffffu) ready = ring_count_wait(mi.done + slot, mi.base + ki_it, blocking, mi.error);
-        }
-      }
-      __syncwarp();
-      if (!__all_sync(0xffffffffu, ready)) return false;
-    }
-    if (ki >= (uint32_t)kRingStages) mbar_wait(&empty[si], ((ki - kRingStages) / kRingStages) & 1u);
-    // the neighbours' (and this CTA's own) generic-proxy stores -> our TMA reads
-    asm volatile("fence.proxy.async;" ::: "memory");
-    if ((threadIdx.x & 31) == 0) issue(ki_tile, si, ki_it);
-    ++ki;
-    ki_tile += gridDim.x;
-    if (ki_tile >= n_tiles) { ki_tile = blockIdx.x; ++ki_it; }
-    return true;
-  };
-
-  uint32_t k = 0, it = 0;
-  for (uint32_t tile = blockIdx.x;; tile += gridDim.x, ++k) {
-    if (tile >= n_tiles) {
-      if (!MULTI || ++it >= (uint32_t)mi.n_it) break;
-      tile = blockIdx.x;
-    }
+  for (uint32_t tile = blockIdx.x, k = 0; tile < n_tiles; tile += gridDim.x, ++k) {
     const int s = k % kRingStages;
     const uint32_t parity = (k / kRingStages) & 1u;
     uint32_t l, tx, ty;
     decode(tile, l, tx, ty);
-    // where this iteration writes, and (slabs) which halo slots / sequence numbers / edge counters it uses
-    float* __restrict__ xo_ptr = MULTI ? sel2(mi.x_io, (it + 1) & 1u) : x_out;
-    float* __restrict__ yo_ptr = MULTI ? sel2(mi.y_io, (it + 1) & 1u) : y_out;
-    unsigned y_wait_seq = h.y_wait_seq, x_wait_seq = h.x_wait_seq;
-    unsigned x_signal_seq = h.x_signal_seq, y_signal_seq = h.y_signal_seq;
-    if (SLAB && MULTI) { y_wait_seq += it; x_wait_seq += it; x_signal_seq += it; y_signal_seq += it; }
-    if (MULTI && col == kRingCols - 1) {
-      while (ki <= k) multi_issue(true);          // this work item must be on its way
-      if (ki == k + 1) multi_issue(false);        // prefetch the next one if its neighbourhood is ready
-    }
     const int cx = tx * kRingTX, cy = ty * kRingTY;
     unsigned char* base = smem + s * kRingStageBytes;
     float (*s_p1)[kRingRows] = reinterpret_cast<float (*)[kRingRows]>(base);
@@ -802,8 +336,8 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
     uint4 pre_a = make_uint4(0u, 0u, 0u, 0u), pre_b = make_uint4(0u, 0u, 0u, 0u);
     const uint4* pre_p = nullptr;
     if (SLAB) {
-      if (left_edge && y_wait_seq) pre_p = sel3(h.yl_ll, y_wait_seq % 3u) + halo_ll;
-      else if (right_edge) pre_p = sel2(h.xr_ll, x_wait_seq & 1u) + halo_ll;
+      if (left_edge && h.y_wait_seq) pre_p = sel3(h.yl_ll, h.y_wait_seq % 3u) + halo_ll;
+      else if (right_edge) pre_p = sel2(h.xr_ll, h.x_wait_seq & 1u) + halo_ll;
       if (pre_p) { ll_ld_line(pre_p, pre_a); ll_ld_line(pre_p + 1, pre_b); }
     }
     mbar_wait(&full[s], parity);
@@ -819,15 +353,15 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
       if (left_edge) {
         // y.gx of column -1: the left neighbour's previous iteration, row group by row group
         unsigned long long tw0 = 0;
-        if (mi.trace) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tw0));
-        if (y_wait_seq) ll_finish_load4(pre_p, y_wait_seq, pre_a, pre_b, a, h.error);
-        if (mi.trace) {
+        if (trace.buf) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tw0));
+        if (h.y_wait_seq) ll_finish_load4(pre_p, h.y_wait_seq, pre_a, pre_b, a, h.error);
+        if (trace.buf) {
           unsigned long long tw1;
           asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tw1));
-          atomicMax(mi.trace + 4 * mi.trace_slot + 2, tw1 - tw0);
+          atomicMax(trace.buf + 4 * trace.slot + 2, tw1 - tw0);
         }
         // (refresh) the column before it, read BEFORE this thread's x store lets the neighbour move on
-        if (CHECK && q_boxes && y_wait_seq > 1u) ll_read4(sel3(h.yl_ll, (y_wait_seq - 1u) % 3u) + halo_ll, qa_halo);
+        if (CHECK && q_boxes && h.y_wait_seq > 1u) ll_read4(sel3(h.yl_ll, (h.y_wait_seq - 1u) % 3u) + halo_ll, qa_halo);
       }
       VecIO<4>::ld(&s_p2[col][4 + r0], o);
       const float up = s_p2[col][4 + r0 - 1];
@@ -870,8 +404,8 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
       }
       VecIO<4>::st(&s_xn[col][r0], xn);
       if (col < kRingTX && r0 < kRingTY && gy < g.ny) {
-        VecIO<4>::st(xo_ptr + gy + gx * g.ny + plane_off, xn);
-        if (left_edge) ll_store4(sel2(h.x_out_ll, x_signal_seq & 1u) + halo_ll, xn, x_signal_seq);   // -> left neighbour
+        VecIO<4>::st(x_out + gy + gx * g.ny + plane_off, xn);
+        if (left_edge) ll_store4(sel2(h.x_out_ll, h.x_signal_seq & 1u) + halo_ll, xn, h.x_signal_seq);   // -> left neighbour
         if (CHECK) {
           // dual residual on the owned pixels: w^ = (x - x+)/(tau sqrt T) - sqrt T K^T y_prev,
           // diff = w^ + sqrt T K^T y
@@ -930,14 +464,14 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
       if (right_edge) {
         // x+ / x of column nx: the right neighbour's column 0 of THIS iteration and of the previous one
         unsigned long long tw0 = 0;
-        if (mi.trace) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tw0));
-        ll_finish_load4(pre_p, x_wait_seq, pre_a, pre_b, rn, h.error);
-        if (mi.trace) {
+        if (trace.buf) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tw0));
+        ll_finish_load4(pre_p, h.x_wait_seq, pre_a, pre_b, rn, h.error);
+        if (trace.buf) {
           unsigned long long tw1;
           asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tw1));
-          atomicMax(mi.trace + 4 * mi.trace_slot + 3, tw1 - tw0);
+          atomicMax(trace.buf + 4 * trace.slot + 3, tw1 - tw0);
         }
-        ll_read4(sel2(h.xr_ll, (x_wait_seq - 1u) & 1u) + halo_ll, ro);
+        ll_read4(sel2(h.xr_ll, (h.x_wait_seq - 1u) & 1u) + halo_ll, ro);
       } else {
         VecIO<4>::ld(&s_xn[col + 1][r0], rn);
         VecIO<4>::ld(&s_x[col + 1][r0], ro);
@@ -964,9 +498,9 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
       }
       if (f_simple) norm2_lanes<4, 2, true>(fn_f, arg, cf, tau_f);
       else norm2_lanes<4, 2, false>(fn_f, arg, cf, tau_f);
-      VecIO<4>::st(yo_ptr + idx, arg[0]);
-      VecIO<4>::st(yo_ptr + (size_t)g.L * g.nxny + idx, arg[1]);
-      if (right_edge) ll_store4(sel3(h.y_out_ll, y_signal_seq % 3u) + halo_ll, arg[0], y_signal_seq);   // -> right neighbour
+      VecIO<4>::st(y_out + idx, arg[0]);
+      VecIO<4>::st(y_out + (size_t)g.L * g.nxny + idx, arg[1]);
+      if (right_edge) ll_store4(sel3(h.y_out_ll, h.y_signal_seq % 3u) + halo_ll, arg[0], h.y_signal_seq);   // -> right neighbour
       if (CHECK) {
         // primal residual: z^ = (y - y+)/(sigma sqrt S) + sqrt S ((1+theta) K x+ - theta K x),
         // diff = z^ - sqrt S K x+
@@ -989,37 +523,18 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
     // this warp is done with stage s (operand boxes and x+ tile)
     __syncwarp();
     if ((threadIdx.x & 31) == 0) mbar_arrive(&empty[s]);
-    if (!MULTI && col == kRingCols - 1) {       // warp 31 refills the stage once every warp has left it
+    if (col == kRingCols - 1) {       // warp 31 refills the stage once every warp has left it
       const uint32_t next = tile + kRingStages * gridDim.x;
       if (next < n_tiles) {
         mbar_wait(&empty[s], parity);
-        if (producer) issue(next, s, 0u);
+        if (producer) issue(next, s);
       }
-    }
-    if (MULTI && col == kRingCols - 1) {
-      // First put the next work item into the stage that is being freed (its neighbourhood is probed while the
-      // other warps are still in phase B; multi_issue waits for the stage itself), THEN publish this tile's
-      // iteration count: the release at gpu scope is a full fence and must not sit in front of the TMA issue.
-      // Every warp has left work item k once `empty` completes, i.e. has issued its stores; they are ordered
-      // before the release through that mbarrier (cumulativity).
-      const bool issued = multi_issue(false);
-      mbar_wait(&empty[s], parity);
-      if (producer && !(mi.debug & 1)) {
-        if (!mi.coarse) {
-          unsigned* cnt = mi.done + (l * div_per_plane.d + tx * div_tiles_y.d + ty);
-          asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(cnt), "r"(mi.base + it + 1u) : "memory");
-        } else if (tile + gridDim.x >= n_tiles) {      // this CTA's last tile of the iteration
-          asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(mi.done + blockIdx.x), "r"(mi.base + it + 1u)
-                       : "memory");
-        }
-      }
-      if (!issued) multi_issue(false);
     }
   }
-  if (mi.trace && threadIdx.x == 0) {
+  if (trace.buf && threadIdx.x == 0) {
     unsigned long long now;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-    atomicMax(mi.trace + 4 * mi.trace_slot + 1, now);
+    atomicMax(trace.buf + 4 * trace.slot + 1, now);
   }
   if (CHECK) {
     block_sum2(acc_d0, acc_d1);
@@ -1069,8 +584,8 @@ RingTrace& ring_trace() {
   static RingTrace t;
   return t;
 }
-RingMulti ring_trace_next() {
-  RingMulti m;
+RingTraceSlot ring_trace_next() {
+  RingTraceSlot m;
   static const bool on = [] { const char* e = getenv("PB_RING_TRACE"); return e && atoi(e) != 0; }();
   if (!on) return m;
   RingTrace& t = ring_trace();
@@ -1080,8 +595,8 @@ RingMulti ring_trace_next() {
     for (unsigned i = 0; i < kRingTraceSlots; ++i) init[4 * i] = ~0ull;
     cudaMemcpy(t.buf, init.data(), init.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice);
   }
-  m.trace = t.buf;
-  m.trace_slot = t.next++ % kRingTraceSlots;
+  m.buf = t.buf;
+  m.slot = t.next++ % kRingTraceSlots;
   return m;
 }
 
@@ -1092,15 +607,13 @@ struct RingArgs {
   double* part_d = nullptr;
   double* part_p = nullptr;
   const RingHalo* halo = nullptr;      // slab mode
-  CUtensorMap mxb;                     // multi-iteration launches: x boxes over the second buffer set
-  const RingMulti* multi = nullptr;
   const RingFinish* finish = nullptr;  // residual-refresh launches that finalize the iteration in the kernel
 };
 
-template <int FN_G, int FN_F, bool CHECK, bool SLAB, bool MULTI = false>
+template <int FN_G, int FN_F, bool CHECK, bool SLAB>
 unsigned ring_launch_k(Context* ctx, const RingArgs& a, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf,
                        float Tval, float Sval, const PdhgState* st, float* x_out, float* y_out, bool dry_run) {
-  auto kernel = grad2d_iteration_ring_kernel<FN_G, FN_F, CHECK, SLAB, MULTI>;
+  auto kernel = grad2d_iteration_ring_kernel<FN_G, FN_F, CHECK, SLAB>;
   static bool configured = false, ok = false;
   if (!configured) {
     configured = true;
@@ -1115,48 +628,25 @@ unsigned ring_launch_k(Context* ctx, const RingArgs& a, const GradGeom& g, const
   if (dry_run) return grid;
   RingHalo h;
   if (SLAB) h = *a.halo;
-  if (MULTI) {
-    // the CTAs wait for each other's tiles: all of them have to be resident -> cooperative launch
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(kRingThreads);
-    cfg.dynamicSmemBytes = kRingSmemBytes;
-    cfg.stream = ctx->stream;
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeCooperative;
-    attr.val.cooperative = 1;
-    cfg.attrs = &attr;
-    cfg.numAttrs = 1;
-    const cudaError_t e = cudaLaunchKernelEx(
-        &cfg, kernel, a.mp1, a.mp2, a.mx, a.mf, a.mq1, a.mq2, g, pg, pf, Tval, Sval, st,
-        FastDiv((uint64_t)tiles_x * tiles_y), FastDiv(tiles_y), (uint32_t)n_tiles, a.ktyprev_zero, a.part_d, a.part_p,
-        x_out, y_out, tiles_x, h, a.mxb, *a.multi, RingFinish());
-    if (e != cudaSuccess) { cudaGetLastError(); return 0; }
-    return grid;
-  }
-  {
-    // programmatic stream serialization: see griddepcontrol in the kernel.  Measured (profiles/r02_scaling.md): the
-    // launch-to-launch gap drops from 3.8 to 1.8 us on one GPU, but on slabs the end-of-kernel flush of the
-    // NVLink halo stores dominates the gap and early-resident CTAs cost more than they hide (period 54.3 vs
-    // 52.9 us at 2 x 2048 columns), so slabs keep plain stream order.  PB_RING_PDL=0/1 overrides.
-    static const int pdl_env = [] { const char* e = getenv("PB_RING_PDL"); return e ? atoi(e) : -1; }();
-    const bool pdl = pdl_env >= 0 ? pdl_env != 0 : !SLAB;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(kRingThreads);
-    cfg.dynamicSmemBytes = kRingSmemBytes;
-    cfg.stream = ctx->stream;
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr.val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = &attr;
-    cfg.numAttrs = pdl ? 1 : 0;
-    const cudaError_t e = cudaLaunchKernelEx(
-        &cfg, kernel, a.mp1, a.mp2, a.mx, a.mf, a.mq1, a.mq2, g, pg, pf, Tval, Sval, st,
-        FastDiv((uint64_t)tiles_x * tiles_y), FastDiv(tiles_y), (uint32_t)n_tiles, a.ktyprev_zero, a.part_d, a.part_p,
-        x_out, y_out, tiles_x, h, a.mx, ring_trace_next(), (CHECK && a.finish) ? *a.finish : RingFinish());
-    if (e != cudaSuccess) { cudaGetLastError(); return 0; }
-  }
+  // programmatic stream serialization: see griddepcontrol in the kernel.  Measured (profiles/r02_scaling.md): the
+  // launch-to-launch gap drops from 3.8 to 1.8 us on one GPU, but on slabs the end-of-kernel flush of the
+  // NVLink halo stores dominates the gap and early-resident CTAs cost more than they hide (period 54.3 vs
+  // 52.9 us at 2 x 2048 columns), so slabs keep plain stream order.
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid);
+  cfg.blockDim = dim3(kRingThreads);
+  cfg.dynamicSmemBytes = kRingSmemBytes;
+  cfg.stream = ctx->stream;
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr.val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = &attr;
+  cfg.numAttrs = SLAB ? 0 : 1;
+  const cudaError_t e = cudaLaunchKernelEx(
+      &cfg, kernel, a.mp1, a.mp2, a.mx, a.mf, a.mq1, a.mq2, g, pg, pf, Tval, Sval, st,
+      FastDiv((uint64_t)tiles_x * tiles_y), FastDiv(tiles_y), (uint32_t)n_tiles, a.ktyprev_zero, a.part_d, a.part_p,
+      x_out, y_out, tiles_x, h, ring_trace_next(), (CHECK && a.finish) ? *a.finish : RingFinish());
+  if (e != cudaSuccess) { cudaGetLastError(); return 0; }
   return grid;
 }
 
@@ -1207,8 +697,6 @@ inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
 
 }  // namespace
 
-static int tile_mode();
-
 // copies the trace (up to n launches x 4 values) to the host; returns the number of launches recorded so far
 unsigned tile_ring_trace_read(unsigned long long* h_out, unsigned n) {
   RingTrace& t = ring_trace();
@@ -1217,46 +705,6 @@ unsigned tile_ring_trace_read(unsigned long long* h_out, unsigned n) {
   const unsigned k = std::min(std::min(n, t.next), kRingTraceSlots);
   if (k) cudaMemcpy(h_out, t.buf, (size_t)k * 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
   return t.next;
-}
-
-// ---- several non-refresh iterations in one launch (experimental, PB_RING_ITERS > 1) ----------------------------
-unsigned tile_ring_tile_count(const StencilPlan& plan) {
-  const GradGeom& g = plan.geom;
-  const uint64_t n = (uint64_t)((g.nx + kRingTX - 1) / kRingTX) * ((g.ny + kRingTY - 1) / kRingTY) * g.L;
-  return n < (1ull << 31) ? (unsigned)n : 0u;
-}
-
-// Iterations it = 0 .. n_it-1: even ones read (x_a, y_a) and write (x_b, y_b), odd ones the other way round.
-// Returns the number of CTAs, 0 if the launch was not possible (the caller then runs single iterations).
-unsigned tile_multi_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
-                                     float* x_a, float* y_a, float* x_b, float* y_b, ScaleRef T, ScaleRef S,
-                                     const PdhgState* st, const RingMulti& multi, const RingHalo* halo) {
-  if (tile_mode() != 2 || multi.n_it < 2 || !multi.done) return 0;
-  const GradGeom& g = plan.geom;
-  RingArgs a;
-  a.halo = halo;
-  a.multi = &multi;
-  if (!tensor_map_for(y_a, g.ny, g.nx, 2 * g.L, kRingRows, kRingCols + 1, a.mp1)) return 0;
-  if (!tensor_map_for(y_a, g.ny, g.nx, 2 * g.L, kRingR2, kRingCols, a.mp2)) return 0;
-  if (!tensor_map_for(x_a, g.ny, g.nx, g.L, kRingRows, kRingCols, a.mx)) return 0;
-  if (!tensor_map_for(y_b, g.ny, g.nx, 2 * g.L, kRingRows, kRingCols + 1, a.mq1)) return 0;
-  if (!tensor_map_for(y_b, g.ny, g.nx, 2 * g.L, kRingR2, kRingCols, a.mq2)) return 0;
-  if (!tensor_map_for(x_b, g.ny, g.nx, g.L, kRingRows, kRingCols, a.mxb)) return 0;
-  const float* f = pg.coeffs.ptr[1] ? pg.coeffs.ptr[1] : x_a;      // unused when b is a scalar
-  if (!tensor_map_for(f, g.ny, g.nx, g.L, kRingRows, kRingCols, a.mf)) return 0;
-#define PB_ARGS ctx, a, g, pg, pf, T.val, S.val, st, x_b, y_b, false
-  unsigned grid;
-  if (pg.fn == PB_FUN_SQUARE && pf.fn == PB_FUN_IND_LEQ0)
-    grid = halo ? ring_launch_k<PB_FUN_SQUARE, PB_FUN_IND_LEQ0, false, true, true>(PB_ARGS)
-                : ring_launch_k<PB_FUN_SQUARE, PB_FUN_IND_LEQ0, false, false, true>(PB_ARGS);
-  else
-    grid = halo ? ring_launch_k<-1, -1, false, true, true>(PB_ARGS) : ring_launch_k<-1, -1, false, false, true>(PB_ARGS);
-#undef PB_ARGS
-  if (grid) {
-    PB_CHECK_LAUNCH();
-    ctx->launches++;
-  }
-  return grid;
 }
 
 // Can the whole iteration run as one tiled pass?  K = one planar BlockGradient2D (no identity rows),
@@ -1284,68 +732,35 @@ bool tile_iteration_supported(const StencilPlan& plan, const std::vector<ProxDes
   return true;
 }
 
-static int tile_mode();
-bool tile_ring_available() { return tile_mode() == 2 && encode_tiled_fn() != nullptr; }
-
-static int tile_mode() {
-  // PB_TILE_MODE: 2 (default) persistent TMA ring, 1 one-shot TMA tiles, 0 plain loads (A/B experiments)
-  static const int mode = [] { const char* e = getenv("PB_TILE_MODE"); return e ? atoi(e) : 2; }();
-  return mode;
+bool tile_ring_available(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf, bool slab) {
+  const RingHalo halo;                 // selects the slab variants; a dry run reads nothing from it
+  for (const bool check : {false, true})
+    if (!ring_launch(ctx, plan.geom, pg, pf, nullptr, nullptr, nullptr, 0.f, 0.f, nullptr, check, true, nullptr,
+                     nullptr, nullptr, nullptr, true, slab ? &halo : nullptr))
+      return false;
+  return true;
 }
 
-// Residual-refresh iteration as one tiled pass (persistent ring only).  Returns the number of partial
-// pairs written to EACH of part_d / part_p, or 0 when the caller has to run the two-pass kernels.
+// Residual-refresh iteration as one tiled pass.  Returns the number of partial pairs written to EACH of part_d /
+// part_p.
 unsigned tile_check_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
                                      const float* x, const float* y, const float* y_prev, ScaleRef T, ScaleRef S,
                                      const PdhgState* st, bool ktyprev_zero, double* part_d, double* part_p,
-                                     float* x_out, float* y_out, bool dry_run, const RingHalo* halo,
-                                     const RingFinish* finish) {
-  if (tile_mode() != 2) return 0;
+                                     float* x_out, float* y_out, const RingHalo* halo, const RingFinish* finish) {
   const unsigned n = ring_launch(ctx, plan.geom, pg, pf, x, y, y_prev, T.val, S.val, st, true, ktyprev_zero, part_d,
-                                 part_p, x_out, y_out, dry_run, halo, finish);
-  if (n && !dry_run) {
-    PB_CHECK_LAUNCH();
-    ctx->launches++;
-  }
+                                 part_p, x_out, y_out, false, halo, finish);
+  if (!n) fail(PB_ERR_CUDA, "the one-pass ring kernel could not be launched");
+  PB_CHECK_LAUNCH();
+  ctx->launches++;
   return n;
 }
 
 void tile_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
                            const float* x, const float* y, ScaleRef T, ScaleRef S, const PdhgState* st,
                            float* x_out, float* y_out, const RingHalo* halo) {
-  const GradGeom& g = plan.geom;
-  if (halo) {
-    // slab mode: only the ring kernel speaks the halo protocol (tile_ring_available() was checked at Initialize)
-    if (!ring_launch(ctx, g, pg, pf, x, y, nullptr, T.val, S.val, st, false, true, nullptr, nullptr, x_out, y_out,
-                     false, halo))
-      fail(PB_ERR_CUDA, "slab decomposition: the one-pass ring kernel could not be launched");
-    PB_CHECK_LAUNCH();
-    ctx->launches++;
-    return;
-  }
-  // tile shape: long columns segments keep DRAM pages busy, wide tiles keep the halo share low;
-  // PB_TILE_SHAPE (0..3) overrides the default for experiments
-  static const int shape = [] { const char* e = getenv("PB_TILE_SHAPE"); return e ? atoi(e) : 0; }();
-  const int mode = tile_mode();
-  if (mode == 2 && ring_launch(ctx, g, pg, pf, x, y, nullptr, T.val, S.val, st, false, true, nullptr, nullptr, x_out,
-                               y_out, false, nullptr)) {
-    PB_CHECK_LAUNCH();
-    ctx->launches++;
-    return;
-  }
-  if (mode >= 1 && tma_launch(ctx, g, pg, pf, x, y, T.val, S.val, st, x_out, y_out)) {
-    PB_CHECK_LAUNCH();
-    ctx->launches++;
-    return;
-  }
-#define PB_ARGS ctx, g, pg, pf, x, y, T.val, S.val, st, x_out, y_out
-  switch (shape) {
-    case 1: tile_launch_g<16, 256>(PB_ARGS); break;
-    case 2: tile_launch_g<8, 512>(PB_ARGS); break;
-    case 3: tile_launch_g<16, 128>(PB_ARGS); break;
-    default: tile_launch_g<32, 128>(PB_ARGS); break;
-  }
-#undef PB_ARGS
+  if (!ring_launch(ctx, plan.geom, pg, pf, x, y, nullptr, T.val, S.val, st, false, true, nullptr, nullptr, x_out,
+                   y_out, false, halo))
+    fail(PB_ERR_CUDA, "the one-pass ring kernel could not be launched");
   PB_CHECK_LAUNCH();
   ctx->launches++;
 }

@@ -16,10 +16,8 @@ There are only two slots per direction (index = sequence number & 1); a slot is 
 segment j of it and reads segments j and j+1 (its halo rows belong to the next tile).  The model runs the ranks' tiles under a
 random scheduler and checks that every read returns the column of exactly the expected (rank, iteration) -- i.e.
 that no slot is overwritten before its last reader is done and no reader runs ahead of its writer -- and that the
-schedule never deadlocks.  Two local orderings are modelled:
-  * one launch per iteration (what ships): a rank's iteration it+1 starts after all its tiles of iteration it;
-  * several iterations per launch (experimental RingMulti): tile j of iteration it+1 only needs tiles j-1, j, j+1
-    of both groups of iteration it on its own rank."""
+schedule never deadlocks.  Locally, one launch runs per iteration: a rank's iteration it+1 starts after all its
+tiles of iteration it."""
 import random
 
 import pytest
@@ -38,7 +36,7 @@ class Rank:
         self.edge_count = {}
 
 
-def run_model(world, n_iters, n_tiles, multi, check_every, seed):
+def run_model(world, n_iters, n_tiles, check_every, seed):
     rng = random.Random(seed)
     ranks = [Rank(r, world, n_tiles) for r in range(world)]
     # pending work: (rank, group, tile) -> next iteration (1-based)
@@ -54,20 +52,15 @@ def run_model(world, n_iters, n_tiles, multi, check_every, seed):
                     if it > n_iters:
                         continue
                     # local ordering
-                    if multi:
-                        nb = [t for t in (j - 1, j, j + 1) if 0 <= t < n_tiles]
-                        if any(rk.done[g][t] < it - 1 for g in ("L", "R") for t in nb):
-                            continue
-                    else:
-                        if any(rk.done[g][t] < it - 1 for g in ("L", "R") for t in range(n_tiles)):
-                            continue
+                    if any(rk.done[g][t] < it - 1 for g in ("L", "R") for t in range(n_tiles)):
+                        continue
                     # halo waits (iteration 1 = the two-pass iteration 0 of the solver: K^T y := 0, no y halo)
                     if grp == "L" and rk.has_left and it > 1 and rk.y_flag < it - 1:
                         continue
                     if grp == "R" and rk.has_right and rk.x_flag < it:
                         continue
                     enabled.append((rk, grp, j, it))
-        assert enabled, f"deadlock after {completed} of {total} tile steps (world={world}, multi={multi}, seed={seed})"
+        assert enabled, f"deadlock after {completed} of {total} tile steps (world={world}, seed={seed})"
         rk, grp, j, it = rng.choice(enabled)
         refresh = check_every and it % check_every == 0
         segs = [t for t in (j, j + 1) if t < n_tiles]
@@ -100,11 +93,10 @@ def run_model(world, n_iters, n_tiles, multi, check_every, seed):
     return steps
 
 
-@pytest.mark.parametrize("multi", [False, True])
 @pytest.mark.parametrize("world", [2, 3, 4])
-def test_two_slot_halo_protocol_is_safe_and_live(world, multi):
+def test_two_slot_halo_protocol_is_safe_and_live(world):
     for seed in range(40):
-        run_model(world, n_iters=7, n_tiles=3, multi=multi, check_every=3, seed=seed)
+        run_model(world, n_iters=7, n_tiles=3, check_every=3, seed=seed)
 
 
 # Sanity of the model itself: if a group published its sequence number after its FIRST tile, a neighbour could
@@ -172,7 +164,7 @@ class LLRank:
         self.done = {"L": [0] * n_tiles, "R": [0] * n_tiles}
 
 
-def run_model_ll(world, n_iters, n_tiles, multi, check_every, seed, y_slots=3):
+def run_model_ll(world, n_iters, n_tiles, check_every, seed, y_slots=3):
     rng = random.Random(seed)
     ranks = [LLRank(r, world, n_tiles, y_slots) for r in range(world)]
     total = world * 2 * n_tiles * n_iters
@@ -185,11 +177,7 @@ def run_model_ll(world, n_iters, n_tiles, multi, check_every, seed, y_slots=3):
                     it = rk.done[grp][j] + 1
                     if it > n_iters:
                         continue
-                    if multi:
-                        nb = [t for t in (j - 1, j, j + 1) if 0 <= t < n_tiles]
-                        if any(rk.done[g][t] < it - 1 for g in ("L", "R") for t in nb):
-                            continue
-                    elif any(rk.done[g][t] < it - 1 for g in ("L", "R") for t in range(n_tiles)):
+                    if any(rk.done[g][t] < it - 1 for g in ("L", "R") for t in range(n_tiles)):
                         continue
                     segs = [t for t in (j, j + 1) if t < n_tiles]
                     # the waits: tags in the data (iteration 1 = the two-pass iteration 0 of the solver, no y halo)
@@ -216,15 +204,14 @@ def run_model_ll(world, n_iters, n_tiles, multi, check_every, seed, y_slots=3):
     return "ok"
 
 
-@pytest.mark.parametrize("multi", [False, True])
 @pytest.mark.parametrize("world", [2, 3, 4])
-def test_flag_in_data_halo_protocol_is_safe_and_live(world, multi):
+def test_flag_in_data_halo_protocol_is_safe_and_live(world):
     for seed in range(60):
-        assert run_model_ll(world, n_iters=8, n_tiles=3, multi=multi, check_every=3, seed=seed) == "ok"
-        assert run_model_ll(world, n_iters=8, n_tiles=4, multi=multi, check_every=1, seed=seed) == "ok"
+        assert run_model_ll(world, n_iters=8, n_tiles=3, check_every=3, seed=seed) == "ok"
+        assert run_model_ll(world, n_iters=8, n_tiles=4, check_every=1, seed=seed) == "ok"
 
 
 def test_flag_in_data_model_needs_the_third_y_slot():
-    outcomes = {run_model_ll(3, n_iters=8, n_tiles=3, multi=False, check_every=1, seed=s, y_slots=2) for s in range(300)}
+    outcomes = {run_model_ll(3, n_iters=8, n_tiles=3, check_every=1, seed=s, y_slots=2) for s in range(300)}
     assert "stale previous y halo" in outcomes, "two y slots should be caught as unsafe under refresh reads"
     assert "deadlock" not in outcomes
