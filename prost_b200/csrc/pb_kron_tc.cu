@@ -22,7 +22,6 @@
 // * one persistent CTA per SM (16 worker warps + one MMA warp), tiles of 128 points round-robin.
 #include <algorithm>
 #include <cstdint>
-#include <cstdlib>
 #include <cstring>
 #include <vector>
 
@@ -126,10 +125,8 @@ struct KronTcArgs {
   uint32_t n_out, n_in, n_out_pad, k_pad;
   size_t d;
   uint32_t tmem_cols;
-  uint32_t lag;               // 1 or 2: iterations between writing a tile's operands and draining its accumulator
   uint32_t tma_out;           // kron(K, I): results leave as one TMA tensor store per warp (32 points x its columns)
   uint32_t stage_out;         // kron(I, K): results leave through a shared-memory tile (n_out % 4 == 0, n_out <= 64)
-  uint32_t debug;             // timing experiments (results unusable): 1 no MMAs, 2 no result stores, 4 no X loads, 8 no split / smem stores
   const int* skip;
 };
 
@@ -148,9 +145,9 @@ struct KronTcArgs {
 //
 // Roles: 16 worker warps (load -> split -> shared memory; TMEM -> HBM) and one MMA warp.  Per operand / accumulator
 // buffer b (two of each): workers arrive on full[b] after writing tile j's operands, the MMA warp waits for it, issues
-// the 3 * k_pad / 8 MMAs and commits them to done[accumulator]; every worker waits for that before it drains tile j, which
-// is also what allows it to overwrite buffer b with tile j + 2.  No CTA-wide barrier inside the loop.
-template <bool IDFIRST, bool SET, int DEPTH>
+// the 3 * k_pad / 8 MMAs and commits them to done[b]; every worker waits for that before it drains tile j, which is
+// also what allows it to overwrite buffer b with tile j + 2.  No CTA-wide barrier inside the loop.
+template <bool IDFIRST, bool SET>
 __global__ void __launch_bounds__(kTcThreads, 1) kron_tc_kernel(const KronTcArgs a,
                                                                 const __grid_constant__ CUtensorMap out_map) {
   if (a.skip && *a.skip) return;
@@ -165,9 +162,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) kron_tc_kernel(const KronTcArgs
   uint8_t* const f_hi = tc_smem + 4 * xb;
   uint8_t* const f_lo = f_hi + fb;
   uint64_t* const full = reinterpret_cast<uint64_t*>(f_lo + fb);
-  uint64_t* const done = full + 2;                        // one per accumulator (lag + 1 of them)
+  uint64_t* const done = full + 2;                        // one per accumulator
   uint32_t* const tmem_slot = reinterpret_cast<uint32_t*>(full + 6);
-  const uint32_t lag = a.lag, nacc = a.lag + 1;           // tiles between a tile's MMAs and its drain; accumulators
 
   for (uint32_t i = tid; i < fb / 16; i += kTcThreads) {
     reinterpret_cast<uint4*>(f_hi)[i] = __ldg(a.f_hi + i);
@@ -178,7 +174,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) kron_tc_kernel(const KronTcArgs
     tc_mbar_init(&full[1], kTcWorkerWarps);
     tc_mbar_init(&done[0], 1);
     tc_mbar_init(&done[1], 1);
-    tc_mbar_init(&done[2], 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == 0) {
@@ -209,15 +204,14 @@ __global__ void __launch_bounds__(kTcThreads, 1) kron_tc_kernel(const KronTcArgs
       if (lane == 0) {
         const uint32_t xh = tc_smem_u32(x_hi0 + buf * 2 * xb);
         const uint64_t da_hi0 = tc_smem_desc(xh, 128u, sbo), da_lo0 = tc_smem_desc(xh + xb, 128u, sbo);
-        const uint32_t acc = j % nacc;
-        const uint32_t dst = tmem + acc * a.n_out_pad;
-        for (uint32_t ko = 0; ko < ko_count && !(a.debug & 1u); ++ko) {
+        const uint32_t dst = tmem + buf * a.n_out_pad;
+        for (uint32_t ko = 0; ko < ko_count; ++ko) {
           const uint64_t step = ko * 16u;                      // 256 bytes per k-step, in 16-byte units
           tc_mma_tf32(dst, da_hi0 + step, db_hi0 + step, idesc, ko > 0);
           tc_mma_tf32(dst, da_lo0 + step, db_hi0 + step, idesc, 1u);
           tc_mma_tf32(dst, da_hi0 + step, db_lo0 + step, idesc, 1u);
         }
-        tc_commit(&done[j % nacc]);
+        tc_commit(&done[buf]);
       }
       __syncwarp();
     }
@@ -244,7 +238,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) kron_tc_kernel(const KronTcArgs
       ukn[it] = (ok && 4 * kc < a.n_in) ? min(4u, a.n_in - 4 * kc) : 0u;
       gsrc[it] = IDFIRST ? a.rhs + (size_t)pt * a.n_in + 4 * kc : a.rhs + (size_t)(4 * kc) * a.d + pt;
     }
-    float4 stage[DEPTH][kTcUnits];
+    float4 stage[kTcUnits];
 
     const size_t dd = a.d, dd2 = 2 * dd, dd3 = 3 * dd;
     auto load_tile = [&](float4 (&st)[kTcUnits], size_t t) {
@@ -254,7 +248,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) kron_tc_kernel(const KronTcArgs
 #pragma unroll
       for (uint32_t it = 0; it < kTcUnits; ++it) {
         st[it] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (upt[it] == 0xffffffffu || (a.debug & 4u)) continue;
+        if (upt[it] == 0xffffffffu) continue;
         const float* src = gsrc[it] + base;
         if (IDFIRST) {
           if (ukn[it] > 0 && (whole || p0 + upt[it] < dd)) st[it] = __ldcs(reinterpret_cast<const float4*>(src));
@@ -276,7 +270,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) kron_tc_kernel(const KronTcArgs
       uint8_t* const lo = hi + xb;
 #pragma unroll
       for (uint32_t it = 0; it < kTcUnits; ++it) {
-        if (upt[it] != 0xffffffffu && !(a.debug & 8u)) {
+        if (upt[it] != 0xffffffffu) {
           const float4 v = st[it];
           float4 h, l;
           h.x = tc_round_tf32(v.x); h.y = tc_round_tf32(v.y); h.z = tc_round_tf32(v.z); h.w = tc_round_tf32(v.w);
@@ -330,12 +324,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) kron_tc_kernel(const KronTcArgs
         }
       }
     };
-    // accumulator of tile t (TMEM half `buf`) -> HBM
+    // accumulator of tile t (TMEM half `acc`) -> HBM
     auto drain = [&](size_t t, uint32_t acc, uint32_t parity) {
       tc_mbar_wait(&done[acc], parity);
       tc_fence_after();
       const size_t p0 = t * kTcPoints;
-      const bool live = p0 + row < dd && !(a.debug & 2u);
+      const bool live = p0 + row < dd;
       const uint32_t taddr = tmem + ((32u * lb) << 16) + acc * a.n_out_pad;
       if (!IDFIRST && a.tma_out) {
         // kron(K, I) through TMA: the warp's 32 points x cols accumulators go to its own [cols][32] shared-memory tile
@@ -368,7 +362,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) kron_tc_kernel(const KronTcArgs
         tc_fence_before();
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncwarp();
-        if (lane == 0 && !(a.debug & 2u)) {
+        if (lane == 0) {
           const uint64_t map = reinterpret_cast<uint64_t>(&out_map);
           const uint32_t src = tc_smem_u32(tile);
           const int x = (int)(p0 + 32 * lb), y = (int)c_begin;
@@ -434,50 +428,39 @@ __global__ void __launch_bounds__(kTcThreads, 1) kron_tc_kernel(const KronTcArgs
         const size_t rows_valid = min((size_t)kTcPoints, dd - p0);
         const uint32_t units = (uint32_t)rows_valid * q_per_row;
         float4* const out = reinterpret_cast<float4*>(a.res + p0 * a.n_out);
-        if (!(a.debug & 2u)) {
 #pragma unroll
-          for (uint32_t it = 0; it < kTcUnits; ++it) {
-            const uint32_t u = it * kTcWorkers + tid;
-            if (u < units) {
-              float4 o = *reinterpret_cast<const float4*>(stg + cp_soff[it]);
-              if (!SET) { const float4 r = out[u]; o.x += r.x; o.y += r.y; o.z += r.z; o.w += r.w; }
-              __stcs(out + u, o);
-            }
+        for (uint32_t it = 0; it < kTcUnits; ++it) {
+          const uint32_t u = it * kTcWorkers + tid;
+          if (u < units) {
+            float4 o = *reinterpret_cast<const float4*>(stg + cp_soff[it]);
+            if (!SET) { const float4 r = out[u]; o.x += r.x; o.y += r.y; o.z += r.z; o.w += r.w; }
+            __stcs(out + u, o);
           }
         }
         tc_worker_barrier();                                           // before the next tile overwrites it
       }
     };
 
-#pragma unroll
-    for (int s = 0; s < DEPTH; ++s)
-      if (blockIdx.x + s * stride < tiles) load_tile(stage[s], blockIdx.x + s * stride);
-    // Tile j of this CTA: operand buffer j % 2, accumulator j % nacc; it is drained `lag` iterations after its
-    // operands were written, so that its MMAs (and their completion latency) are off the workers' critical path.
-    size_t t = blockIdx.x;
+    if (blockIdx.x < tiles) load_tile(stage, blockIdx.x);
+    // Tile j of this CTA (tile t = blockIdx.x + j * stride): operand buffer and accumulator j % 2.  It is drained in
+    // iteration j + 1, after tile j + 1's operands were written, so that its MMAs (and their completion latency) are
+    // off the workers' critical path; the iteration past the last tile only drains.
     uint32_t j = 0;
-    auto drain_seq = [&](uint32_t jt) { drain(blockIdx.x + (size_t)jt * stride, jt % nacc, (jt / nacc) & 1u); };
-    while (t < tiles) {
-#pragma unroll
-      for (int s = 0; s < DEPTH; ++s) {
-        if (t < tiles) {
-          const uint32_t buf = j & 1;
-          // operand buffer `buf` was last read by the MMAs of tile j - 2.  lag 1: this thread waited for them when
-          // it drained tile j - 2 in the previous iteration; lag 2: wait here (they finished long ago)
-          if (lag == 2 && j >= 2) tc_mbar_wait(&done[(j - 2) % nacc], ((j - 2) / nacc) & 1u);
-          store_tile(stage[s], buf);
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) tc_mbar_arrive(&full[buf]);
-          if (t + DEPTH * stride < tiles) load_tile(stage[s], t + DEPTH * stride);
-          if (j >= lag) drain_seq(j - lag);
-          t += stride;
-          ++j;
-        }
+    for (size_t t = blockIdx.x;; t += stride, ++j) {
+      if (t < tiles) {
+        const uint32_t buf = j & 1;
+        // operand buffer `buf` was last read by the MMAs of tile j - 2: this thread waited for them when it drained
+        // tile j - 2 in the previous iteration
+        store_tile(stage, buf);
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) tc_mbar_arrive(&full[buf]);
+        if (t + stride < tiles) load_tile(stage, t + stride);
       }
+      if (j >= 1) drain(t - stride, (j - 1) & 1, ((j - 1) >> 1) & 1);
+      if (t >= tiles) break;
     }
-    for (uint32_t jt = j >= lag ? j - lag : 0; jt < j; ++jt) drain_seq(jt);
     if (!IDFIRST && a.tma_out && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
   }
   tc_fence_before();
@@ -498,17 +481,11 @@ inline float host_round_tf32(float x) {     // cvt.rna.tf32.f32: nearest, ties a
   return r;
 }
 
-int tc_env(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-
 }  // namespace
 
 bool KronTensorCore::supported(bool id_first, uint32_t n_out, uint32_t n_in, size_t d, const float* res,
                                const float* rhs) {
-  static const int enabled = tc_env("PB_KRON_TC", 1);
-  if (!enabled || d == 0 || n_out == 0 || n_in == 0) return false;
+  if (d == 0 || n_out == 0 || n_in == 0) return false;
   const uint32_t k_pad = (n_in + 7u) & ~7u, n_pad = (n_out + 15u) & ~15u;
   if (k_pad > kTcMaxIn || n_pad > kTcMaxOut) return false;
   if ((size_t)n_in * n_out < 512) return false;            // small factors: the fp32 kernels are at the HBM bound
@@ -534,10 +511,10 @@ static TcEncodeTiledFn tc_encode_fn() {
   }();
   return fn;
 }
-// res of kron(K, I) as a 2-D tensor [n_out rows][d points]; box = 32 points x the columns of one warp
+// res of kron(K, I) as a 2-D tensor [n_out rows][d points]; box = 32 points x the columns of one warp.  false: the
+// results leave through per-thread stores instead
 static bool tc_out_map(float* res, size_t d, uint32_t n_out, uint32_t cols, CUtensorMap& m) {
-  static const int enabled = tc_env("PB_KRON_TC_TMA_OUT", 1);
-  if (!enabled || d % 4 != 0 || (reinterpret_cast<uintptr_t>(res) & 15u) != 0 || cols > 256 || d >= (1ull << 31)) return false;
+  if (d % 4 != 0 || (reinterpret_cast<uintptr_t>(res) & 15u) != 0 || cols > 256 || d >= (1ull << 31)) return false;
   TcEncodeTiledFn enc = tc_encode_fn();
   if (!enc) return false;
   const cuuint64_t dims[2] = {(cuuint64_t)d, (cuuint64_t)n_out};
@@ -575,7 +552,6 @@ void KronTensorCore::pack(Context* ctx, const float* k, uint32_t n_out, uint32_t
 
 void KronTensorCore::launch(Context* ctx, bool id_first, const Packed& f, float* res, const float* rhs, uint32_t n_out,
                             uint32_t n_in, size_t d, bool set) {
-  static const int depth = tc_env("PB_KRON_TC_DEPTH", 1);
   KronTcArgs a;
   a.res = res;
   a.rhs = rhs;
@@ -586,13 +562,9 @@ void KronTensorCore::launch(Context* ctx, bool id_first, const Packed& f, float*
   a.n_out_pad = f.n_pad;
   a.k_pad = f.k_pad;
   a.d = d;
-  static const int lag = tc_env("PB_KRON_TC_LAG", 1);          // 2 measures the same (profiles/r02_operators.md)
-  a.lag = (lag >= 2 && 3 * f.n_pad <= 512) ? 2u : 1u;        // 512 TMEM columns per SM
-  uint32_t cols = 32;
-  while (cols < (a.lag + 1) * f.n_pad) cols *= 2;
+  uint32_t cols = 32;                                        // two accumulators, a power of two >= 32 columns
+  while (cols < 2 * f.n_pad) cols *= 2;
   a.tmem_cols = cols;
-  static const int debug = tc_env("PB_KRON_TC_DEBUG", 0);
-  a.debug = (uint32_t)debug;
   a.skip = ctx->skip_flag;
   const size_t smem = smem_bytes(id_first, n_out, f.n_pad, f.k_pad);
   a.stage_out = stages_output(id_first, n_out) ? 1u : 0u;
@@ -601,15 +573,13 @@ void KronTensorCore::launch(Context* ctx, bool id_first, const Packed& f, float*
   a.tma_out = (!id_first && tc_out_map(res, d, n_out, f.n_pad / 4, out_map)) ? 1u : 0u;
   const size_t tiles = (d + kTcPoints - 1) / kTcPoints;
   const unsigned grid = (unsigned)std::min<size_t>(tiles, (size_t)ctx->num_sms);
-#define PB_TC(I, S, D)                                                                                       \
+#define PB_TC(I, S)                                                                                          \
   do {                                                                                                       \
-    PB_CUDA(cudaFuncSetAttribute(kron_tc_kernel<I, S, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    kron_tc_kernel<I, S, D><<<grid, kTcThreads, smem, ctx->stream>>>(a, out_map);                            \
+    PB_CUDA(cudaFuncSetAttribute(kron_tc_kernel<I, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    kron_tc_kernel<I, S><<<grid, kTcThreads, smem, ctx->stream>>>(a, out_map);                               \
   } while (0)
-#define PB_TC_D(I, S) do { if (depth <= 1) PB_TC(I, S, 1); else PB_TC(I, S, 2); } while (0)
-  if (id_first) { if (set) PB_TC_D(true, true); else PB_TC_D(true, false); }
-  else { if (set) PB_TC_D(false, true); else PB_TC_D(false, false); }
-#undef PB_TC_D
+  if (id_first) { if (set) PB_TC(true, true); else PB_TC(true, false); }
+  else { if (set) PB_TC(false, true); else PB_TC(false, false); }
 #undef PB_TC
 }
 

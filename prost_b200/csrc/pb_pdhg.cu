@@ -395,11 +395,8 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
              tile_iteration_supported(stencil_, g_descs_, f_descs_, problem_->right_ref(), problem_->left_ref()) &&
              tile_ring_available(ctx_, stencil_, g_descs_[0], f_descs_[0], comm_ != nullptr);
   // slabs: the one-pass kernel stores its edge columns straight into the neighbours' memory, so it
-  // needs the peer-to-peer halo blocks (PB_SLAB_TILE=0: two passes)
-  if (comm_) {
-    static const bool slab_tile = [] { const char* e = getenv("PB_SLAB_TILE"); return !e || atoi(e) != 0; }();
-    tile_ok_ = tile_ok_ && slab_tile && stencil_.geom.nx >= 2;
-  }
+  // needs the peer-to-peer halo blocks
+  if (comm_) tile_ok_ = tile_ok_ && stencil_.geom.nx >= 2;
   tile_iterations_ = 0;
   if (comm_) {
     // the halo protocol lives in the specialised stencil passes: one planar gradient operator

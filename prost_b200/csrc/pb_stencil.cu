@@ -68,12 +68,7 @@ static inline unsigned grid_threads(size_t threads) {
   return (unsigned)((threads + kStencilBlock - 1) / kStencilBlock);
 }
 
-// per-pixel label groups: operands staged through shared memory (pb_stencil_staged.cuh); PB_STAGED=0 selects
-// the plain register kernels (A/B experiments)
-static inline bool staged_enabled() {
-  static const bool on = [] { const char* e = getenv("PB_STAGED"); return !e || atoi(e) != 0; }();
-  return on;
-}
+// per-pixel label groups: operands staged through shared memory (pb_stencil_staged.cuh)
 static inline unsigned staged_grid(size_t threads) {
   return (unsigned)((threads + kStagedBlock - 1) / kStagedBlock);
 }
@@ -293,7 +288,7 @@ PB_DECLARE_PRIMAL(PB_FLAVOUR(stencil_primal_simplex_launch)) {
   GradGeom g = with_vec(g0, 1);
   const int cap = g.L <= 4 ? 4 : g.L <= 8 ? 8 : g.L <= 16 ? 16 : 32;
   // operands staged through shared memory (every iteration but the first, uniform T)
-  if (!kty_zero && !T.ptr && staged_enabled()) {
+  if (!kty_zero && !T.ptr) {
     const unsigned sgrid = staged_grid((size_t)g.q * g.nx);
     if (dry_run || sgrid == 0) return sgrid;
     g.halo.n_edge_ctas = staged_grid(g.q);
@@ -408,7 +403,7 @@ PB_DECLARE_DUAL(PB_FLAVOUR(stencil_dual_norm2_launch)) {
   // through shared memory (pb_stencil_staged.cuh)
   bool scalar_coeffs = !d.moreau && !S.ptr;
   for (int k = 0; k < 7; ++k) scalar_coeffs = scalar_coeffs && !d.coeffs.ptr[k];
-  if (per_pixel && g0.L > 4 && scalar_coeffs && staged_enabled()) {
+  if (per_pixel && g0.L > 4 && scalar_coeffs) {
     GradGeom gs = with_vec(g0, 1);
     const unsigned sgrid = staged_grid((size_t)gs.q * gs.nx);
     if (dry_run || sgrid == 0) return sgrid;

@@ -266,7 +266,9 @@ def prox_spectral_cases(small=False):
 
 def linop_kron_tensor_core_cases():
     """Dense Kronecker factors large enough for the tcgen05 path (pb_kron_tc.cu: n_in * n_out >= 512, n_in <= 64):
-    padding of both factor dimensions, tail tiles, more tiles than SMs, overlapping blocks (accumulating stores)."""
+    padding of both factor dimensions, tail tiles, more tiles than SMs, overlapping blocks (accumulating stores).
+    kron(K, I) leaves through TMA tensor stores when d % 4 == 0 and through per-thread stores otherwise (_d1001,
+    _2x2_d258)."""
     r = rng(43)
     g = lambda m, n: r.standard_normal((m, n)).astype(np.float32)
     K16 = g(16, 32)
@@ -281,6 +283,8 @@ def linop_kron_tensor_core_cases():
         "id_kron_dense_18x44_d300": [("id_kron_dense", 0, 0, [g(18, 44), 300])],
         "id_kron_dense_64x64_d57013": [("id_kron_dense", 0, 0, [g(64, 64), 57013])],
         "id_kron_dense_16x32_2x2": [("id_kron_dense", rr * 16 * 260, cc * 32 * 260, [K16, 260]) for rr in (0, 1) for cc in (0, 1)],
+        "dense_kron_id_64x64_d1001": [("dense_kron_id", 0, 0, [g(64, 64), 1001])],
+        "dense_kron_id_16x32_2x2_d258": [("dense_kron_id", rr * 16 * 258, cc * 32 * 258, [K16, 258]) for rr in (0, 1) for cc in (0, 1)],
     }
 
 
