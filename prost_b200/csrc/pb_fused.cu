@@ -6,28 +6,19 @@
 
 namespace pb {
 
-#define PB_DECL_CAP(N)                                                                                  \
-  void fused_primal_cap_##N(Context*, unsigned, const ProxDesc&, const BlockList&, const float*,        \
-                            const float*, const float*, ScaleRef, const PdhgState*, bool, bool, bool,   \
-                            double*, float*);                                                           \
-  void fused_dual_cap_##N(Context*, unsigned, const ProxDesc&, const BlockList&, const float*,          \
-                          const float*, const float*, ScaleRef, const PdhgState*, bool, bool, double*,  \
-                          float*);
-PB_DECL_CAP(1) PB_DECL_CAP(2) PB_DECL_CAP(4) PB_DECL_CAP(8) PB_DECL_CAP(16) PB_DECL_CAP(32) PB_DECL_CAP(64)
+// defined in pb_fused_cap.cu and instantiated there for one CAP per translation unit
+template <int CAP> void fused_primal_cap(Context*, unsigned grid, const ProxDesc&, const BlockList&, const PrimalPass&);
+template <int CAP> void fused_dual_cap(Context*, unsigned grid, const ProxDesc&, const BlockList&, const DualPass&);
 
 unsigned fused_grid(Context* ctx, const ProxDesc& d) {
   // grid-stride: enough CTAs for 8 resident per SM, never more than the work
   return (unsigned)std::min<size_t>(grid_for(d.count), (size_t)ctx->num_sms * 8);
 }
 
-unsigned fused_primal_launch(Context* ctx, const ProxDesc& d, const BlockList& bl, const float* x,
-                             const float* y, const float* y_prev, ScaleRef T, const PdhgState* st,
-                             bool kty_zero, bool ktyprev_zero, bool check, double* partials,
-                             float* x_out) {
+unsigned fused_primal_launch(Context* ctx, const ProxDesc& d, const BlockList& bl, const PrimalPass& p) {
   if (d.count == 0) return 0;
   const unsigned grid = fused_grid(ctx, d);
-#define PB_CASE(N) \
-  case N: fused_primal_cap_##N(ctx, grid, d, bl, x, y, y_prev, T, st, kty_zero, ktyprev_zero, check, partials, x_out); break;
+#define PB_CASE(N) case N: fused_primal_cap<N>(ctx, grid, d, bl, p); break;
   switch (dim_cap(d.dim, d.kind)) {
     PB_CASE(1) PB_CASE(2) PB_CASE(4) PB_CASE(8) PB_CASE(16) PB_CASE(32) PB_CASE(64)
     default: fail(PB_ERR_UNSUPPORTED, "fused pass: group dimension too large");
@@ -38,13 +29,10 @@ unsigned fused_primal_launch(Context* ctx, const ProxDesc& d, const BlockList& b
   return grid;
 }
 
-unsigned fused_dual_launch(Context* ctx, const ProxDesc& d, const BlockList& bl, const float* y,
-                           const float* x_new, const float* x_old, ScaleRef S, const PdhgState* st,
-                           bool kxprev_zero, bool check, double* partials, float* y_out) {
+unsigned fused_dual_launch(Context* ctx, const ProxDesc& d, const BlockList& bl, const DualPass& p) {
   if (d.count == 0) return 0;
   const unsigned grid = fused_grid(ctx, d);
-#define PB_CASE(N) \
-  case N: fused_dual_cap_##N(ctx, grid, d, bl, y, x_new, x_old, S, st, kxprev_zero, check, partials, y_out); break;
+#define PB_CASE(N) case N: fused_dual_cap<N>(ctx, grid, d, bl, p); break;
   switch (dim_cap(d.dim, d.kind)) {
     PB_CASE(1) PB_CASE(2) PB_CASE(4) PB_CASE(8) PB_CASE(16) PB_CASE(32) PB_CASE(64)
     default: fail(PB_ERR_UNSUPPORTED, "fused pass: group dimension too large");

@@ -156,14 +156,36 @@ struct DualSource {
 
 #endif  // __CUDACC__
 
+// Operands of one primal pass over the range of one prox (generic here, specialised in pb_stencil.cuh):
+// x_out = prox_g(x - tau T K^T y).  kty_zero / ktyprev_zero take K^T y / K^T y_prev as 0 (the reference's
+// quirks above); with `check` the pass also writes the dual residual sums to `partials`.
+struct PrimalPass {
+  const float* x = nullptr;
+  const float* y = nullptr;
+  const float* y_prev = nullptr;      // check only
+  ScaleRef T = {};
+  const PdhgState* st = nullptr;
+  bool kty_zero = false, ktyprev_zero = false, check = false;
+  double* partials = nullptr;         // 2 doubles per CTA, check only
+  float* x_out = nullptr;
+};
+
+// Operands of one dual pass: y_out = prox_f*(y + sigma S ((1+theta) K x_new - theta K x_old)).  kxprev_zero
+// takes K x_old as 0; with `check` the pass also writes the primal residual sums to `partials`.
+struct DualPass {
+  const float* y = nullptr;
+  const float* x_new = nullptr;
+  const float* x_old = nullptr;
+  ScaleRef S = {};
+  const PdhgState* st = nullptr;
+  bool kxprev_zero = false, check = false;
+  double* partials = nullptr;         // 2 doubles per CTA, check only
+  float* y_out = nullptr;
+};
+
 // Host-side launchers (pb_fused.cu).  `partials` must hold 2*grid doubles; returns the grid size.
-unsigned fused_primal_launch(Context* ctx, const ProxDesc& d, const BlockList& bl, const float* x,
-                             const float* y, const float* y_prev, ScaleRef T, const PdhgState* st,
-                             bool kty_zero, bool ktyprev_zero, bool check, double* partials,
-                             float* x_out);
-unsigned fused_dual_launch(Context* ctx, const ProxDesc& d, const BlockList& bl, const float* y,
-                           const float* x_new, const float* x_old, ScaleRef S, const PdhgState* st,
-                           bool kxprev_zero, bool check, double* partials, float* y_out);
+unsigned fused_primal_launch(Context* ctx, const ProxDesc& d, const BlockList& bl, const PrimalPass& p);
+unsigned fused_dual_launch(Context* ctx, const ProxDesc& d, const BlockList& bl, const DualPass& p);
 unsigned fused_grid(Context* ctx, const ProxDesc& d);
 
 }  // namespace pb

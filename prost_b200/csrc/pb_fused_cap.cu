@@ -8,44 +8,35 @@
 
 namespace pb {
 
-#define PB_CAT2(a, b) a##b
-#define PB_CAT(a, b) PB_CAT2(a, b)
-
-template <bool CHECK>
-static void primal_launch(Context* ctx, unsigned grid, const ProxDesc& d, const BlockList& bl,
-                          const float* x, const float* y, const float* y_prev, ScaleRef T,
-                          const PdhgState* st, bool kty_zero, bool ktyprev_zero, double* partials,
-                          float* x_out) {
-  PrimalSource<PB_CAP, CHECK> src;
-  src.x = x; src.y = y; src.y_prev = y_prev; src.T = T; src.st = st; src.bl = bl;
-  src.kty_zero = kty_zero; src.ktyprev_zero = ktyprev_zero; src.partials = partials;
-  prox_pass_kernel<PB_CAP, PrimalSource<PB_CAP, CHECK>><<<grid, kBlock, 0, ctx->stream>>>(d, src, x_out, T, false);
+template <int CAP, bool CHECK>
+static void primal_launch(Context* ctx, unsigned grid, const ProxDesc& d, const BlockList& bl, const PrimalPass& p) {
+  PrimalSource<CAP, CHECK> src;
+  src.x = p.x; src.y = p.y; src.y_prev = p.y_prev; src.T = p.T; src.st = p.st; src.bl = bl;
+  src.kty_zero = p.kty_zero; src.ktyprev_zero = p.ktyprev_zero; src.partials = p.partials;
+  prox_pass_kernel<CAP, PrimalSource<CAP, CHECK>><<<grid, kBlock, 0, ctx->stream>>>(d, src, p.x_out, p.T, false);
 }
 
-template <bool CHECK>
-static void dual_launch(Context* ctx, unsigned grid, const ProxDesc& d, const BlockList& bl,
-                        const float* y, const float* x_new, const float* x_old, ScaleRef S,
-                        const PdhgState* st, bool kxprev_zero, double* partials, float* y_out) {
-  DualSource<PB_CAP, CHECK> src;
-  src.y = y; src.x_new = x_new; src.x_old = x_old; src.S = S; src.st = st; src.bl = bl;
-  src.kxprev_zero = kxprev_zero; src.partials = partials;
-  prox_pass_kernel<PB_CAP, DualSource<PB_CAP, CHECK>><<<grid, kBlock, 0, ctx->stream>>>(d, src, y_out, S, false);
+template <int CAP, bool CHECK>
+static void dual_launch(Context* ctx, unsigned grid, const ProxDesc& d, const BlockList& bl, const DualPass& p) {
+  DualSource<CAP, CHECK> src;
+  src.y = p.y; src.x_new = p.x_new; src.x_old = p.x_old; src.S = p.S; src.st = p.st; src.bl = bl;
+  src.kxprev_zero = p.kxprev_zero; src.partials = p.partials;
+  prox_pass_kernel<CAP, DualSource<CAP, CHECK>><<<grid, kBlock, 0, ctx->stream>>>(d, src, p.y_out, p.S, false);
 }
 
-void PB_CAT(fused_primal_cap_, PB_CAP)(Context* ctx, unsigned grid, const ProxDesc& d, const BlockList& bl,
-                                       const float* x, const float* y, const float* y_prev, ScaleRef T,
-                                       const PdhgState* st, bool kty_zero, bool ktyprev_zero, bool check,
-                                       double* partials, float* x_out) {
-  if (check) primal_launch<true>(ctx, grid, d, bl, x, y, y_prev, T, st, kty_zero, ktyprev_zero, partials, x_out);
-  else primal_launch<false>(ctx, grid, d, bl, x, y, y_prev, T, st, kty_zero, ktyprev_zero, partials, x_out);
+template <int CAP>
+void fused_primal_cap(Context* ctx, unsigned grid, const ProxDesc& d, const BlockList& bl, const PrimalPass& p) {
+  if (p.check) primal_launch<CAP, true>(ctx, grid, d, bl, p);
+  else primal_launch<CAP, false>(ctx, grid, d, bl, p);
 }
 
-void PB_CAT(fused_dual_cap_, PB_CAP)(Context* ctx, unsigned grid, const ProxDesc& d, const BlockList& bl,
-                                     const float* y, const float* x_new, const float* x_old, ScaleRef S,
-                                     const PdhgState* st, bool kxprev_zero, bool check, double* partials,
-                                     float* y_out) {
-  if (check) dual_launch<true>(ctx, grid, d, bl, y, x_new, x_old, S, st, kxprev_zero, partials, y_out);
-  else dual_launch<false>(ctx, grid, d, bl, y, x_new, x_old, S, st, kxprev_zero, partials, y_out);
+template <int CAP>
+void fused_dual_cap(Context* ctx, unsigned grid, const ProxDesc& d, const BlockList& bl, const DualPass& p) {
+  if (p.check) dual_launch<CAP, true>(ctx, grid, d, bl, p);
+  else dual_launch<CAP, false>(ctx, grid, d, bl, p);
 }
+
+template void fused_primal_cap<PB_CAP>(Context*, unsigned, const ProxDesc&, const BlockList&, const PrimalPass&);
+template void fused_dual_cap<PB_CAP>(Context*, unsigned, const ProxDesc&, const BlockList&, const DualPass&);
 
 }  // namespace pb

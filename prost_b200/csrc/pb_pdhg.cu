@@ -401,16 +401,16 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
   if (comm_) {
     // the halo protocol lives in the specialised stencil passes: one planar gradient operator
     // (+ identity rows), one prox_g over all columns, Norm2 on the gradient rows
-    const ScaleRef Tr = problem_->right_ref(), Sr = problem_->left_ref();
+    PrimalPass pp;                     // dry runs: is there a specialised pass for each prox?
+    pp.T = problem_->right_ref();
+    DualPass dp;
+    dp.S = problem_->left_ref();
     bool ok = fused_ && stencil_.ok && g_descs_.size() == 1;
-    if (ok)
-      ok = stencil_primal_launch(ctx_, stencil_, g_descs_[0], nullptr, nullptr, nullptr, Tr, nullptr, false,
-                                 false, false, nullptr, nullptr, true) > 0;
+    if (ok) ok = stencil_primal_launch(ctx_, stencil_, g_descs_[0], pp, true) > 0;
     int halo_passes = 0;
     for (auto& d : f_descs_) {
       if (!ok) break;
-      ok = stencil_dual_launch(ctx_, stencil_, d, nullptr, nullptr, nullptr, Sr, nullptr, false, false, nullptr,
-                               nullptr, true) > 0;
+      ok = stencil_dual_launch(ctx_, stencil_, d, dp, true) > 0;
       if (d.index == 0) ++halo_passes;
     }
     ok = ok && halo_passes == 1;
@@ -466,19 +466,20 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
   // partial-sum buffers: one (a, b) pair per CTA of every launch of a pass
   if (fused_) {
     part_d_cap_ = part_p_cap_ = 0;
-    const ScaleRef Tr = problem_->right_ref(), Sr = problem_->left_ref();
-    (void)Tr; (void)Sr;
+    // dry runs of residual-refresh passes over the iterates' buffers (the grid depends on their alignment)
+    PrimalPass pp;
+    pp.x = x_.data(); pp.y = y_.data(); pp.y_prev = y_prev_.data(); pp.check = true; pp.x_out = x_prev_.data();
     for (size_t i = 0; i < g_descs_.size(); ++i) {
       const ProxDesc& d = g_descs_[i];
-      const unsigned sg = stencil_primal_launch(ctx_, stencil_, d, x_.data(), y_.data(), y_prev_.data(), g_scale_[i],
-                                                nullptr, false, false, true, nullptr, x_prev_.data(), true);
-      part_d_cap_ += std::max(sg, fused_grid(ctx_, d));
+      pp.T = g_scale_[i];
+      part_d_cap_ += std::max(stencil_primal_launch(ctx_, stencil_, d, pp, true), fused_grid(ctx_, d));
     }
+    DualPass dp;
+    dp.y = y_.data(); dp.x_new = x_.data(); dp.x_old = x_prev_.data(); dp.check = true; dp.y_out = y_prev_.data();
     for (size_t i = 0; i < f_descs_.size(); ++i) {
       const ProxDesc& d = f_descs_[i];
-      const unsigned sg = stencil_dual_launch(ctx_, stencil_, d, y_.data(), x_.data(), x_prev_.data(), f_scale_[i],
-                                              nullptr, false, true, nullptr, y_prev_.data(), true);
-      part_p_cap_ += std::max(sg, fused_grid(ctx_, d));
+      dp.S = f_scale_[i];
+      part_p_cap_ += std::max(stencil_dual_launch(ctx_, stencil_, d, dp, true), fused_grid(ctx_, d));
     }
   } else {
     part_p_cap_ = std::min<size_t>(grid_for(m), (size_t)ctx_->num_sms * 8);
@@ -501,54 +502,55 @@ void BackendPDHG::iteration_fused() {
   RingHalo ring_halo;
   const bool tiled = tile_ok_ && iteration_ > 0;
   if (tiled && comm_) ring_halo = slab_ring_halo();
-  const RingHalo* rh = (tiled && comm_) ? &ring_halo : nullptr;
-  // the residual-refresh launch folds the sums, combines them across ranks and advances the step-size state
-  // itself (RingFinish) unless the halos travel through NCCL staging buffers (no peer-mapped slots then)
   bool finished_in_kernel = false;
-  if (tiled && check) {
-    const bool can_finish = !comm_ || comm_->world() == 1 || comm_->reduce_p2p();
+  if (tiled) {
+    // whole iteration in one pass over HBM (pb_tile.cu): x_prev_ <- x^{k+1}, y_prev_ <- y^{k+1}
+    TilePass tp;
+    tp.x = x_.data(); tp.y = y_.data(); tp.T = T; tp.S = S; tp.st = st; tp.x_out = x_prev_.data();
+    tp.y_out = y_prev_.data();
+    tp.halo = comm_ ? &ring_halo : nullptr;
     RingFinish fin;
-    if (can_finish) fin = ring_finish();
-    // residual-refresh iteration in one pass: x_prev_ <- x^{k+1}; y^{k+1} cannot overwrite y_prev_ (the
-    // pass reads y^{k-1} from it), so it goes to a third buffer that then takes y_prev_'s place
-    nd = np = tile_check_iteration_launch(ctx_, stencil_, g_descs_[0], f_descs_[0], x_.data(), y_.data(),
-                                          y_prev_.data(), T, S, st, iteration_ <= 1, part_d_.data(), part_p_.data(),
-                                          x_prev_.data(), y_prev_staging(), rh, can_finish ? &fin : nullptr);
-    finished_in_kernel = can_finish;
-    tile_check_iterations_++;
+    if (check) {
+      // the residual-refresh launch folds the sums, combines them across ranks and advances the step-size state
+      // itself (RingFinish) unless the halos travel through NCCL staging buffers (no peer-mapped slots then)
+      finished_in_kernel = !comm_ || comm_->world() == 1 || comm_->reduce_p2p();
+      if (finished_in_kernel) { fin = ring_finish(); tp.finish = &fin; }
+      tp.check = true;
+      tp.y_prev = y_prev_.data();
+      tp.ktyprev_zero = iteration_ <= 1;
+      tp.part_d = part_d_.data(); tp.part_p = part_p_.data();
+      // y^{k+1} cannot overwrite y_prev_ (the pass reads y^{k-1} from it), so it goes to a third buffer that
+      // then takes y_prev_'s place
+      tp.y_out = y_prev_staging();
+    }
+    nd = np = tile_iteration_launch(ctx_, stencil_, g_descs_[0], f_descs_[0], tp);
     x_.swap(x_prev_);
-    y_prev_.swap(y_stage_);      // y_prev_ now holds y^{k+1}, y_stage_ the dead y^{k-1}
+    if (check) {
+      y_prev_.swap(y_stage_);    // y_prev_ now holds y^{k+1}, y_stage_ the dead y^{k-1}
+      tile_check_iterations_++;
+    }
     y_.swap(y_prev_);            // y_ = y^{k+1}, y_prev_ = y^k
     tile_iterations_++;
     if (prof_ev_) {
       PB_CUDA(cudaEventRecord(prof_ev_[1], ctx_->stream));
       PB_CUDA(cudaEventRecord(prof_ev_[2], ctx_->stream));
     }
-  } else if (tiled) {
-    // whole iteration in one pass over HBM (pb_tile.cu): x_prev_ <- x^{k+1}, y_prev_ <- y^{k+1}
-    tile_iteration_launch(ctx_, stencil_, g_descs_[0], f_descs_[0], x_.data(), y_.data(), T, S, st,
-                          x_prev_.data(), y_prev_.data(), rh);
-    x_.swap(x_prev_);
-    y_.swap(y_prev_);
-    tile_iterations_++;
-    if (prof_ev_) {
-      PB_CUDA(cudaEventRecord(prof_ev_[1], ctx_->stream));
-      PB_CUDA(cudaEventRecord(prof_ev_[2], ctx_->stream));
-    }
   } else {
-    // primal pass: x_prev_ <- prox_g(x_ - tau T K^T y_), then swap so that x_ is x^{k+1}
+    // primal pass: x_prev_ <- prox_g(x_ - tau T K^T y_), then swap so that x_ is x^{k+1}.  Each prox range runs
+    // the specialised stencil pass where one covers it, the generic fused pass otherwise.
     unsigned off = 0;
     unsigned xs = 0, ys = 0;
     if (comm_) { xs = ++comm_->x_seq; slab_primal_halo(xs); }
+    PrimalPass pp;
+    pp.x = x_.data(); pp.y = y_.data(); pp.y_prev = y_prev_.data(); pp.st = st;
+    pp.kty_zero = iteration_ == 0; pp.ktyprev_zero = iteration_ <= 1; pp.check = check;
+    pp.x_out = x_prev_.data();
     for (size_t i = 0; i < g_descs_.size(); ++i) {
       const ProxDesc& d = g_descs_[i];
-      const ScaleRef Td = g_scale_[i];
-      unsigned g = stencil_primal_launch(ctx_, stencil_, d, x_.data(), y_.data(), y_prev_.data(), Td, st,
-                                         iteration_ == 0, iteration_ <= 1, check,
-                                         part_d_.data() + 2 * (size_t)off, x_prev_.data());
-      if (g == 0)
-        g = fused_primal_launch(ctx_, d, blocks_, x_.data(), y_.data(), y_prev_.data(), Td, st, iteration_ == 0,
-                                iteration_ <= 1, check, part_d_.data() + 2 * (size_t)off, x_prev_.data());
+      pp.T = g_scale_[i];
+      pp.partials = part_d_.data() + 2 * (size_t)off;
+      unsigned g = stencil_primal_launch(ctx_, stencil_, d, pp);
+      if (g == 0) g = fused_primal_launch(ctx_, d, blocks_, pp);
       off += g;
     }
     nd = off;
@@ -558,14 +560,16 @@ void BackendPDHG::iteration_fused() {
 
     // dual pass: y_prev_ <- prox_f*(y_ + sigma S K(2x^{k+1} - x^k)) (theta-extrapolated), then swap
     off = 0;
+    DualPass dp;
+    dp.y = y_.data(); dp.x_new = x_.data(); dp.x_old = x_prev_.data(); dp.st = st;
+    dp.kxprev_zero = iteration_ == 0; dp.check = check;
+    dp.y_out = y_prev_.data();
     for (size_t i = 0; i < f_descs_.size(); ++i) {
       const ProxDesc& d = f_descs_[i];
-      const ScaleRef Sd = f_scale_[i];
-      unsigned g = stencil_dual_launch(ctx_, stencil_, d, y_.data(), x_.data(), x_prev_.data(), Sd, st,
-                                       iteration_ == 0, check, part_p_.data() + 2 * (size_t)off, y_prev_.data());
-      if (g == 0)
-        g = fused_dual_launch(ctx_, d, blocks_, y_.data(), x_.data(), x_prev_.data(), Sd, st, iteration_ == 0,
-                              check, part_p_.data() + 2 * (size_t)off, y_prev_.data());
+      dp.S = f_scale_[i];
+      dp.partials = part_p_.data() + 2 * (size_t)off;
+      unsigned g = stencil_dual_launch(ctx_, stencil_, d, dp);
+      if (g == 0) g = fused_dual_launch(ctx_, d, blocks_, dp);
       off += g;
     }
     np = off;

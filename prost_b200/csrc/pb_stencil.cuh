@@ -99,6 +99,25 @@ struct RingFinish {
   CrossSum cross;
 };
 
+// Operands of one launch of the ring kernel: the primal and the dual pass of one iteration (PrimalPass /
+// DualPass in one).  With `check` it also reads y_prev and writes the dual (part_d) and primal (part_p)
+// residual sums; `halo` selects the slab variants.
+struct TilePass {
+  const float* x = nullptr;
+  const float* y = nullptr;
+  const float* y_prev = nullptr;       // check only
+  ScaleRef T = {}, S = {};             // uniform: only .val is read
+  const PdhgState* st = nullptr;
+  bool check = false;
+  bool ktyprev_zero = true;            // check only
+  double* part_d = nullptr;            // check only
+  double* part_p = nullptr;
+  float* x_out = nullptr;
+  float* y_out = nullptr;
+  const RingHalo* halo = nullptr;      // slab mode
+  const RingFinish* finish = nullptr;  // check only: the launch finalizes the iteration itself
+};
+
 struct GradGeom {
   uint32_t nx = 0, ny = 0, L = 0, nxny = 0, plane = 0;
   uint32_t q = 0;                 // ny / VEC
@@ -692,13 +711,10 @@ StencilPlan plan_stencil(const std::vector<std::shared_ptr<Block>>& blocks, size
 
 // Each returns 0 when the (operator, prox) pair is not covered by a specialised kernel (the caller
 // then uses the generic fused kernel), otherwise the number of CTAs launched (= partial pairs written).
-unsigned stencil_primal_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& d, const float* x,
-                               const float* y, const float* y_prev, ScaleRef T, const PdhgState* st,
-                               bool kty_zero, bool ktyprev_zero, bool check, double* partials, float* x_out,
+// dry_run: only the grid the pass would launch; the operand pointers are read for their alignment.
+unsigned stencil_primal_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& d, const PrimalPass& p,
                                bool dry_run = false);
-unsigned stencil_dual_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& d, const float* y,
-                             const float* x_new, const float* x_old, ScaleRef S, const PdhgState* st,
-                             bool kxprev_zero, bool check, double* partials, float* y_out,
+unsigned stencil_dual_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& d, const DualPass& p,
                              bool dry_run = false);
 
 // ---- whole iteration as one tiled pass (pb_tile.cu) ---------------------------------------------
@@ -706,18 +722,10 @@ bool tile_iteration_supported(const StencilPlan& plan, const std::vector<ProxDes
                               const std::vector<ProxDesc>& fd, ScaleRef T, ScaleRef S);
 // can the ring kernel run this plan, plain and residual-refresh launch alike (slab: the halo variants)?
 bool tile_ring_available(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf, bool slab);
-// plain iteration as one tiled pass; raises PB_ERR_CUDA if the ring kernel cannot be launched
-void tile_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
-                           const float* x, const float* y, ScaleRef T, ScaleRef S, const PdhgState* st,
-                           float* x_out, float* y_out, const RingHalo* halo = nullptr);
-// residual-refresh iteration as one tiled pass; returns the number of (a, b) partial pairs written to each of
-// part_d (dual residual sums) and part_p (primal residual sums); raises PB_ERR_CUDA if the ring kernel cannot
-// be launched
-unsigned tile_check_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
-                                     const float* x, const float* y, const float* y_prev, ScaleRef T, ScaleRef S,
-                                     const PdhgState* st, bool ktyprev_zero, double* part_d, double* part_p,
-                                     float* x_out, float* y_out, const RingHalo* halo = nullptr,
-                                     const RingFinish* finish = nullptr);
+// one iteration as one tiled pass; returns the number of (a, b) partial pairs written to each of part_d and
+// part_p (0 unless p.check); raises PB_ERR_CUDA if the ring kernel cannot be launched
+unsigned tile_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
+                               const TilePass& p);
 unsigned tile_ring_trace_read(unsigned long long* h_out, unsigned n);      // PB_RING_TRACE experiments
 
 }  // namespace pb

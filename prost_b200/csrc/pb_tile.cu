@@ -600,19 +600,14 @@ RingTraceSlot ring_trace_next() {
   return m;
 }
 
-struct RingArgs {
+// the TMA descriptors of a launch (see the kernel's parameters)
+struct RingMaps {
   CUtensorMap mp1, mp2, mx, mf, mq1, mq2;
-  bool check = false;
-  int ktyprev_zero = 1;
-  double* part_d = nullptr;
-  double* part_p = nullptr;
-  const RingHalo* halo = nullptr;      // slab mode
-  const RingFinish* finish = nullptr;  // residual-refresh launches that finalize the iteration in the kernel
 };
 
 template <int FN_G, int FN_F, bool CHECK, bool SLAB>
-unsigned ring_launch_k(Context* ctx, const RingArgs& a, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf,
-                       float Tval, float Sval, const PdhgState* st, float* x_out, float* y_out, bool dry_run) {
+unsigned ring_launch_k(Context* ctx, const RingMaps& m, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf,
+                       const TilePass& p, bool dry_run) {
   auto kernel = grad2d_iteration_ring_kernel<FN_G, FN_F, CHECK, SLAB>;
   static bool configured = false, ok = false;
   if (!configured) {
@@ -627,7 +622,7 @@ unsigned ring_launch_k(Context* ctx, const RingArgs& a, const GradGeom& g, const
   const unsigned grid = (unsigned)std::min<uint64_t>(n_tiles, (uint64_t)ctx->num_sms);
   if (dry_run) return grid;
   RingHalo h;
-  if (SLAB) h = *a.halo;
+  if (SLAB) h = *p.halo;
   // programmatic stream serialization: see griddepcontrol in the kernel.  Measured (profiles/r02_scaling.md): the
   // launch-to-launch gap drops from 3.8 to 1.8 us on one GPU, but on slabs the end-of-kernel flush of the
   // NVLink halo stores dominates the gap and early-resident CTAs cost more than they hide (period 54.3 vs
@@ -643,54 +638,42 @@ unsigned ring_launch_k(Context* ctx, const RingArgs& a, const GradGeom& g, const
   cfg.attrs = &attr;
   cfg.numAttrs = SLAB ? 0 : 1;
   const cudaError_t e = cudaLaunchKernelEx(
-      &cfg, kernel, a.mp1, a.mp2, a.mx, a.mf, a.mq1, a.mq2, g, pg, pf, Tval, Sval, st,
-      FastDiv((uint64_t)tiles_x * tiles_y), FastDiv(tiles_y), (uint32_t)n_tiles, a.ktyprev_zero, a.part_d, a.part_p,
-      x_out, y_out, tiles_x, h, ring_trace_next(), (CHECK && a.finish) ? *a.finish : RingFinish());
+      &cfg, kernel, m.mp1, m.mp2, m.mx, m.mf, m.mq1, m.mq2, g, pg, pf, p.T.val, p.S.val, p.st,
+      FastDiv((uint64_t)tiles_x * tiles_y), FastDiv(tiles_y), (uint32_t)n_tiles, p.ktyprev_zero ? 1 : 0, p.part_d,
+      p.part_p, p.x_out, p.y_out, tiles_x, h, ring_trace_next(), (CHECK && p.finish) ? *p.finish : RingFinish());
   if (e != cudaSuccess) { cudaGetLastError(); return 0; }
   return grid;
 }
 
 template <int FN_G, int FN_F>
-unsigned ring_launch_fn(Context* ctx, const RingArgs& a, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf,
-                        float Tval, float Sval, const PdhgState* st, float* x_out, float* y_out, bool dry_run) {
-  if (a.halo) {
-    if (a.check) return ring_launch_k<FN_G, FN_F, true, true>(ctx, a, g, pg, pf, Tval, Sval, st, x_out, y_out, dry_run);
-    return ring_launch_k<FN_G, FN_F, false, true>(ctx, a, g, pg, pf, Tval, Sval, st, x_out, y_out, dry_run);
-  }
-  if (a.check) return ring_launch_k<FN_G, FN_F, true, false>(ctx, a, g, pg, pf, Tval, Sval, st, x_out, y_out, dry_run);
-  return ring_launch_k<FN_G, FN_F, false, false>(ctx, a, g, pg, pf, Tval, Sval, st, x_out, y_out, dry_run);
+unsigned ring_launch_fn(Context* ctx, const RingMaps& m, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf,
+                        const TilePass& p, bool dry_run) {
+  auto launch = p.halo ? (p.check ? ring_launch_k<FN_G, FN_F, true, true> : ring_launch_k<FN_G, FN_F, false, true>)
+                       : (p.check ? ring_launch_k<FN_G, FN_F, true, false> : ring_launch_k<FN_G, FN_F, false, false>);
+  return launch(ctx, m, g, pg, pf, p, dry_run);
 }
 
 // returns the number of CTAs (= residual partial pairs per residual when check), 0 if not launched
-unsigned ring_launch(Context* ctx, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf, const float* x,
-                     const float* y, const float* y_prev, float Tval, float Sval, const PdhgState* st, bool check,
-                     bool ktyprev_zero, double* part_d, double* part_p, float* x_out, float* y_out, bool dry_run,
-                     const RingHalo* halo, const RingFinish* finish = nullptr) {
-  RingArgs a;
-  a.halo = halo;
-  a.finish = finish;
-  a.check = check;
-  a.ktyprev_zero = ktyprev_zero ? 1 : 0;
-  a.part_d = part_d;
-  a.part_p = part_p;
+unsigned ring_launch(Context* ctx, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf, const TilePass& p,
+                     bool dry_run) {
+  RingMaps m;
   if (!dry_run) {
-    if (!tensor_map_for(y, g.ny, g.nx, 2 * g.L, kRingRows, kRingCols + 1, a.mp1)) return 0;
-    if (!tensor_map_for(y, g.ny, g.nx, 2 * g.L, kRingR2, kRingCols, a.mp2)) return 0;
-    if (!tensor_map_for(x, g.ny, g.nx, g.L, kRingRows, kRingCols, a.mx)) return 0;
-    const float* f = pg.coeffs.ptr[1] ? pg.coeffs.ptr[1] : x;      // unused when b is a scalar
-    if (!tensor_map_for(f, g.ny, g.nx, g.L, kRingRows, kRingCols, a.mf)) return 0;
-    const float* q = (check && !ktyprev_zero) ? y_prev : y;         // unused otherwise
-    if (!tensor_map_for(q, g.ny, g.nx, 2 * g.L, kRingRows, kRingCols + 1, a.mq1)) return 0;
-    if (!tensor_map_for(q, g.ny, g.nx, 2 * g.L, kRingR2, kRingCols, a.mq2)) return 0;
+    if (!tensor_map_for(p.y, g.ny, g.nx, 2 * g.L, kRingRows, kRingCols + 1, m.mp1)) return 0;
+    if (!tensor_map_for(p.y, g.ny, g.nx, 2 * g.L, kRingR2, kRingCols, m.mp2)) return 0;
+    if (!tensor_map_for(p.x, g.ny, g.nx, g.L, kRingRows, kRingCols, m.mx)) return 0;
+    const float* f = pg.coeffs.ptr[1] ? pg.coeffs.ptr[1] : p.x;    // unused when b is a scalar
+    if (!tensor_map_for(f, g.ny, g.nx, g.L, kRingRows, kRingCols, m.mf)) return 0;
+    const float* q = (p.check && !p.ktyprev_zero) ? p.y_prev : p.y;  // unused otherwise
+    if (!tensor_map_for(q, g.ny, g.nx, 2 * g.L, kRingRows, kRingCols + 1, m.mq1)) return 0;
+    if (!tensor_map_for(q, g.ny, g.nx, 2 * g.L, kRingR2, kRingCols, m.mq2)) return 0;
   } else if (!encode_tiled_fn()) {
     return 0;
   }
-#define PB_ARGS ctx, a, g, pg, pf, Tval, Sval, st, x_out, y_out, dry_run
   const bool leq0 = pf.fn == PB_FUN_IND_LEQ0;
-  if (pg.fn == PB_FUN_SQUARE) return leq0 ? ring_launch_fn<PB_FUN_SQUARE, PB_FUN_IND_LEQ0>(PB_ARGS) : ring_launch_fn<PB_FUN_SQUARE, -1>(PB_ARGS);
-  if (pg.fn == PB_FUN_ABS) return leq0 ? ring_launch_fn<PB_FUN_ABS, PB_FUN_IND_LEQ0>(PB_ARGS) : ring_launch_fn<PB_FUN_ABS, -1>(PB_ARGS);
-  return leq0 ? ring_launch_fn<-1, PB_FUN_IND_LEQ0>(PB_ARGS) : ring_launch_fn<-1, -1>(PB_ARGS);
-#undef PB_ARGS
+  auto launch = pg.fn == PB_FUN_SQUARE ? (leq0 ? ring_launch_fn<PB_FUN_SQUARE, PB_FUN_IND_LEQ0> : ring_launch_fn<PB_FUN_SQUARE, -1>)
+              : pg.fn == PB_FUN_ABS    ? (leq0 ? ring_launch_fn<PB_FUN_ABS, PB_FUN_IND_LEQ0> : ring_launch_fn<PB_FUN_ABS, -1>)
+                                       : (leq0 ? ring_launch_fn<-1, PB_FUN_IND_LEQ0> : ring_launch_fn<-1, -1>);
+  return launch(ctx, m, g, pg, pf, p, dry_run);
 }
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
@@ -734,35 +717,22 @@ bool tile_iteration_supported(const StencilPlan& plan, const std::vector<ProxDes
 
 bool tile_ring_available(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf, bool slab) {
   const RingHalo halo;                 // selects the slab variants; a dry run reads nothing from it
-  for (const bool check : {false, true})
-    if (!ring_launch(ctx, plan.geom, pg, pf, nullptr, nullptr, nullptr, 0.f, 0.f, nullptr, check, true, nullptr,
-                     nullptr, nullptr, nullptr, true, slab ? &halo : nullptr))
-      return false;
+  TilePass p;
+  p.halo = slab ? &halo : nullptr;
+  for (const bool check : {false, true}) {
+    p.check = check;
+    if (!ring_launch(ctx, plan.geom, pg, pf, p, true)) return false;
+  }
   return true;
 }
 
-// Residual-refresh iteration as one tiled pass.  Returns the number of partial pairs written to EACH of part_d /
-// part_p.
-unsigned tile_check_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
-                                     const float* x, const float* y, const float* y_prev, ScaleRef T, ScaleRef S,
-                                     const PdhgState* st, bool ktyprev_zero, double* part_d, double* part_p,
-                                     float* x_out, float* y_out, const RingHalo* halo, const RingFinish* finish) {
-  const unsigned n = ring_launch(ctx, plan.geom, pg, pf, x, y, y_prev, T.val, S.val, st, true, ktyprev_zero, part_d,
-                                 part_p, x_out, y_out, false, halo, finish);
+unsigned tile_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
+                               const TilePass& p) {
+  const unsigned n = ring_launch(ctx, plan.geom, pg, pf, p, false);
   if (!n) fail(PB_ERR_CUDA, "the one-pass ring kernel could not be launched");
   PB_CHECK_LAUNCH();
   ctx->launches++;
-  return n;
-}
-
-void tile_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
-                           const float* x, const float* y, ScaleRef T, ScaleRef S, const PdhgState* st,
-                           float* x_out, float* y_out, const RingHalo* halo) {
-  if (!ring_launch(ctx, plan.geom, pg, pf, x, y, nullptr, T.val, S.val, st, false, true, nullptr, nullptr, x_out,
-                   y_out, false, halo))
-    fail(PB_ERR_CUDA, "the one-pass ring kernel could not be launched");
-  PB_CHECK_LAUNCH();
-  ctx->launches++;
+  return p.check ? n : 0;
 }
 
 }  // namespace pb
