@@ -10,6 +10,17 @@
 
 namespace pb {
 
+// device-visible control words of one rank (lives at the start of the IPC block)
+struct HaloFlags {
+  unsigned x_seq;        // sequence number of the newest x halo written by the RIGHT neighbour
+  unsigned y_seq;        // sequence number of the newest y halo written by the LEFT neighbour
+  unsigned done_primal;  // local: edge CTAs of the running primal pass that finished
+  unsigned done_dual;    // local: same for the dual pass
+  int error;             // set by a kernel whose halo wait timed out
+  unsigned red_count;    // local: reductions over ranks executed so far (pb_crosssum.cuh)
+  int pad[10];
+};
+
 namespace {
 
 // ---- lazily loaded NCCL entry points ---------------------------------------------------------------
@@ -131,13 +142,14 @@ void Comm::ensure_halo(size_t col_floats) {
   const double mean = chk[0] / world_;
   if (chk[1] / world_ != mean * mean)
     fail(PB_ERR_INVALID, "slab decomposition: ranks disagree on the halo column size (ny * L)");
+  x_seq_ = y_seq_ = 0;
+  halo_in_ll_ = false;
   if (col_floats == col_floats_ && block_) {
     // same geometry as before: just reset the control words
     PB_CUDA(cudaStreamSynchronize(s));
     barrier();
     PB_CUDA(cudaMemsetAsync(block_, 0, kFlagBytes + 4 * col_floats_ * sizeof(float) + 5 * ll_lines() * sizeof(uint4), s));
     PB_CUDA(cudaStreamSynchronize(s));
-    x_seq = y_seq = 0;
     barrier();
     return;
   }
@@ -145,7 +157,6 @@ void Comm::ensure_halo(size_t col_floats) {
   barrier();                       // nobody still reads a block that is about to be unmapped
   release_halo();
   col_floats_ = col_floats;
-  x_seq = y_seq = 0;
   const size_t bytes = kFlagBytes + 4 * col_floats * sizeof(float) + 5 * ll_lines() * sizeof(uint4);
   PB_CUDA(cudaMalloc(&block_, bytes));
   PB_CUDA(cudaMemsetAsync(block_, 0, bytes, s));
@@ -263,40 +274,116 @@ __global__ void halo_unpack_ll_kernel(const uint4* __restrict__ ll, float* __res
 
 }  // namespace
 
-void Comm::pack_ll(unsigned xs, unsigned ys) {
-  if (!p2p_ || world_ == 1 || !block_) return;
+// Primal pass number xs: reads the y columns the left neighbour's dual passes ys / ys-1 delivered, hands column 0
+// of the new x to the left.
+SlabHalo Comm::primal_halo() {
+  const unsigned xs = ++x_seq_, ys = y_seq_;
+  SlabHalo h;
+  h.has_left = has_left();
+  h.has_right = has_right();
+  h.in_a = y_slot(ys);
+  h.in_b = y_slot(ys - 1);
+  h.out = x_out(xs);
+  if (p2p_ && h.has_left) {
+    h.wait_flag = &flags_->y_seq;
+    h.wait_seq = ys;
+    h.done_counter = &flags_->done_primal;
+    h.signal_flag = &static_cast<HaloFlags*>(left_block_)->x_seq;    // the left neighbour's
+    h.signal_seq = xs;
+    h.error = &flags_->error;
+  }
+  return h;
+}
+
+// Dual pass number ys: reads the x columns of the right neighbour's primal passes xs / xs-1, hands the last column
+// of the new x-component of y to the right.  NCCL staging mode: first the primal pass's x column moves to the left.
+SlabHalo Comm::dual_halo() {
+  const unsigned xs = x_seq_, ys = ++y_seq_;
+  if (!p2p_ && world_ > 1) {
+    PB_NCCL(nccl().GroupStart());
+    if (has_left()) PB_NCCL(nccl().Send(stage_x_.data(), col_floats_, ncclFloat, rank_ - 1, as_comm(nccl_), ctx_->stream));
+    if (has_right()) PB_NCCL(nccl().Recv(x_slot(xs), col_floats_, ncclFloat, rank_ + 1, as_comm(nccl_), ctx_->stream));
+    PB_NCCL(nccl().GroupEnd());
+  }
+  SlabHalo h;
+  h.has_left = has_left();
+  h.has_right = has_right();
+  h.in_a = x_slot(xs);
+  h.in_b = x_slot(xs - 1);
+  h.out = y_out(ys);
+  if (p2p_ && h.has_right) {
+    h.wait_flag = &flags_->x_seq;
+    h.wait_seq = xs;
+    h.done_counter = &flags_->done_dual;
+    h.signal_flag = &static_cast<HaloFlags*>(right_block_)->y_seq;   // the right neighbour's
+    h.signal_seq = ys;
+    h.error = &flags_->error;
+  }
+  return h;
+}
+
+// NCCL staging mode: the dual pass's y column moves to the right.  Peer-to-peer with ring_follows: the received
+// plain columns x(x_seq), y(y_seq) are repacked into the local flag-in-data slots once their sequence words arrive.
+void Comm::end_two_pass_iteration(bool ring_follows) {
+  halo_in_ll_ = false;
+  if (!p2p_ && world_ > 1) {
+    PB_NCCL(nccl().GroupStart());
+    if (has_right()) PB_NCCL(nccl().Send(stage_y_.data(), col_floats_, ncclFloat, rank_ + 1, as_comm(nccl_), ctx_->stream));
+    if (has_left()) PB_NCCL(nccl().Recv(y_slot(y_seq_), col_floats_, ncclFloat, rank_ - 1, as_comm(nccl_), ctx_->stream));
+    PB_NCCL(nccl().GroupEnd());
+  }
+  if (!ring_follows || !p2p_ || world_ == 1 || !block_) return;
   const unsigned groups = static_cast<unsigned>(col_floats_ / 4);
   const unsigned grid = std::max(1u, std::min(64u, (groups + 255u) / 256u));
   if (has_right())
-    halo_pack_ll_kernel<<<grid, 256, 0, ctx_->stream>>>(x_slot(xs), const_cast<uint4*>(x_ll(xs)), xs, &flags_->x_seq,
-                                                        groups, &flags_->error);
+    halo_pack_ll_kernel<<<grid, 256, 0, ctx_->stream>>>(x_slot(x_seq_), const_cast<uint4*>(x_ll(x_seq_)), x_seq_,
+                                                        &flags_->x_seq, groups, &flags_->error);
   if (has_left())
-    halo_pack_ll_kernel<<<grid, 256, 0, ctx_->stream>>>(y_slot(ys), const_cast<uint4*>(y_ll(ys)), ys, &flags_->y_seq,
-                                                        groups, &flags_->error);
+    halo_pack_ll_kernel<<<grid, 256, 0, ctx_->stream>>>(y_slot(y_seq_), const_cast<uint4*>(y_ll(y_seq_)), y_seq_,
+                                                        &flags_->y_seq, groups, &flags_->error);
   PB_CHECK_LAUNCH();
 }
 
-void Comm::unpack_ll_x(unsigned seq) {
-  if (!p2p_ || world_ == 1 || !block_ || !has_right()) return;
-  const unsigned groups = static_cast<unsigned>(col_floats_ / 4);
-  halo_unpack_ll_kernel<<<std::max(1u, std::min(64u, (groups + 255u) / 256u)), 256, 0, ctx_->stream>>>(
-      x_ll(seq), x_slot(seq), groups);
-  PB_CHECK_LAUNCH();
+// One-pass iteration = primal pass xs and dual pass ys in one launch: the left-edge tiles play the primal pass's
+// part of the protocol, the right-edge tiles the dual pass's.
+RingHalo Comm::ring_halo() {
+  RingHalo h;
+  h.has_left = has_left();
+  h.has_right = has_right();
+  const unsigned ys_in = y_seq_;       // newest y halo (left neighbour's previous iteration)
+  const unsigned xs = ++x_seq_, ys = ++y_seq_;
+  h.error = &flags_->error;
+  if (h.has_left) {
+    for (unsigned p = 0; p < 3; ++p) h.yl_ll[p] = y_ll(p);
+    for (unsigned p = 0; p < 2; ++p) h.x_out_ll[p] = x_ll_out(p);
+    h.y_wait_seq = ys_in;
+    h.x_signal_seq = xs;
+  }
+  if (h.has_right) {
+    for (unsigned p = 0; p < 2; ++p) h.xr_ll[p] = x_ll(p);
+    for (unsigned p = 0; p < 3; ++p) h.y_out_ll[p] = y_ll_out(p);
+    h.x_wait_seq = xs;
+    h.y_signal_seq = ys;
+  }
+  halo_in_ll_ = true;
+  return h;
 }
 
-void Comm::unpack_ll_y(unsigned seq) {
-  if (!p2p_ || world_ == 1 || !block_ || !has_left()) return;
-  const unsigned groups = static_cast<unsigned>(col_floats_ / 4);
-  halo_unpack_ll_kernel<<<std::max(1u, std::min(64u, (groups + 255u) / 256u)), 256, 0, ctx_->stream>>>(
-      y_ll(seq), y_slot(seq), groups);
-  PB_CHECK_LAUNCH();
-}
-
-unsigned* Comm::left_x_seq() const {
-  return (p2p_ && left_block_) ? &static_cast<HaloFlags*>(left_block_)->x_seq : nullptr;
-}
-unsigned* Comm::right_y_seq() const {
-  return (p2p_ && right_block_) ? &static_cast<HaloFlags*>(right_block_)->y_seq : nullptr;
+Comm::PlainHalo Comm::plain_halo() {
+  if (halo_in_ll_ && p2p_ && world_ > 1 && block_) {
+    const unsigned groups = static_cast<unsigned>(col_floats_ / 4);
+    const unsigned grid = std::max(1u, std::min(64u, (groups + 255u) / 256u));
+    auto unpack = [&](const uint4* ll, float* plain) {
+      halo_unpack_ll_kernel<<<grid, 256, 0, ctx_->stream>>>(ll, plain, groups);
+      PB_CHECK_LAUNCH();
+    };
+    if (has_right()) {
+      unpack(x_ll(x_seq_), x_slot(x_seq_));
+      unpack(x_ll(x_seq_ - 1), x_slot(x_seq_ - 1));
+    }
+    if (has_left()) unpack(y_ll(y_seq_ - 1), y_slot(y_seq_ - 1));
+  }
+  return {y_slot(y_seq_ - 1), x_slot(x_seq_), x_slot(x_seq_ - 1)};
 }
 
 bool Comm::reduce_p2p() const {
@@ -331,22 +418,6 @@ CrossSum Comm::cross_sum() const {
   }
   c.error = &flags_->error;
   return c;
-}
-
-void Comm::exchange_x(unsigned seq) {
-  if (p2p_ || world_ == 1) return;
-  PB_NCCL(nccl().GroupStart());
-  if (has_left()) PB_NCCL(nccl().Send(stage_x_.data(), col_floats_, ncclFloat, rank_ - 1, as_comm(nccl_), ctx_->stream));
-  if (has_right()) PB_NCCL(nccl().Recv(x_slot(seq), col_floats_, ncclFloat, rank_ + 1, as_comm(nccl_), ctx_->stream));
-  PB_NCCL(nccl().GroupEnd());
-}
-
-void Comm::exchange_y(unsigned seq) {
-  if (p2p_ || world_ == 1) return;
-  PB_NCCL(nccl().GroupStart());
-  if (has_right()) PB_NCCL(nccl().Send(stage_y_.data(), col_floats_, ncclFloat, rank_ + 1, as_comm(nccl_), ctx_->stream));
-  if (has_left()) PB_NCCL(nccl().Recv(y_slot(seq), col_floats_, ncclFloat, rank_ - 1, as_comm(nccl_), ctx_->stream));
-  PB_NCCL(nccl().GroupEnd());
 }
 
 void Comm::allreduce_sum(double* d_buf, size_t n) {

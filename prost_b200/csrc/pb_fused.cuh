@@ -26,6 +26,8 @@ namespace pb {
 
 constexpr int kMaxFusedBlocks = 6;
 
+struct SlabHalo;   // pb_comm.cuh
+
 struct BlockList {
   int n = 0;
   BlockDesc b[kMaxFusedBlocks];
@@ -158,7 +160,8 @@ struct DualSource {
 
 // Operands of one primal pass over the range of one prox (generic here, specialised in pb_stencil.cuh):
 // x_out = prox_g(x - tau T K^T y).  kty_zero / ktyprev_zero take K^T y / K^T y_prev as 0 (the reference's
-// quirks above); with `check` the pass also writes the dual residual sums to `partials`.
+// quirks above); with `check` the pass also writes the dual residual sums to `partials`.  `halo` (slab mode, read by
+// the specialised passes only) selects their slab variants when it has a neighbour.
 struct PrimalPass {
   const float* x = nullptr;
   const float* y = nullptr;
@@ -168,10 +171,11 @@ struct PrimalPass {
   bool kty_zero = false, ktyprev_zero = false, check = false;
   double* partials = nullptr;         // 2 doubles per CTA, check only
   float* x_out = nullptr;
+  const SlabHalo* halo = nullptr;
 };
 
 // Operands of one dual pass: y_out = prox_f*(y + sigma S ((1+theta) K x_new - theta K x_old)).  kxprev_zero
-// takes K x_old as 0; with `check` the pass also writes the primal residual sums to `partials`.
+// takes K x_old as 0; with `check` the pass also writes the primal residual sums to `partials`.  `halo`: as above.
 struct DualPass {
   const float* y = nullptr;
   const float* x_new = nullptr;
@@ -181,6 +185,7 @@ struct DualPass {
   bool kxprev_zero = false, check = false;
   double* partials = nullptr;         // 2 doubles per CTA, check only
   float* y_out = nullptr;
+  const SlabHalo* halo = nullptr;
 };
 
 // Host-side launchers (pb_fused.cu).  `partials` must hold 2*grid doubles; returns the grid size.

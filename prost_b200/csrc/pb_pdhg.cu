@@ -223,15 +223,11 @@ class BackendPDHG : public Backend {
   void set_slab(Comm* comm) override { comm_ = comm; }
 
  private:
-  // slab mode (comm_ != nullptr): halo descriptors of the two passes, slab-aware K / K^T
-  void slab_primal_halo(unsigned xs);
-  void slab_dual_halo(unsigned xs, unsigned ys);
-  RingHalo slab_ring_halo();           // advances x_seq / y_seq: one-pass iteration on a slab
+  // slab mode (comm_ != nullptr): slab-aware K / K^T
   DeviceBuffer<unsigned> fin_ticket_;        // RingFinish: CTAs of the running residual-refresh launch that are done
   RingFinish ring_finish();
   void slab_apply(float* d_res, const float* d_rhs, const float* d_halo, bool adjoint);
   Comm* comm_ = nullptr;
-  bool halo_in_ll_ = false;            // the newest halo columns live in the ring kernel's flag-in-data slots only
   bool is_check_iteration() const {
     // size_t % int of the reference: a negative residual_iter wraps to a huge modulus, i.e.
     // "only at iteration 0" (Appendix B #4)
@@ -314,7 +310,6 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
   cudaStream_t s = ctx_->stream;
 
   iteration_ = 0;
-  halo_in_ll_ = false;
   PdhgState st{};
   st.tau = static_cast<float>(opts_.tau0);
   st.sigma = static_cast<float>(opts_.sigma0);
@@ -499,9 +494,8 @@ void BackendPDHG::iteration_fused() {
   const PdhgState* st = d_state_.data();
 
   unsigned nd = 0, np = 0;
-  RingHalo ring_halo;
   const bool tiled = tile_ok_ && iteration_ > 0;
-  if (tiled && comm_) ring_halo = slab_ring_halo();
+  const RingHalo ring_halo = tiled && comm_ ? comm_->ring_halo() : RingHalo();
   bool finished_in_kernel = false;
   if (tiled) {
     // whole iteration in one pass over HBM (pb_tile.cu): x_prev_ <- x^{k+1}, y_prev_ <- y^{k+1}
@@ -539,12 +533,12 @@ void BackendPDHG::iteration_fused() {
     // primal pass: x_prev_ <- prox_g(x_ - tau T K^T y_), then swap so that x_ is x^{k+1}.  Each prox range runs
     // the specialised stencil pass where one covers it, the generic fused pass otherwise.
     unsigned off = 0;
-    unsigned xs = 0, ys = 0;
-    if (comm_) { xs = ++comm_->x_seq; slab_primal_halo(xs); }
+    const SlabHalo primal_halo = comm_ ? comm_->primal_halo() : SlabHalo();
     PrimalPass pp;
     pp.x = x_.data(); pp.y = y_.data(); pp.y_prev = y_prev_.data(); pp.st = st;
     pp.kty_zero = iteration_ == 0; pp.ktyprev_zero = iteration_ <= 1; pp.check = check;
     pp.x_out = x_prev_.data();
+    pp.halo = comm_ ? &primal_halo : nullptr;
     for (size_t i = 0; i < g_descs_.size(); ++i) {
       const ProxDesc& d = g_descs_[i];
       pp.T = g_scale_[i];
@@ -555,7 +549,7 @@ void BackendPDHG::iteration_fused() {
     }
     nd = off;
     x_.swap(x_prev_);
-    if (comm_) { comm_->exchange_x(xs); ys = ++comm_->y_seq; slab_dual_halo(xs, ys); }
+    const SlabHalo dual_halo = comm_ ? comm_->dual_halo() : SlabHalo();
     if (prof_ev_) PB_CUDA(cudaEventRecord(prof_ev_[1], ctx_->stream));
 
     // dual pass: y_prev_ <- prox_f*(y_ + sigma S K(2x^{k+1} - x^k)) (theta-extrapolated), then swap
@@ -564,6 +558,7 @@ void BackendPDHG::iteration_fused() {
     dp.y = y_.data(); dp.x_new = x_.data(); dp.x_old = x_prev_.data(); dp.st = st;
     dp.kxprev_zero = iteration_ == 0; dp.check = check;
     dp.y_out = y_prev_.data();
+    dp.halo = comm_ ? &dual_halo : nullptr;
     for (size_t i = 0; i < f_descs_.size(); ++i) {
       const ProxDesc& d = f_descs_[i];
       dp.S = f_scale_[i];
@@ -574,10 +569,9 @@ void BackendPDHG::iteration_fused() {
     }
     np = off;
     y_.swap(y_prev_);
-    if (comm_) { comm_->exchange_y(ys); stencil_.geom.halo = SlabHalo(); }
-    // the one-pass ring kernel reads its halo columns from flag-in-data slots: repack what this two-pass
-    // iteration received (iteration 0 of a ROF-shaped slab problem)
-    if (comm_ && tile_ok_) { comm_->pack_ll(xs, ys); halo_in_ll_ = false; }
+    // with tile_ok_ this is iteration 0 of a ROF-shaped slab problem: the one-pass iterations that follow read the
+    // halo columns it received from the flag-in-data slots
+    if (comm_) comm_->end_two_pass_iteration(tile_ok_);
     if (prof_ev_) PB_CUDA(cudaEventRecord(prof_ev_[2], ctx_->stream));
 
   }
@@ -610,74 +604,6 @@ RingFinish BackendPDHG::ring_finish() {
   f.iteration = iteration_;
   if (comm_ && comm_->world() > 1) f.cross = comm_->cross_sum();
   return f;
-}
-
-// Halo descriptor of the primal pass number `xs` (pb_comm.cuh): reads the y columns the left
-// neighbour's dual passes y_seq / y_seq-1 delivered, hands column 0 of the new x to the left.
-void BackendPDHG::slab_primal_halo(unsigned xs) {
-  SlabHalo h;
-  h.has_left = comm_->has_left();
-  h.has_right = comm_->has_right();
-  const unsigned ys = comm_->y_seq;                  // newest y halo
-  h.in_a = comm_->y_slot(ys);
-  h.in_b = comm_->y_slot(ys - 1);
-  h.out = comm_->x_out(xs);
-  if (comm_->p2p() && h.has_left) {
-    HaloFlags* f = comm_->flags();
-    h.wait_flag = &f->y_seq;
-    h.wait_seq = ys;
-    h.done_counter = &f->done_primal;
-    h.signal_flag = comm_->left_x_seq();
-    h.signal_seq = xs;
-    h.error = &f->error;
-  }
-  stencil_.geom.halo = h;
-}
-
-// One-pass iteration (pb_tile.cu ring kernel) = primal pass `xs` and dual pass `ys` in one launch: the
-// left-edge tiles play the primal pass's part of the protocol, the right-edge tiles the dual pass's.
-RingHalo BackendPDHG::slab_ring_halo() {
-  RingHalo h;
-  h.has_left = comm_->has_left();
-  h.has_right = comm_->has_right();
-  const unsigned ys_in = comm_->y_seq;               // newest y halo (left neighbour's previous iteration)
-  const unsigned xs = ++comm_->x_seq, ys = ++comm_->y_seq;
-  h.error = &comm_->flags()->error;
-  if (h.has_left) {
-    for (unsigned p = 0; p < 3; ++p) h.yl_ll[p] = comm_->y_ll(p);
-    for (unsigned p = 0; p < 2; ++p) h.x_out_ll[p] = comm_->x_ll_out(p);
-    h.y_wait_seq = ys_in;
-    h.x_signal_seq = xs;
-  }
-  if (h.has_right) {
-    for (unsigned p = 0; p < 2; ++p) h.xr_ll[p] = comm_->x_ll(p);
-    for (unsigned p = 0; p < 3; ++p) h.y_out_ll[p] = comm_->y_ll_out(p);
-    h.x_wait_seq = xs;
-    h.y_signal_seq = ys;
-  }
-  halo_in_ll_ = true;
-  return h;
-}
-
-// Dual pass number `ys`: reads the x columns of the right neighbour's primal passes xs / xs-1,
-// hands the last column of the new x-component of y to the right.
-void BackendPDHG::slab_dual_halo(unsigned xs, unsigned ys) {
-  SlabHalo h;
-  h.has_left = comm_->has_left();
-  h.has_right = comm_->has_right();
-  h.in_a = comm_->x_slot(xs);
-  h.in_b = comm_->x_slot(xs - 1);
-  h.out = comm_->y_out(ys);
-  if (comm_->p2p() && h.has_right) {
-    HaloFlags* f = comm_->flags();
-    h.wait_flag = &f->x_seq;
-    h.wait_seq = xs;
-    h.done_counter = &f->done_dual;
-    h.signal_flag = comm_->right_y_seq();
-    h.signal_seq = ys;
-    h.error = &f->error;
-  }
-  stencil_.geom.halo = h;
 }
 
 // K u / K^T p on the local slab including the neighbours' columns (current_solution only)
@@ -855,20 +781,15 @@ void BackendPDHG::current_solution(float* h_x, float* h_z, float* h_y, float* h_
   if (h_y) download_to_host(ctx_, h_y, y_.data(), m);
   if (h_w || h_z) {
     const ScaleRef T = problem_->right_ref(), S = problem_->left_ref();
-    if (fused_ && comm_ && halo_in_ll_) {
-      // one-pass iterations keep the halo columns in flag-in-data slots; slab_apply reads plain columns
-      comm_->unpack_ll_x(comm_->x_seq);
-      comm_->unpack_ll_x(comm_->x_seq - 1);
-      comm_->unpack_ll_y(comm_->y_seq - 1);
-    }
     if (fused_) {
       // K x, K x_prev and K^T y_prev are not stored in fused mode: rebuild them with the
       // unfused operator, honouring the zero-initialised history of the reference
+      const Comm::PlainHalo halo = comm_ ? comm_->plain_halo() : Comm::PlainHalo();
       if (h_w) {
         const size_t cap = std::max(n, m);       // one allocation serves w (n) and z (m)
         if (sol_a_.size() != cap) { sol_a_.resize(cap); sol_b_.resize(cap); }
         if (iteration_ <= 1) PB_CUDA(cudaMemsetAsync(sol_a_.data(), 0, n * sizeof(float), s));
-        else if (comm_) slab_apply(sol_a_.data(), y_prev_.data(), comm_->y_slot(comm_->y_seq - 1), true);
+        else if (comm_) slab_apply(sol_a_.data(), y_prev_.data(), halo.y_prev, true);
         else problem_->apply_K(sol_a_.data(), y_prev_.data(), true);
         w_variable_kernel<<<sgrid(n), kBlock, 0, s>>>(sol_b_.data(), x_prev_.data(), x_.data(), T,
                                                       sol_a_.data(), n, st.tau);
@@ -880,10 +801,10 @@ void BackendPDHG::current_solution(float* h_x, float* h_z, float* h_y, float* h_
         if (sol_a_.size() != cap) { sol_a_.resize(cap); sol_b_.resize(cap); }
         if (sol_c_.size() != m) sol_c_.resize(m);
         if (iteration_ == 0) PB_CUDA(cudaMemsetAsync(sol_a_.data(), 0, m * sizeof(float), s));
-        else if (comm_) slab_apply(sol_a_.data(), x_.data(), comm_->x_slot(comm_->x_seq), false);
+        else if (comm_) slab_apply(sol_a_.data(), x_.data(), halo.x, false);
         else problem_->apply_K(sol_a_.data(), x_.data(), false);
         if (iteration_ <= 1) PB_CUDA(cudaMemsetAsync(sol_b_.data(), 0, m * sizeof(float), s));
-        else if (comm_) slab_apply(sol_b_.data(), x_prev_.data(), comm_->x_slot(comm_->x_seq - 1), false);
+        else if (comm_) slab_apply(sol_b_.data(), x_prev_.data(), halo.x_prev, false);
         else problem_->apply_K(sol_b_.data(), x_prev_.data(), false);
         z_variable_kernel<<<sgrid(m), kBlock, 0, s>>>(sol_c_.data(), y_prev_.data(), y_.data(), S,
                                                       sol_a_.data(), sol_b_.data(), m, st.sigma, st.theta);

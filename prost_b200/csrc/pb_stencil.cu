@@ -50,7 +50,9 @@ unsigned stencil_dual_norm2_launch_slab(Context*, const GradGeom&, bool three_d,
                                         bool dry_run);
 unsigned stencil_dual_identity_launch(Context*, const GradGeom&, const ProxDesc&, const DualPass&, bool dry_run);
 
-static inline GradGeom with_vec(GradGeom g, int vec) {
+// the plan's geometry for threads of `vec` rows, with the pass's halo
+static inline GradGeom with_vec(GradGeom g, int vec, const SlabHalo* halo) {
+  if (halo) g.halo = *halo;
   g.q = g.ny / vec;
   g.div_q = FastDiv(g.q);
   g.div_nx = FastDiv(g.nx);
@@ -154,7 +156,8 @@ unsigned stencil_primal_launch(Context* ctx, const StencilPlan& plan, const Prox
                                bool dry_run) {
   if (!plan.ok || d.index != 0) return 0;
   const GradGeom& g0 = plan.geom;
-  const bool slab = g0.halo.has_left || g0.halo.has_right;
+  // slab kernels where the pass has a neighbour; a communicator of one rank runs the single-GPU ones
+  const bool slab = p.halo && (p.halo->has_left || p.halo->has_right);
   unsigned grid = 0;
   if (d.kind == kProxSimplex)
     grid = (slab ? stencil_primal_simplex_launch_slab : stencil_primal_simplex_launch_single)(ctx, g0, plan.three_d,
@@ -176,9 +179,9 @@ unsigned PB_FLAVOUR(stencil_primal1_launch)(Context* ctx, const GradGeom& g0, bo
               (!p.T.ptr || aligned16(p.T.ptr)) && (!g0.has_id || g0.id_row % 4 == 0);
   for (int k = 0; k < 7; ++k)
     if (d.coeffs.ptr[k] && !aligned16(d.coeffs.ptr[k])) vec4 = false;
-  if (g0.halo.has_left && vec4 && !aligned16(g0.halo.out)) vec4 = false;
+  if (p.halo && p.halo->has_left && vec4 && !aligned16(p.halo->out)) vec4 = false;
   const int vec = vec4 ? 4 : 1;
-  GradGeom g = with_vec(g0, vec);
+  GradGeom g = with_vec(g0, vec, p.halo);
   g.halo.n_edge_ctas = count_edge_ctas(g.q, g.L);
   const unsigned grid = grid_threads((size_t)g.q * g.nx * g.L);
   if (dry_run || grid == 0) return grid;
@@ -207,7 +210,7 @@ unsigned stencil_dual_launch(Context* ctx, const StencilPlan& plan, const ProxDe
                              bool dry_run) {
   if (!plan.ok) return 0;
   const GradGeom& g = plan.geom;
-  const bool slab = g.halo.has_left || g.halo.has_right;
+  const bool slab = p.halo && (p.halo->has_left || p.halo->has_right);
   const uint32_t grad_rows = (plan.three_d ? 3u : 2u) * g.plane;
   unsigned grid = 0;
   if (d.index == 0 && d.kind == kProxNorm2 && (size_t)d.count * d.dim == grad_rows)
@@ -268,7 +271,7 @@ unsigned PB_FLAVOUR(stencil_primal_simplex_launch)(Context* ctx, const GradGeom&
   // simplex over the labels of a pixel: planar, count = nx*ny, dim = L (2-D gradient only)
   if (three_d || d.interleaved || d.moreau || d.count != g0.nxny || d.dim != g0.L || g0.L < 2 || g0.L > 32)
     return 0;
-  GradGeom g = with_vec(g0, 1);
+  GradGeom g = with_vec(g0, 1, p.halo);
   const int cap = g.L <= 4 ? 4 : g.L <= 8 ? 8 : g.L <= 16 ? 16 : 32;
   // operands staged through shared memory (every iteration but the first, uniform T)
   if (!p.kty_zero && !p.T.ptr) {
@@ -366,13 +369,13 @@ unsigned PB_FLAVOUR(stencil_dual_norm2_launch)(Context* ctx, const GradGeom& g0,
   for (int k = 0; k < 7; ++k)
     if (d.coeffs.ptr[k] && !aligned16(d.coeffs.ptr[k])) vec4 = false;
   if (per_pixel && g0.L > 4) vec4 = false;             // keep the group within the register budget
-  if (g0.halo.has_right && vec4 && !aligned16(g0.halo.out)) vec4 = false;
+  if (p.halo && p.halo->has_right && vec4 && !aligned16(p.halo->out)) vec4 = false;
   // per-pixel groups over more than 4 labels, scalar weights, uniform Sigma on these rows: operands staged
   // through shared memory (pb_stencil_staged.cuh)
   bool scalar_coeffs = !d.moreau && !p.S.ptr;
   for (int k = 0; k < 7; ++k) scalar_coeffs = scalar_coeffs && !d.coeffs.ptr[k];
   if (per_pixel && g0.L > 4 && scalar_coeffs) {
-    GradGeom gs = with_vec(g0, 1);
+    GradGeom gs = with_vec(g0, 1, p.halo);
     const unsigned sgrid = staged_grid((size_t)gs.q * gs.nx);
     if (dry_run || sgrid == 0) return sgrid;
     gs.halo.n_edge_ctas = staged_grid(gs.q);
@@ -383,7 +386,7 @@ unsigned PB_FLAVOUR(stencil_dual_norm2_launch)(Context* ctx, const GradGeom& g0,
     if (launched) return sgrid;
   }
   const int vec = vec4 ? 4 : 1;
-  GradGeom g = with_vec(g0, vec);
+  GradGeom g = with_vec(g0, vec, p.halo);
   g.halo.n_edge_ctas = count_edge_ctas(g.q, per_voxel ? g.L : 1u);
   const unsigned grid = grid_threads((size_t)g.q * g.nx * (per_voxel ? g.L : 1u));
   if (dry_run || grid == 0) return grid;

@@ -24,67 +24,13 @@
 #pragma once
 
 #include "pb_backend.cuh"
+#include "pb_comm.cuh"
 #include "pb_crosssum.cuh"
 #include "pb_fused.cuh"
 #include "pb_prox.cuh"
 #include "pb_reduce.cuh"
 
 namespace pb {
-
-// Slab decomposition along x (SURVEY.md 8(e)): the local grid is a block of columns of a wider
-// image.  The primal pass talks to the LEFT neighbour through its column x = 0 (it needs the
-// neighbour's last column of the x-component of y for the divergence and hands over its new
-// column 0 of x); the dual pass talks to the RIGHT neighbour through its column x = nx-1 (it needs
-// the neighbour's first column of x_new / x_old for the forward difference and hands over its new
-// last column of the x-component of y).  `in_a / in_b` are the received columns of the pass's two
-// stencil operands (primal: y, y_prev; dual: x_new, x_old), laid out  y + l*ny.  `out` is where the
-// outgoing column goes: the neighbour's slot mapped over NVLink (peer-to-peer mode) or a local
-// staging buffer (NCCL mode, all flag pointers null).  See pb_comm.cuh for the protocol.
-struct SlabHalo {
-  int has_left = 0, has_right = 0;
-  const float* in_a = nullptr;
-  const float* in_b = nullptr;
-  float* out = nullptr;
-  const unsigned* wait_flag = nullptr;   // local sequence word the neighbour publishes to
-  unsigned wait_seq = 0;                 // edge threads spin until *wait_flag >= wait_seq (0: no wait)
-  unsigned* done_counter = nullptr;      // local: counts finished edge CTAs of this launch
-  unsigned n_edge_ctas = 0;
-  unsigned* signal_flag = nullptr;       // neighbour's sequence word (peer memory)
-  unsigned signal_seq = 0;
-  int* error = nullptr;                  // set when a wait times out
-};
-
-// Halo descriptor of the one-pass ring kernel (pb_tile.cu) on a slab: ONE launch does the primal and the dual
-// step, so it talks to both neighbours.  Its edge columns travel in a flag-in-data layout ("LL", as in NCCL's
-// low-latency protocol): every group of four rows is two 16-byte lines {v0, seq, v1, seq} {v2, seq, v3, seq},
-// each 8-byte half carrying the sequence number of the iteration that produced it.  The producer's edge warp
-// stores the lines straight into the neighbour's memory over NVLink (8-byte halves arrive atomically); the
-// consumer's edge warp polls the two lines of ITS rows until all four tags match -- no system-scope fence, no
-// edge-tile counter and no separate flag sit between the neighbour's store and this GPU's load (round 1 paid a
-// fence.sys on the compute path plus a counter and a flag hop per edge and iteration, profiles/r01_scaling.md).
-//   left edge  (tiles of column 0): waits for the left neighbour's newest y.gx column nx-1 (sequence
-//              y_wait_seq, produced by its PREVIOUS iteration) row group by row group, computes column 0 and
-//              stores its new x column 0 into the left neighbour's x slot tagged x_signal_seq;
-//   right edge (tiles owning column nx-1): waits for the right neighbour's new x column 0 of THIS iteration
-//              (x_wait_seq; the previous iterate's column is still in the other slot), stores its new y.gx
-//              column nx-1 into the right neighbour's y slot tagged y_signal_seq.
-// Slot reuse: x has two slots (sequence & 1), y three (sequence % 3: the residual-refresh launch also reads the
-// y column before the newest one).  A row group is overwritten only by a thread that has already consumed what
-// the overwritten data fed (x: the producer of x(s+2)[r] has seen y(s+1)[r], whose producer had read x(s)[r];
-// y(s+3)[r] needs x(s+3)[r], i.e. the neighbour has started launch s+3 and finished every read of launch s+2).
-// The left-edge tile column is walked first and the right-edge one in the second wave (pb_tile.cu: decode), so
-// in steady state the columns arrive before they are needed.
-struct RingHalo {
-  int has_left = 0, has_right = 0;
-  const uint4* yl_ll[3] = {nullptr, nullptr, nullptr};   // local y slots by (sequence % 3), written by the left rank
-  const uint4* xr_ll[2] = {nullptr, nullptr};            // local x slots by (sequence & 1), written by the right rank
-  uint4* x_out_ll[2] = {nullptr, nullptr};               // the left neighbour's x slots
-  uint4* y_out_ll[3] = {nullptr, nullptr, nullptr};      // the right neighbour's y slots
-  unsigned y_wait_seq = 0;             // newest y column from the left (0: none yet)
-  unsigned x_wait_seq = 0;             // x column of this iteration from the right
-  unsigned x_signal_seq = 0, y_signal_seq = 0;
-  int* error = nullptr;                // set when a wait times out
-};
 
 // Residual-refresh launches of the ring kernel finish the iteration themselves: the last CTA to arrive (ticket)
 // folds the per-CTA partial sums in index order, on slabs combines them across ranks through peer-mapped slots
@@ -125,7 +71,7 @@ struct GradGeom {
   int has_id = 0;                 // identity block  id_factor * I  at rows [id_row, id_row + plane)
   uint32_t id_row = 0;
   float id_factor = 1.f;
-  SlabHalo halo;                  // all zero on a single GPU
+  SlabHalo halo;                  // the pass's PrimalPass / DualPass::halo, all zero on a single GPU
 };
 
 constexpr int kStencilBlock = 128;

@@ -137,7 +137,7 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
-// ---- flag-in-data halo lines (RingHalo, pb_stencil.cuh) --------------------------------------------------------
+// ---- flag-in-data halo lines (RingHalo, pb_comm.cuh) -----------------------------------------------------------
 // four rows = two 16-byte lines {v0, seq, v1, seq} {v2, seq, v3, seq}; volatile accesses go to L2, the point of
 // coherence for the neighbour's NVLink stores
 __device__ __forceinline__ void ll_ld_line(const uint4* p, uint4& v) {
