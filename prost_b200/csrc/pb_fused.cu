@@ -18,6 +18,7 @@ unsigned fused_grid(Context* ctx, const ProxDesc& d) {
 unsigned fused_primal_launch(Context* ctx, const ProxDesc& d, const BlockList& bl, const PrimalPass& p) {
   if (d.count == 0) return 0;
   const unsigned grid = fused_grid(ctx, d);
+  check_partials_fit(p.check, grid, p.partials_cap);
 #define PB_CASE(N) case N: fused_primal_cap<N>(ctx, grid, d, bl, p); break;
   switch (dim_cap(d.dim, d.kind)) {
     PB_CASE(1) PB_CASE(2) PB_CASE(4) PB_CASE(8) PB_CASE(16) PB_CASE(32) PB_CASE(64)
@@ -32,6 +33,7 @@ unsigned fused_primal_launch(Context* ctx, const ProxDesc& d, const BlockList& b
 unsigned fused_dual_launch(Context* ctx, const ProxDesc& d, const BlockList& bl, const DualPass& p) {
   if (d.count == 0) return 0;
   const unsigned grid = fused_grid(ctx, d);
+  check_partials_fit(p.check, grid, p.partials_cap);
 #define PB_CASE(N) case N: fused_dual_cap<N>(ctx, grid, d, bl, p); break;
   switch (dim_cap(d.dim, d.kind)) {
     PB_CASE(1) PB_CASE(2) PB_CASE(4) PB_CASE(8) PB_CASE(16) PB_CASE(32) PB_CASE(64)

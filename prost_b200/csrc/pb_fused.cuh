@@ -170,6 +170,7 @@ struct PrimalPass {
   const PdhgState* st = nullptr;
   bool kty_zero = false, ktyprev_zero = false, check = false;
   double* partials = nullptr;         // 2 doubles per CTA, check only
+  unsigned partials_cap = 0;          // (a, b) pairs left at partials
   float* x_out = nullptr;
   const SlabHalo* halo = nullptr;
 };
@@ -184,11 +185,20 @@ struct DualPass {
   const PdhgState* st = nullptr;
   bool kxprev_zero = false, check = false;
   double* partials = nullptr;         // 2 doubles per CTA, check only
+  unsigned partials_cap = 0;          // (a, b) pairs left at partials
   float* y_out = nullptr;
   const SlabHalo* halo = nullptr;
 };
 
-// Host-side launchers (pb_fused.cu).  `partials` must hold 2*grid doubles; returns the grid size.
+// A residual-refresh pass writes one (a, b) pair per CTA at its partials: refuses a grid that would write past the
+// `cap` pairs left there.
+inline void check_partials_fit(bool check, unsigned grid, unsigned cap) {
+  if (check && grid > cap)
+    fail(PB_ERR_CUDA, "residual-refresh pass of " + std::to_string(grid) + " CTAs has room for only " +
+                          std::to_string(cap) + " partial sums");
+}
+
+// Host-side launchers (pb_fused.cu); return the grid size.
 unsigned fused_primal_launch(Context* ctx, const ProxDesc& d, const BlockList& bl, const PrimalPass& p);
 unsigned fused_dual_launch(Context* ctx, const ProxDesc& d, const BlockList& bl, const DualPass& p);
 unsigned fused_grid(Context* ctx, const ProxDesc& d);

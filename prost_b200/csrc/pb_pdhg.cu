@@ -385,10 +385,9 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
   vote(!(ny0 > 0 && ny0 != m), PB_ERR_INVALID, "Initial dual solution has wrong size.");
 
   { PB_TRACE_SCOPE("  plan_fused"); fused_ = plan_fused(); }
-  // one-pass iterations run the ring kernel only: its dry run decides here, a launch that fails later is an error
+  // one-pass iterations run the ring kernel only: whether it can is decided here, a launch that fails later is an error
   tile_ok_ = fused_ && opts_.fuse == 1 &&
-             tile_iteration_supported(stencil_, g_descs_, f_descs_, problem_->right_ref(), problem_->left_ref()) &&
-             tile_ring_available(ctx_, stencil_, g_descs_[0], f_descs_[0], comm_ != nullptr);
+             tile_ring_available(stencil_, g_descs_, f_descs_, problem_->right_ref(), problem_->left_ref(), comm_ != nullptr);
   // slabs: the one-pass kernel stores its edge columns straight into the neighbours' memory, so it
   // needs the peer-to-peer halo blocks
   if (comm_) tile_ok_ = tile_ok_ && stencil_.geom.nx >= 2;
@@ -396,16 +395,11 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
   if (comm_) {
     // the halo protocol lives in the specialised stencil passes: one planar gradient operator
     // (+ identity rows), one prox_g over all columns, Norm2 on the gradient rows
-    PrimalPass pp;                     // dry runs: is there a specialised pass for each prox?
-    pp.T = problem_->right_ref();
-    DualPass dp;
-    dp.S = problem_->left_ref();
-    bool ok = fused_ && stencil_.ok && g_descs_.size() == 1;
-    if (ok) ok = stencil_primal_launch(ctx_, stencil_, g_descs_[0], pp, true) > 0;
+    bool ok = fused_ && g_descs_.size() == 1 && stencil_primal_cover(stencil_, g_descs_[0]) > 0;
     int halo_passes = 0;
     for (auto& d : f_descs_) {
       if (!ok) break;
-      ok = stencil_dual_launch(ctx_, stencil_, d, dp, true) > 0;
+      ok = stencil_dual_cover(ctx_, stencil_, d) > 0;
       if (d.index == 0) ++halo_passes;
     }
     ok = ok && halo_passes == 1;
@@ -461,20 +455,11 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
   // partial-sum buffers: one (a, b) pair per CTA of every launch of a pass
   if (fused_) {
     part_d_cap_ = part_p_cap_ = 0;
-    // dry runs of residual-refresh passes over the iterates' buffers (the grid depends on their alignment)
-    PrimalPass pp;
-    pp.x = x_.data(); pp.y = y_.data(); pp.y_prev = y_prev_.data(); pp.check = true; pp.x_out = x_prev_.data();
-    for (size_t i = 0; i < g_descs_.size(); ++i) {
-      const ProxDesc& d = g_descs_[i];
-      pp.T = g_scale_[i];
-      part_d_cap_ += std::max(stencil_primal_launch(ctx_, stencil_, d, pp, true), fused_grid(ctx_, d));
-    }
-    DualPass dp;
-    dp.y = y_.data(); dp.x_new = x_.data(); dp.x_old = x_prev_.data(); dp.check = true; dp.y_out = y_prev_.data();
-    for (size_t i = 0; i < f_descs_.size(); ++i) {
-      const ProxDesc& d = f_descs_[i];
-      dp.S = f_scale_[i];
-      part_p_cap_ += std::max(stencil_dual_launch(ctx_, stencil_, d, dp, true), fused_grid(ctx_, d));
+    for (auto& d : g_descs_) part_d_cap_ += std::max(stencil_primal_cover(stencil_, d), fused_grid(ctx_, d));
+    for (auto& d : f_descs_) part_p_cap_ += std::max(stencil_dual_cover(ctx_, stencil_, d), fused_grid(ctx_, d));
+    if (tile_ok_) {
+      part_d_cap_ = std::max(part_d_cap_, tile_ring_grid(ctx_, stencil_));
+      part_p_cap_ = std::max(part_p_cap_, tile_ring_grid(ctx_, stencil_));
     }
   } else {
     part_p_cap_ = std::min<size_t>(grid_for(m), (size_t)ctx_->num_sms * 8);
@@ -512,7 +497,7 @@ void BackendPDHG::iteration_fused() {
       tp.check = true;
       tp.y_prev = y_prev_.data();
       tp.ktyprev_zero = iteration_ <= 1;
-      tp.part_d = part_d_.data(); tp.part_p = part_p_.data();
+      tp.part_d = part_d_.data(); tp.part_p = part_p_.data(); tp.part_cap = std::min(part_d_cap_, part_p_cap_);
       // y^{k+1} cannot overwrite y_prev_ (the pass reads y^{k-1} from it), so it goes to a third buffer that
       // then takes y_prev_'s place
       tp.y_out = y_prev_staging();
@@ -543,6 +528,7 @@ void BackendPDHG::iteration_fused() {
       const ProxDesc& d = g_descs_[i];
       pp.T = g_scale_[i];
       pp.partials = part_d_.data() + 2 * (size_t)off;
+      pp.partials_cap = part_d_cap_ - off;
       unsigned g = stencil_primal_launch(ctx_, stencil_, d, pp);
       if (g == 0) g = fused_primal_launch(ctx_, d, blocks_, pp);
       off += g;
@@ -563,6 +549,7 @@ void BackendPDHG::iteration_fused() {
       const ProxDesc& d = f_descs_[i];
       dp.S = f_scale_[i];
       dp.partials = part_p_.data() + 2 * (size_t)off;
+      dp.partials_cap = part_p_cap_ - off;
       unsigned g = stencil_dual_launch(ctx_, stencil_, d, dp);
       if (g == 0) g = fused_dual_launch(ctx_, d, blocks_, dp);
       off += g;

@@ -34,21 +34,17 @@ constexpr bool kSlab = PB_STENCIL_SLAB != 0;
 #define PB_FLAVOUR(name) name##_single
 #endif
 
-// Each returns the grid it launched, or would launch when dry_run, and 0 when it does not cover the pass; the
-// caller (stencil_primal_launch / stencil_dual_launch) checks and counts the launch.
-unsigned stencil_primal1_launch_single(Context*, const GradGeom&, bool three_d, const ProxDesc&, const PrimalPass&,
-                                       bool dry_run);
-unsigned stencil_primal1_launch_slab(Context*, const GradGeom&, bool three_d, const ProxDesc&, const PrimalPass&,
-                                     bool dry_run);
+// Each launches the pass of a prox that stencil_primal_cover / stencil_dual_cover assigned to it and returns the
+// grid; the caller (stencil_primal_launch / stencil_dual_launch) checks and counts the launch.
+unsigned stencil_primal1_launch_single(Context*, const GradGeom&, bool three_d, const ProxDesc&, const PrimalPass&);
+unsigned stencil_primal1_launch_slab(Context*, const GradGeom&, bool three_d, const ProxDesc&, const PrimalPass&);
 unsigned stencil_primal_simplex_launch_single(Context*, const GradGeom&, bool three_d, const ProxDesc&,
-                                              const PrimalPass&, bool dry_run);
+                                              const PrimalPass&);
 unsigned stencil_primal_simplex_launch_slab(Context*, const GradGeom&, bool three_d, const ProxDesc&,
-                                            const PrimalPass&, bool dry_run);
-unsigned stencil_dual_norm2_launch_single(Context*, const GradGeom&, bool three_d, const ProxDesc&, const DualPass&,
-                                          bool dry_run);
-unsigned stencil_dual_norm2_launch_slab(Context*, const GradGeom&, bool three_d, const ProxDesc&, const DualPass&,
-                                        bool dry_run);
-unsigned stencil_dual_identity_launch(Context*, const GradGeom&, const ProxDesc&, const DualPass&, bool dry_run);
+                                            const PrimalPass&);
+unsigned stencil_dual_norm2_launch_single(Context*, const GradGeom&, bool three_d, const ProxDesc&, const DualPass&);
+unsigned stencil_dual_norm2_launch_slab(Context*, const GradGeom&, bool three_d, const ProxDesc&, const DualPass&);
+unsigned stencil_dual_identity_launch(Context*, const GradGeom&, const ProxDesc&, const DualPass&);
 
 // the plan's geometry for threads of `vec` rows, with the pass's halo
 static inline GradGeom with_vec(GradGeom g, int vec, const SlabHalo* halo) {
@@ -65,10 +61,18 @@ static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t
 static inline unsigned grid_threads(size_t threads) {
   return (unsigned)((threads + kStencilBlock - 1) / kStencilBlock);
 }
+// threads of `vec` rows over n_l label planes of every column
+static inline unsigned stencil_grid(const GradGeom& g, int vec, uint32_t n_l) {
+  return grid_threads((size_t)(g.ny / vec) * g.nx * n_l);
+}
 
 // per-pixel label groups: operands staged through shared memory (pb_stencil_staged.cuh)
 static inline unsigned staged_grid(size_t threads) {
   return (unsigned)((threads + kStagedBlock - 1) / kStagedBlock);
+}
+
+static inline unsigned identity_grid(const Context* ctx, const ProxDesc& d) {
+  return (unsigned)std::min<size_t>(grid_for(d.count), (size_t)ctx->num_sms * 16);
 }
 template <class Kernel>
 static bool staged_configure(Kernel kernel, size_t smem) {
@@ -95,6 +99,7 @@ template <int VEC, int CAPL, int KIND, int FN, bool THREE_D, bool HAS_ID>
 static void primal_launch(Context* ctx, unsigned grid, const GradGeom& g, const ProxDesc& d, const PrimalPass& p) {
   auto kernel = p.check ? grad_primal_kernel<VEC, CAPL, KIND, FN, THREE_D, HAS_ID, true, kSlab>
                         : grad_primal_kernel<VEC, CAPL, KIND, FN, THREE_D, HAS_ID, false, kSlab>;
+  check_partials_fit(p.check, grid, p.partials_cap);
   kernel<<<grid, kStencilBlock, 0, ctx->stream>>>(g, d, p.x, p.y, p.y_prev, p.T, p.st, p.kty_zero, p.ktyprev_zero,
                                                   p.partials, p.x_out);
 }
@@ -152,29 +157,54 @@ static void primal1_geom(Context* ctx, unsigned grid, const GradGeom& g, bool th
 }
 
 #if !PB_STENCIL_SLAB
-unsigned stencil_primal_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& d, const PrimalPass& p,
-                               bool dry_run) {
-  if (!plan.ok || d.index != 0) return 0;
-  const GradGeom& g0 = plan.geom;
+unsigned stencil_primal_cover(const StencilPlan& plan, const ProxDesc& d) {
+  const GradGeom& g = plan.geom;
+  if (!plan.ok || d.index != 0 || d.count == 0) return 0;
+  // one-element groups over every voxel
+  if (d.kind == kProxElem1D || d.kind == kProxZero) return d.dim == 1 && d.count == g.plane ? stencil_grid(g, 1, g.L) : 0;
+  // simplex over the labels of a pixel: planar, count = nx*ny, dim = L (2-D gradient only)
+  if (d.kind == kProxSimplex && !plan.three_d && !d.interleaved && !d.moreau && d.count == g.nxny && d.dim == g.L &&
+      g.L >= 2 && g.L <= 32)
+    return std::max(staged_grid(g.nxny), stencil_grid(g, 1, 1));
+  return 0;
+}
+
+unsigned stencil_dual_cover(const Context* ctx, const StencilPlan& plan, const ProxDesc& d) {
+  const GradGeom& g = plan.geom;
+  if (!plan.ok || d.count == 0) return 0;
+  const uint32_t ncomp = plan.three_d ? 3u : 2u;
+  if (d.index == 0 && d.kind == kProxNorm2 && (size_t)d.count * d.dim == ncomp * g.plane) {
+    if (d.interleaved) return 0;
+    // the gradient components of a voxel
+    if (d.count == g.plane && d.dim == ncomp) return stencil_grid(g, 1, g.L);
+    // those of all labels of a pixel (2-D); staged through shared memory above 4 labels
+    if (plan.three_d || g.L <= 1 || g.L > 32 || d.count != g.nxny || d.dim != ncomp * g.L) return 0;
+    return g.L > 4 ? std::max(staged_grid(g.nxny), stencil_grid(g, 1, 1)) : stencil_grid(g, 1, 1);
+  }
+  // the identity rows: a leaf prox held in at most 8 registers
+  const int cap = dim_cap(d.dim, d.kind);
+  if (g.has_id && d.index == g.id_row && (size_t)d.count * d.dim == g.plane && cap > 0 && cap <= 8)
+    return identity_grid(ctx, d);
+  return 0;
+}
+
+unsigned stencil_primal_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& d, const PrimalPass& p) {
+  if (!stencil_primal_cover(plan, d)) return 0;
   // slab kernels where the pass has a neighbour; a communicator of one rank runs the single-GPU ones
   const bool slab = p.halo && (p.halo->has_left || p.halo->has_right);
-  unsigned grid = 0;
-  if (d.kind == kProxSimplex)
-    grid = (slab ? stencil_primal_simplex_launch_slab : stencil_primal_simplex_launch_single)(ctx, g0, plan.three_d,
-                                                                                              d, p, dry_run);
-  else if (d.kind == kProxElem1D || d.kind == kProxZero)
-    grid = (slab ? stencil_primal1_launch_slab : stencil_primal1_launch_single)(ctx, g0, plan.three_d, d, p, dry_run);
-  if (grid && !dry_run) {
-    PB_CHECK_LAUNCH();
-    ctx->launches++;
-  }
+  const unsigned grid =
+      d.kind == kProxSimplex
+          ? (slab ? stencil_primal_simplex_launch_slab : stencil_primal_simplex_launch_single)(ctx, plan.geom,
+                                                                                               plan.three_d, d, p)
+          : (slab ? stencil_primal1_launch_slab : stencil_primal1_launch_single)(ctx, plan.geom, plan.three_d, d, p);
+  PB_CHECK_LAUNCH();
+  ctx->launches++;
   return grid;
 }
 #endif  // !PB_STENCIL_SLAB
 
 unsigned PB_FLAVOUR(stencil_primal1_launch)(Context* ctx, const GradGeom& g0, bool three_d, const ProxDesc& d,
-                                            const PrimalPass& p, bool dry_run) {
-  if (d.dim != 1 || d.count != g0.plane) return 0;
+                                            const PrimalPass& p) {
   bool vec4 = (g0.ny % 4 == 0) && aligned16(p.x) && aligned16(p.y) && aligned16(p.y_prev) && aligned16(p.x_out) &&
               (!p.T.ptr || aligned16(p.T.ptr)) && (!g0.has_id || g0.id_row % 4 == 0);
   for (int k = 0; k < 7; ++k)
@@ -183,8 +213,7 @@ unsigned PB_FLAVOUR(stencil_primal1_launch)(Context* ctx, const GradGeom& g0, bo
   const int vec = vec4 ? 4 : 1;
   GradGeom g = with_vec(g0, vec, p.halo);
   g.halo.n_edge_ctas = count_edge_ctas(g.q, g.L);
-  const unsigned grid = grid_threads((size_t)g.q * g.nx * g.L);
-  if (dry_run || grid == 0) return grid;
+  const unsigned grid = stencil_grid(g, vec, g.L);
   // Function1D members with their own instantiation (the data terms of the reference's examples:
   // quadratic for ROF, abs for TV-L1); every other member dispatches at run time (FN = -1)
   if (d.kind == kProxElem1D) {
@@ -206,22 +235,16 @@ unsigned PB_FLAVOUR(stencil_primal1_launch)(Context* ctx, const GradGeom& g0, bo
 }
 
 #if !PB_STENCIL_SLAB
-unsigned stencil_dual_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& d, const DualPass& p,
-                             bool dry_run) {
-  if (!plan.ok) return 0;
-  const GradGeom& g = plan.geom;
+unsigned stencil_dual_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& d, const DualPass& p) {
+  if (!stencil_dual_cover(ctx, plan, d)) return 0;
   const bool slab = p.halo && (p.halo->has_left || p.halo->has_right);
-  const uint32_t grad_rows = (plan.three_d ? 3u : 2u) * g.plane;
-  unsigned grid = 0;
-  if (d.index == 0 && d.kind == kProxNorm2 && (size_t)d.count * d.dim == grad_rows)
-    grid = (slab ? stencil_dual_norm2_launch_slab : stencil_dual_norm2_launch_single)(ctx, g, plan.three_d, d, p,
-                                                                                      dry_run);
-  else if (g.has_id && d.index == g.id_row && (size_t)d.count * d.dim == g.plane)
-    grid = stencil_dual_identity_launch(ctx, g, d, p, dry_run);
-  if (grid && !dry_run) {
-    PB_CHECK_LAUNCH();
-    ctx->launches++;
-  }
+  // Norm2 on the gradient rows, otherwise the identity rows
+  const unsigned grid =
+      d.index == 0 && d.kind == kProxNorm2
+          ? (slab ? stencil_dual_norm2_launch_slab : stencil_dual_norm2_launch_single)(ctx, plan.geom, plan.three_d, d, p)
+          : stencil_dual_identity_launch(ctx, plan.geom, d, p);
+  PB_CHECK_LAUNCH();
+  ctx->launches++;
   return grid;
 }
 #endif  // !PB_STENCIL_SLAB
@@ -233,6 +256,7 @@ static bool simplex_staged_launch_k(Context* ctx, unsigned grid, const GradGeom&
                                     const PrimalPass& p) {
   constexpr int LC = CAPL < kStagedChunk ? CAPL : kStagedChunk;
   auto launch = [&](auto kernel, size_t smem) {
+    check_partials_fit(CHECK, grid, p.partials_cap);
     kernel<<<grid, kStagedBlock, smem, ctx->stream>>>(g, d, p.x, p.y, p.y_prev, p.T.val, p.st, p.ktyprev_zero ? 1 : 0,
                                                       p.partials, p.x_out);
   };
@@ -266,17 +290,13 @@ static bool simplex_staged_launch(Context* ctx, unsigned grid, const GradGeom& g
                  : simplex_staged_launch_k<CAPL, false, false>(ctx, grid, g, d, p);
 }
 
-unsigned PB_FLAVOUR(stencil_primal_simplex_launch)(Context* ctx, const GradGeom& g0, bool three_d, const ProxDesc& d,
-                                                   const PrimalPass& p, bool dry_run) {
-  // simplex over the labels of a pixel: planar, count = nx*ny, dim = L (2-D gradient only)
-  if (three_d || d.interleaved || d.moreau || d.count != g0.nxny || d.dim != g0.L || g0.L < 2 || g0.L > 32)
-    return 0;
+unsigned PB_FLAVOUR(stencil_primal_simplex_launch)(Context* ctx, const GradGeom& g0, bool, const ProxDesc& d,
+                                                   const PrimalPass& p) {
   GradGeom g = with_vec(g0, 1, p.halo);
   const int cap = g.L <= 4 ? 4 : g.L <= 8 ? 8 : g.L <= 16 ? 16 : 32;
   // operands staged through shared memory (every iteration but the first, uniform T)
   if (!p.kty_zero && !p.T.ptr) {
-    const unsigned sgrid = staged_grid((size_t)g.q * g.nx);
-    if (dry_run || sgrid == 0) return sgrid;
+    const unsigned sgrid = staged_grid(g.nxny);
     g.halo.n_edge_ctas = staged_grid(g.q);
     bool launched = false;
     switch (cap) {
@@ -288,8 +308,7 @@ unsigned PB_FLAVOUR(stencil_primal_simplex_launch)(Context* ctx, const GradGeom&
     if (launched) return sgrid;
   }
   g.halo.n_edge_ctas = count_edge_ctas(g.q, 1);
-  const unsigned grid = grid_threads((size_t)g.q * g.nx);
-  if (dry_run || grid == 0) return grid;
+  const unsigned grid = stencil_grid(g, 1, 1);
 #define PB_CASE(C)                                                                      \
   case C:                                                                               \
     if (g.has_id) primal_launch<1, C, kProxSimplex, -1, false, true>(ctx, grid, g, d, p); \
@@ -307,6 +326,7 @@ static bool dual_staged_launch_k(Context* ctx, unsigned grid, const GradGeom& g,
                                  const DualPass& p) {
   constexpr int LC = CAPL < kStagedChunk ? CAPL : kStagedChunk;
   auto launch = [&](auto kernel, size_t smem) {
+    check_partials_fit(CHECK, grid, p.partials_cap);
     kernel<<<grid, kStagedBlock, smem, ctx->stream>>>(g, d, p.y, p.x_new, p.x_old, p.S.val, p.st, p.kxprev_zero ? 1 : 0,
                                                       p.partials, p.y_out);
   };
@@ -344,6 +364,7 @@ template <int VEC, int CAPL, int FN, bool THREE_D>
 static void dual_launch_fn(Context* ctx, unsigned grid, const GradGeom& g, const ProxDesc& d, const DualPass& p) {
   auto kernel = p.check ? grad_dual_norm2_kernel<VEC, CAPL, FN, THREE_D, true, kSlab>
                         : grad_dual_norm2_kernel<VEC, CAPL, FN, THREE_D, false, kSlab>;
+  check_partials_fit(p.check, grid, p.partials_cap);
   kernel<<<grid, kStencilBlock, 0, ctx->stream>>>(g, d, p.y, p.x_new, p.x_old, p.S, p.st, p.kxprev_zero, p.partials,
                                                   p.y_out);
 }
@@ -358,12 +379,8 @@ static void dual_launch(Context* ctx, unsigned grid, const GradGeom& g, const Pr
 }
 
 unsigned PB_FLAVOUR(stencil_dual_norm2_launch)(Context* ctx, const GradGeom& g0, bool three_d, const ProxDesc& d,
-                                               const DualPass& p, bool dry_run) {
-  if (d.interleaved) return 0;
-  const uint32_t ncomp = three_d ? 3u : 2u;
-  const bool per_voxel = d.count == g0.plane && d.dim == ncomp;
-  const bool per_pixel = !three_d && g0.L > 1 && d.count == g0.nxny && d.dim == ncomp * g0.L && g0.L <= 32;
-  if (!per_voxel && !per_pixel) return 0;
+                                               const DualPass& p) {
+  const bool per_voxel = d.count == g0.plane && d.dim == (three_d ? 3u : 2u), per_pixel = !per_voxel;
   bool vec4 = (g0.ny % 4 == 0) && aligned16(p.y) && aligned16(p.x_new) && aligned16(p.x_old) && aligned16(p.y_out) &&
               (!p.S.ptr || aligned16(p.S.ptr)) && (g0.plane % 4 == 0);
   for (int k = 0; k < 7; ++k)
@@ -376,8 +393,7 @@ unsigned PB_FLAVOUR(stencil_dual_norm2_launch)(Context* ctx, const GradGeom& g0,
   for (int k = 0; k < 7; ++k) scalar_coeffs = scalar_coeffs && !d.coeffs.ptr[k];
   if (per_pixel && g0.L > 4 && scalar_coeffs) {
     GradGeom gs = with_vec(g0, 1, p.halo);
-    const unsigned sgrid = staged_grid((size_t)gs.q * gs.nx);
-    if (dry_run || sgrid == 0) return sgrid;
+    const unsigned sgrid = staged_grid(gs.nxny);
     gs.halo.n_edge_ctas = staged_grid(gs.q);
     bool launched = false;
     if (gs.L <= 8) launched = dual_staged_launch<8>(ctx, sgrid, gs, d, p);
@@ -388,8 +404,7 @@ unsigned PB_FLAVOUR(stencil_dual_norm2_launch)(Context* ctx, const GradGeom& g0,
   const int vec = vec4 ? 4 : 1;
   GradGeom g = with_vec(g0, vec, p.halo);
   g.halo.n_edge_ctas = count_edge_ctas(g.q, per_voxel ? g.L : 1u);
-  const unsigned grid = grid_threads((size_t)g.q * g.nx * (per_voxel ? g.L : 1u));
-  if (dry_run || grid == 0) return grid;
+  const unsigned grid = stencil_grid(g, vec, per_voxel ? g.L : 1u);
   if (per_voxel) {
     if (three_d) {
       if (vec == 4) dual_launch<4, 1, true>(ctx, grid, g, d, p);
@@ -454,13 +469,10 @@ static void ident_launch(Context* ctx, unsigned grid, const GradGeom& g, const P
   else ident_launch_k<CAP, -1>(ctx, grid, g, d, p);
 }
 
-unsigned stencil_dual_identity_launch(Context* ctx, const GradGeom& g, const ProxDesc& d, const DualPass& p,
-                                      bool dry_run) {
-  const int cap = dim_cap(d.dim, d.kind);
-  if (cap == 0 || cap > 8) return 0;
-  const unsigned grid = (unsigned)std::min<size_t>(grid_for(d.count), (size_t)ctx->num_sms * 16);
-  if (dry_run || d.count == 0) return d.count ? grid : 0;
-  switch (cap) {
+unsigned stencil_dual_identity_launch(Context* ctx, const GradGeom& g, const ProxDesc& d, const DualPass& p) {
+  const unsigned grid = identity_grid(ctx, d);
+  check_partials_fit(p.check, grid, p.partials_cap);
+  switch (dim_cap(d.dim, d.kind)) {
     case 1: ident_launch<1>(ctx, grid, g, d, p); break;
     case 2: ident_launch<2>(ctx, grid, g, d, p); break;
     case 4: ident_launch<4>(ctx, grid, g, d, p); break;

@@ -58,6 +58,7 @@ struct TilePass {
   bool ktyprev_zero = true;            // check only
   double* part_d = nullptr;            // check only
   double* part_p = nullptr;
+  unsigned part_cap = 0;               // check only: (a, b) pairs that fit at part_d and at part_p
   float* x_out = nullptr;
   float* y_out = nullptr;
   const RingHalo* halo = nullptr;      // slab mode
@@ -655,19 +656,21 @@ struct StencilPlan {
 // Recognises the operator structure; `blocks` are the problem's non-zero blocks.
 StencilPlan plan_stencil(const std::vector<std::shared_ptr<Block>>& blocks, size_t nrows, size_t ncols);
 
-// Each returns 0 when the (operator, prox) pair is not covered by a specialised kernel (the caller
-// then uses the generic fused kernel), otherwise the number of CTAs launched (= partial pairs written).
-// dry_run: only the grid the pass would launch; the operand pointers are read for their alignment.
-unsigned stencil_primal_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& d, const PrimalPass& p,
-                               bool dry_run = false);
-unsigned stencil_dual_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& d, const DualPass& p,
-                             bool dry_run = false);
+// Does a specialised pass cover prox `d` of the plan's operator?  0 if not (the generic fused pass runs it), otherwise
+// the largest grid any variant of that pass launches for it, i.e. the most (a, b) partial pairs it writes.  Which
+// variant runs is decided per launch, from the operands' alignment and the iteration.
+unsigned stencil_primal_cover(const StencilPlan& plan, const ProxDesc& d);
+unsigned stencil_dual_cover(const Context* ctx, const StencilPlan& plan, const ProxDesc& d);
+// Each returns 0 when the pass is not covered, otherwise the number of CTAs launched (= partial pairs written).
+unsigned stencil_primal_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& d, const PrimalPass& p);
+unsigned stencil_dual_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& d, const DualPass& p);
 
 // ---- whole iteration as one tiled pass (pb_tile.cu) ---------------------------------------------
-bool tile_iteration_supported(const StencilPlan& plan, const std::vector<ProxDesc>& gd,
-                              const std::vector<ProxDesc>& fd, ScaleRef T, ScaleRef S);
-// can the ring kernel run this plan, plain and residual-refresh launch alike (slab: the halo variants)?
-bool tile_ring_available(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf, bool slab);
+// Can the one-pass ring kernel run every iteration after the first (slab: its halo variants)?
+bool tile_ring_available(const StencilPlan& plan, const std::vector<ProxDesc>& gd, const std::vector<ProxDesc>& fd,
+                         ScaleRef T, ScaleRef S, bool slab);
+// its grid, i.e. the (a, b) partial pairs a residual-refresh launch writes to each of part_d and part_p
+unsigned tile_ring_grid(const Context* ctx, const StencilPlan& plan);
 // one iteration as one tiled pass; returns the number of (a, b) partial pairs written to each of part_d and
 // part_p (0 unless p.check); raises PB_ERR_CUDA if the ring kernel cannot be launched
 unsigned tile_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,

@@ -605,24 +605,48 @@ struct RingMaps {
   CUtensorMap mp1, mp2, mx, mf, mq1, mq2;
 };
 
-template <int FN_G, int FN_F, bool CHECK, bool SLAB>
-unsigned ring_launch_k(Context* ctx, const RingMaps& m, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf,
-                       const TilePass& p, bool dry_run) {
-  auto kernel = grad2d_iteration_ring_kernel<FN_G, FN_F, CHECK, SLAB>;
-  static bool configured = false, ok = false;
-  if (!configured) {
-    configured = true;
-    ok = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kRingSmemBytes) == cudaSuccess;
-    cudaGetLastError();
-  }
-  if (!ok) return 0;
-  const uint32_t tiles_x = (g.nx + kRingTX - 1) / kRingTX, tiles_y = (g.ny + kRingTY - 1) / kRingTY;
-  const uint64_t n_tiles = (uint64_t)tiles_x * tiles_y * g.L;
-  if (n_tiles == 0 || n_tiles >= (1ull << 31)) return 0;
-  const unsigned grid = (unsigned)std::min<uint64_t>(n_tiles, (uint64_t)ctx->num_sms);
-  if (dry_run) return grid;
+// the ring kernel's tiles: tiles_x * tiles_y owned tiles per label plane, walked by at most one CTA per SM
+struct RingTiles {
+  uint32_t x, y;
+  uint64_t n;
+  explicit RingTiles(const GradGeom& g)
+      : x((g.nx + kRingTX - 1) / kRingTX), y((g.ny + kRingTY - 1) / kRingTY), n((uint64_t)x * y * g.L) {}
+  unsigned grid(const Context* ctx) const { return (unsigned)std::min<uint64_t>(n, (uint64_t)ctx->num_sms); }
+};
+
+// (every instantiation has the same parameters)
+template <int FN_G, int FN_F>
+auto ring_kernel_fn(bool check, bool slab) {
+  return slab ? (check ? grad2d_iteration_ring_kernel<FN_G, FN_F, true, true>
+                       : grad2d_iteration_ring_kernel<FN_G, FN_F, false, true>)
+              : (check ? grad2d_iteration_ring_kernel<FN_G, FN_F, true, false>
+                       : grad2d_iteration_ring_kernel<FN_G, FN_F, false, false>);
+}
+
+auto ring_kernel(const ProxDesc& pg, const ProxDesc& pf, bool check, bool slab) {
+  const bool leq0 = pf.fn == PB_FUN_IND_LEQ0;
+  auto pick = pg.fn == PB_FUN_SQUARE ? (leq0 ? ring_kernel_fn<PB_FUN_SQUARE, PB_FUN_IND_LEQ0> : ring_kernel_fn<PB_FUN_SQUARE, -1>)
+            : pg.fn == PB_FUN_ABS    ? (leq0 ? ring_kernel_fn<PB_FUN_ABS, PB_FUN_IND_LEQ0> : ring_kernel_fn<PB_FUN_ABS, -1>)
+                                     : (leq0 ? ring_kernel_fn<-1, PB_FUN_IND_LEQ0> : ring_kernel_fn<-1, -1>);
+  return pick(check, slab);
+}
+
+// returns the number of CTAs (= residual partial pairs per residual when check), 0 if not launched
+unsigned ring_launch(Context* ctx, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf, const TilePass& p) {
+  RingMaps m;
+  if (!tensor_map_for(p.y, g.ny, g.nx, 2 * g.L, kRingRows, kRingCols + 1, m.mp1)) return 0;
+  if (!tensor_map_for(p.y, g.ny, g.nx, 2 * g.L, kRingR2, kRingCols, m.mp2)) return 0;
+  if (!tensor_map_for(p.x, g.ny, g.nx, g.L, kRingRows, kRingCols, m.mx)) return 0;
+  const float* f = pg.coeffs.ptr[1] ? pg.coeffs.ptr[1] : p.x;    // unused when b is a scalar
+  if (!tensor_map_for(f, g.ny, g.nx, g.L, kRingRows, kRingCols, m.mf)) return 0;
+  const float* q = (p.check && !p.ktyprev_zero) ? p.y_prev : p.y;  // unused otherwise
+  if (!tensor_map_for(q, g.ny, g.nx, 2 * g.L, kRingRows, kRingCols + 1, m.mq1)) return 0;
+  if (!tensor_map_for(q, g.ny, g.nx, 2 * g.L, kRingR2, kRingCols, m.mq2)) return 0;
+  const RingTiles t(g);
+  const unsigned grid = t.grid(ctx);
+  check_partials_fit(p.check, grid, p.part_cap);
   RingHalo h;
-  if (SLAB) h = *p.halo;
+  if (p.halo) h = *p.halo;
   // programmatic stream serialization: see griddepcontrol in the kernel.  Measured (profiles/r02_scaling.md): the
   // launch-to-launch gap drops from 3.8 to 1.8 us on one GPU, but on slabs the end-of-kernel flush of the
   // NVLink halo stores dominates the gap and early-resident CTAs cost more than they hide (period 54.3 vs
@@ -636,44 +660,13 @@ unsigned ring_launch_k(Context* ctx, const RingMaps& m, const GradGeom& g, const
   attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr.val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = &attr;
-  cfg.numAttrs = SLAB ? 0 : 1;
+  cfg.numAttrs = p.halo ? 0 : 1;
   const cudaError_t e = cudaLaunchKernelEx(
-      &cfg, kernel, m.mp1, m.mp2, m.mx, m.mf, m.mq1, m.mq2, g, pg, pf, p.T.val, p.S.val, p.st,
-      FastDiv((uint64_t)tiles_x * tiles_y), FastDiv(tiles_y), (uint32_t)n_tiles, p.ktyprev_zero ? 1 : 0, p.part_d,
-      p.part_p, p.x_out, p.y_out, tiles_x, h, ring_trace_next(), (CHECK && p.finish) ? *p.finish : RingFinish());
+      &cfg, ring_kernel(pg, pf, p.check, p.halo != nullptr), m.mp1, m.mp2, m.mx, m.mf, m.mq1, m.mq2, g, pg, pf,
+      p.T.val, p.S.val, p.st, FastDiv((uint64_t)t.x * t.y), FastDiv(t.y), (uint32_t)t.n, p.ktyprev_zero ? 1 : 0,
+      p.part_d, p.part_p, p.x_out, p.y_out, t.x, h, ring_trace_next(), (p.check && p.finish) ? *p.finish : RingFinish());
   if (e != cudaSuccess) { cudaGetLastError(); return 0; }
   return grid;
-}
-
-template <int FN_G, int FN_F>
-unsigned ring_launch_fn(Context* ctx, const RingMaps& m, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf,
-                        const TilePass& p, bool dry_run) {
-  auto launch = p.halo ? (p.check ? ring_launch_k<FN_G, FN_F, true, true> : ring_launch_k<FN_G, FN_F, false, true>)
-                       : (p.check ? ring_launch_k<FN_G, FN_F, true, false> : ring_launch_k<FN_G, FN_F, false, false>);
-  return launch(ctx, m, g, pg, pf, p, dry_run);
-}
-
-// returns the number of CTAs (= residual partial pairs per residual when check), 0 if not launched
-unsigned ring_launch(Context* ctx, const GradGeom& g, const ProxDesc& pg, const ProxDesc& pf, const TilePass& p,
-                     bool dry_run) {
-  RingMaps m;
-  if (!dry_run) {
-    if (!tensor_map_for(p.y, g.ny, g.nx, 2 * g.L, kRingRows, kRingCols + 1, m.mp1)) return 0;
-    if (!tensor_map_for(p.y, g.ny, g.nx, 2 * g.L, kRingR2, kRingCols, m.mp2)) return 0;
-    if (!tensor_map_for(p.x, g.ny, g.nx, g.L, kRingRows, kRingCols, m.mx)) return 0;
-    const float* f = pg.coeffs.ptr[1] ? pg.coeffs.ptr[1] : p.x;    // unused when b is a scalar
-    if (!tensor_map_for(f, g.ny, g.nx, g.L, kRingRows, kRingCols, m.mf)) return 0;
-    const float* q = (p.check && !p.ktyprev_zero) ? p.y_prev : p.y;  // unused otherwise
-    if (!tensor_map_for(q, g.ny, g.nx, 2 * g.L, kRingRows, kRingCols + 1, m.mq1)) return 0;
-    if (!tensor_map_for(q, g.ny, g.nx, 2 * g.L, kRingR2, kRingCols, m.mq2)) return 0;
-  } else if (!encode_tiled_fn()) {
-    return 0;
-  }
-  const bool leq0 = pf.fn == PB_FUN_IND_LEQ0;
-  auto launch = pg.fn == PB_FUN_SQUARE ? (leq0 ? ring_launch_fn<PB_FUN_SQUARE, PB_FUN_IND_LEQ0> : ring_launch_fn<PB_FUN_SQUARE, -1>)
-              : pg.fn == PB_FUN_ABS    ? (leq0 ? ring_launch_fn<PB_FUN_ABS, PB_FUN_IND_LEQ0> : ring_launch_fn<PB_FUN_ABS, -1>)
-                                       : (leq0 ? ring_launch_fn<-1, PB_FUN_IND_LEQ0> : ring_launch_fn<-1, -1>);
-  return launch(ctx, m, g, pg, pf, p, dry_run);
 }
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
@@ -690,11 +683,11 @@ unsigned tile_ring_trace_read(unsigned long long* h_out, unsigned n) {
   return t.next;
 }
 
-// Can the whole iteration run as one tiled pass?  K = one planar BlockGradient2D (no identity rows),
+// The whole iteration runs as one tiled pass for K = one planar BlockGradient2D (no identity rows),
 // prox_g = one Elem1D over all columns with scalar weights (b may be per pixel), prox_f* = one
 // Norm2 over the (gx, gy) pair of every voxel with scalar weights, uniform T and Sigma.
-bool tile_iteration_supported(const StencilPlan& plan, const std::vector<ProxDesc>& gd,
-                              const std::vector<ProxDesc>& fd, ScaleRef T, ScaleRef S) {
+bool tile_ring_available(const StencilPlan& plan, const std::vector<ProxDesc>& gd, const std::vector<ProxDesc>& fd,
+                         ScaleRef T, ScaleRef S, bool slab) {
   if (!plan.ok || plan.three_d) return false;
   const GradGeom& g = plan.geom;
   if (g.has_id) return false;
@@ -712,23 +705,24 @@ bool tile_iteration_supported(const StencilPlan& plan, const std::vector<ProxDes
     return false;
   for (int k = 0; k < 7; ++k)
     if (pf.coeffs.ptr[k]) return false;
-  return true;
-}
-
-bool tile_ring_available(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf, bool slab) {
-  const RingHalo halo;                 // selects the slab variants; a dry run reads nothing from it
-  TilePass p;
-  p.halo = slab ? &halo : nullptr;
+  const uint64_t n_tiles = RingTiles(g).n;
+  if (n_tiles == 0 || n_tiles >= (1ull << 31) || !encode_tiled_fn()) return false;
+  // the plain and the residual-refresh kernel, with the shared memory they launch with
   for (const bool check : {false, true}) {
-    p.check = check;
-    if (!ring_launch(ctx, plan.geom, pg, pf, p, true)) return false;
+    if (cudaFuncSetAttribute(ring_kernel(pg, pf, check, slab), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             kRingSmemBytes) != cudaSuccess) {
+      cudaGetLastError();
+      return false;
+    }
   }
   return true;
 }
 
+unsigned tile_ring_grid(const Context* ctx, const StencilPlan& plan) { return RingTiles(plan.geom).grid(ctx); }
+
 unsigned tile_iteration_launch(Context* ctx, const StencilPlan& plan, const ProxDesc& pg, const ProxDesc& pf,
                                const TilePass& p) {
-  const unsigned n = ring_launch(ctx, plan.geom, pg, pf, p, false);
+  const unsigned n = ring_launch(ctx, plan.geom, pg, pf, p);
   if (!n) fail(PB_ERR_CUDA, "the one-pass ring kernel could not be launched");
   PB_CHECK_LAUNCH();
   ctx->launches++;
