@@ -247,6 +247,7 @@ class BackendPDHG : public Backend {
   bool fused_ = false;
   bool tile_ok_ = false;               // non-check iterations run as one tiled pass (pb_tile.cu)
   unsigned long long tile_iterations_ = 0, tile_check_iterations_ = 0;
+  bool ring_went_forward_ = true;      // direction of the last ring launch (iteration 0 counts as forward)
   unsigned long long iteration_ = 0;
 
   // iterates: x_/y_ current, x_prev_/y_prev_ previous (ping-pong in fused mode)
@@ -392,6 +393,7 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
   // needs the peer-to-peer halo blocks
   if (comm_) tile_ok_ = tile_ok_ && stencil_.geom.nx >= 2;
   tile_iterations_ = 0;
+  ring_went_forward_ = true;
   if (comm_) {
     // the halo protocol lives in the specialised stencil passes: one planar gradient operator
     // (+ identity rows), one prox_g over all columns, Norm2 on the gradient rows
@@ -488,6 +490,11 @@ void BackendPDHG::iteration_fused() {
     tp.x = x_.data(); tp.y = y_.data(); tp.T = T; tp.S = S; tp.st = st; tp.x_out = x_prev_.data();
     tp.y_out = y_prev_.data();
     tp.halo = comm_ ? &ring_halo : nullptr;
+    // plain single-GPU launches alternate the walk direction, so each starts on the tiles whose operands the
+    // previous launch left in L2.  Residual-refresh launches go forward, so that each CTA sums the same pixels in
+    // the same order whatever came before; slab launches go forward because the halo protocol needs that order.
+    tp.reverse = !check && !comm_ && ring_went_forward_;
+    ring_went_forward_ = !tp.reverse;
     RingFinish fin;
     if (check) {
       // the residual-refresh launch folds the sums, combines them across ranks and advances the step-size state

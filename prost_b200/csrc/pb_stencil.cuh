@@ -63,6 +63,7 @@ struct TilePass {
   float* y_out = nullptr;
   const RingHalo* halo = nullptr;      // slab mode
   const RingFinish* finish = nullptr;  // check only: the launch finalizes the iteration itself
+  bool reverse = false;                // walk the tiles last to first (ignored in slab mode)
 };
 
 struct GradGeom {

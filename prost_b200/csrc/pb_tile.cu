@@ -5,7 +5,8 @@
 // TX x TY pixels is computed in two phases:
 //   phase A  x+ = prox_g(x - tau T K^T y) on the tile PLUS one halo column (x = cx+TX) and one
 //            halo row vector (y = cy+TY): the forward differences of the dual step need x+ there.  x+ and
-//            x of the extended tile go to shared memory; the tile's own x+ is written to HBM.
+//            x of the extended tile go to shared memory; the tile's own x+ is written to HBM.  A tile at the
+//            image bottom has no tile below it and owns its halo row vector as well.
 //   phase B  y+ = prox_f*(y + sigma S ((1+theta) K x+ - theta K x)) on the tile, with K x+ and K x
 //            taken from shared memory.
 // HBM traffic per pixel: read y (2), x, f; write x+, y+ (2) = 7 floats = 28 B instead of 44 B; the
@@ -94,7 +95,13 @@ bool tensor_map_for(const float* base, uint32_t ny, uint32_t nx, uint32_t planes
 // TMA, completion signalled on mbarriers), so HBM streams continuously while the 32 warps compute the
 // current tile.
 //   computed x+ region 32 columns x 128 rows = 1024 row vectors = exactly one per thread;
-//   owned tile         31 columns x 124 rows (the last column / 4 rows are the halo of the neighbours).
+//   owned tile         31 columns x 124 rows (the last column / 4 rows are the halo of the neighbours);
+//                      the bottom tile of a tile column owns all 128 rows: nothing below it needs them, and
+//                      the forward difference of the image's last row is 0 anyway, so at ny = 4096 the
+//                      33 tile rows cover 32 x 124 + 128 rows exactly instead of leaving a 34th with 4 rows.
+// Walk: CTA b takes tiles b, b + grid, b + 2 grid, ... (label plane, then tile column, then tile row).  Plain
+// single-GPU launches alternate between this order and its reverse, so that the first tiles a launch reads are
+// the last ones the previous launch wrote, while those are still in L2.
 // Operand boxes per tile at owned-tile origin (cy, cx); out-of-image elements are zero-filled by TMA,
 // which is exactly the K^T boundary rule for x = -1 and y = -1:
 //   p1    (cy,   cx-1)   33 columns x 128 rows   gx component of y incl. the left neighbour column
@@ -208,15 +215,17 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
     const __grid_constant__ CUtensorMap map_q1, const __grid_constant__ CUtensorMap map_q2, const GradGeom g,
     const ProxDesc pg, const ProxDesc pf, const float Tval, const float Sval,
     const PdhgState* __restrict__ st, const FastDiv div_per_plane, const FastDiv div_tiles_y,
-    const uint32_t n_tiles, const int ktyprev_zero, double* __restrict__ part_d, double* __restrict__ part_p,
-    float* __restrict__ x_out, float* __restrict__ y_out, const uint32_t tiles_x, const RingHalo h,
-    const RingTraceSlot trace, const RingFinish fin) {
+    const uint32_t n_tiles, const bool reverse, const int ktyprev_zero, double* __restrict__ part_d,
+    double* __restrict__ part_p, float* __restrict__ x_out, float* __restrict__ y_out, const uint32_t tiles_x,
+    const RingHalo h, const RingTraceSlot trace, const RingFinish fin) {
   extern __shared__ __align__(128) unsigned char smem[];
   // tile -> (label plane, tile column, tile row).  On a slab the left-edge tile column is walked first (its new x
   // column leaves at the start of the launch) and the right-edge one at the first position of the SECOND wave:
   // its tiles need the right neighbour's x column of this very iteration, which that rank's first wave produces.
+  // Slabs therefore never walk in reverse.  The producer and the consumers decode the same way.
   const uint32_t right_pos = min(tiles_x - 1u, (gridDim.x + div_tiles_y.d - 1u) / div_tiles_y.d);
   auto decode = [&](uint32_t tile, uint32_t& l, uint32_t& tx, uint32_t& ty) {
+    if (!SLAB && reverse) tile = n_tiles - 1u - tile;
     uint32_t rem;
     div_per_plane.divmod(tile, l, rem);
     div_tiles_y.divmod(rem, tx, ty);
@@ -325,6 +334,8 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
     float (*s_xn)[kRingRows] = reinterpret_cast<float (*)[kRingRows]>(smem + kRingOffXn + s * kRingXBytes);
 
     const uint32_t gx = cx + col, gy = cy + r0;
+    // this thread's rows belong to the tile (x+ store, dual step, both residual sums); see the owned tile above
+    const bool own_rows = r0 < kRingTY || cy + kRingRows >= g.ny;
     const uint32_t plane_off = l * g.nxny;
     // slab edges (warp-uniform): column 0 takes y.gx of column -1 from the left neighbour's halo; the
     // owner of column nx-1 takes x+ / x of column nx from the right neighbour's halo
@@ -403,7 +414,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
         }
       }
       VecIO<4>::st(&s_xn[col][r0], xn);
-      if (col < kRingTX && r0 < kRingTY && gy < g.ny) {
+      if (col < kRingTX && own_rows && gy < g.ny) {
         VecIO<4>::st(x_out + gy + gx * g.ny + plane_off, xn);
         if (left_edge) ll_store4(sel2(h.x_out_ll, h.x_signal_seq & 1u) + halo_ll, xn, h.x_signal_seq);   // -> left neighbour
         if (CHECK) {
@@ -455,7 +466,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
     if (col < kRingTX) mbar_wait(&col_ready[s * kRingCols + col + 1], parity);
 
     // ---- phase B: y+ at the owned point (col, r0..r0+3) ---------------------------------------------------
-    if (col < kRingTX && r0 < kRingTY && gx < g.nx && gy < g.ny) {
+    if (col < kRingTX && own_rows && gx < g.nx && gy < g.ny) {
       const uint32_t idx = gy + gx * g.ny + plane_off;
       float arg[2][4];
       float cn[4], co[4], rn[4], ro[4];
@@ -476,7 +487,9 @@ __global__ void __launch_bounds__(kRingThreads, 1) grad2d_iteration_ring_kernel(
         VecIO<4>::ld(&s_xn[col + 1][r0], rn);
         VecIO<4>::ld(&s_x[col + 1][r0], ro);
       }
-      const float dn = s_xn[col][r0 + 4], dold = s_x[col][r0 + 4];
+      // the row vector below; at r0 = 124 (bottom tile) that is row 0 of column col + 1 <= 31, inside the tile,
+      // and last_row discards it
+      const float dn = (&s_xn[col][r0])[4], dold = (&s_x[col][r0])[4];
       const bool last_col = gx == g.nx - 1 && !(SLAB && h.has_right), last_row = gy + 4 >= g.ny;
       float k1x[4], k0x[4], k1y[4], k0y[4];
 #pragma unroll
@@ -605,12 +618,15 @@ struct RingMaps {
   CUtensorMap mp1, mp2, mx, mf, mq1, mq2;
 };
 
-// the ring kernel's tiles: tiles_x * tiles_y owned tiles per label plane, walked by at most one CTA per SM
+// the ring kernel's tiles: tiles_x * tiles_y owned tiles per label plane, walked by at most one CTA per SM; the
+// bottom tile row owns kRingRows rows, the others kRingTY: tiles_y = max(1, ceil((ny - 4) / kRingTY))
 struct RingTiles {
   uint32_t x, y;
   uint64_t n;
   explicit RingTiles(const GradGeom& g)
-      : x((g.nx + kRingTX - 1) / kRingTX), y((g.ny + kRingTY - 1) / kRingTY), n((uint64_t)x * y * g.L) {}
+      : x((g.nx + kRingTX - 1) / kRingTX),
+        y(g.ny == 0 ? 0 : (std::max(g.ny, (uint32_t)kRingRows) - (kRingRows - kRingTY) + kRingTY - 1) / kRingTY),
+        n((uint64_t)x * y * g.L) {}
   unsigned grid(const Context* ctx) const { return (unsigned)std::min<uint64_t>(n, (uint64_t)ctx->num_sms); }
 };
 
@@ -663,7 +679,7 @@ unsigned ring_launch(Context* ctx, const GradGeom& g, const ProxDesc& pg, const 
   cfg.numAttrs = p.halo ? 0 : 1;
   const cudaError_t e = cudaLaunchKernelEx(
       &cfg, ring_kernel(pg, pf, p.check, p.halo != nullptr), m.mp1, m.mp2, m.mx, m.mf, m.mq1, m.mq2, g, pg, pf,
-      p.T.val, p.S.val, p.st, FastDiv((uint64_t)t.x * t.y), FastDiv(t.y), (uint32_t)t.n, p.ktyprev_zero ? 1 : 0,
+      p.T.val, p.S.val, p.st, FastDiv((uint64_t)t.x * t.y), FastDiv(t.y), (uint32_t)t.n, p.reverse, p.ktyprev_zero ? 1 : 0,
       p.part_d, p.part_p, p.x_out, p.y_out, t.x, h, ring_trace_next(), (p.check && p.finish) ? *p.finish : RingFinish());
   if (e != cudaSuccess) { cudaGetLastError(); return 0; }
   return grid;
