@@ -310,7 +310,8 @@ typedef struct pb_pdhg_options {
                                  problem has the ROF shape (pb_tile.cu); 3: like 1 without the tiled
                                  pass; 2: generic fused kernels only; 0: reference-shaped unfused
                                  kernels */
-  const float* normest_x0;    /* optional ncols-vector start for normest (parity runs) */
+  const float* normest_x0;    /* optional ncols-vector start for normest (parity runs); on a slab the rank's
+                                 slice of the global start vector (its local ncols floats) */
 } pb_pdhg_options;
 void pb_solver_default_options(pb_solver_options* o);   /* matlab/+prost/options.m:3-14 */
 void pb_pdhg_default_options(pb_pdhg_options* o);       /* matlab/+prost/+backend/pdhg.m:3-14 */
@@ -380,7 +381,12 @@ int pb_backend_device_iterates(pb_backend* b, float** d_x, float** d_y);
  * mapped neighbour memory over NVLink; NCCL send/recv staging when PB_HALO=nccl or IPC is
  * unavailable) and the four residual sums are all-reduced with NCCL at residual_iter boundaries.
  * With a communicator attached, pb_backend_initialize / iterate / residuals / current_solution and
- * pb_solver_solve are COLLECTIVE: every rank must make the same calls. */
+ * pb_solver_solve are COLLECTIVE: every rank must make the same calls.
+ * The default options work as on one GPU: on slabs, scale_steps_operator runs the power iteration on the global
+ * operator (edge columns exchanged with the neighbours, sums over the ranks; the default start vector is the
+ * single-GPU one restricted to the slab); on row shards, alpha scaling gives the preconditioners of the whole
+ * operator (pb_problem_get_scaling then returns the global T and this rank's rows of Sigma).
+ * pb_problem_normest itself is rank-local on a slab's problem. */
 #define PB_COMM_ID_BYTES 128
 /* rank 0 creates the id (an ncclUniqueId); the host distributes the 128 bytes to all ranks
  * (torch.distributed broadcast, MPI_Bcast, a file, ...) */
@@ -398,7 +404,9 @@ int pb_comm_allreduce_sum(pb_comm* c, double* h_buf, size_t n);
  * BackendPDHG: a slab of image COLUMNS (stencil halos travel peer to peer inside the kernels).
  * BackendADMM: a block of ROWS of K and of the f-side proxes (SURVEY.md 8(e)); columns and the n-side vectors are
  *   replicated, K^T r is summed over the ranks with one ncclAllReduce of n floats per adjoint apply
- *   (cgls.hpp:290-357, backend_admm.cu:198-272 on one GPU), sums over rows inside the reduction kernels. */
+ *   (cgls.hpp:290-357, backend_admm.cu:198-272 on one GPU), sums over rows inside the reduction kernels.  With alpha
+ *   scaling, pb_backend_initialize replaces the rank-local preconditioners by those of the whole operator (column
+ *   sums over all ranks' rows, the empty-row carry across the ranks). */
 int pb_backend_set_slab(pb_backend* b, pb_comm* c);
 
 /* ---- Solver loop: Solver<T>::Solve, src/solver.cu:122-209 ------------------------------- */

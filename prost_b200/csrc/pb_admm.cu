@@ -506,15 +506,16 @@ void BackendADMM::initialize(const float*, size_t, const float*, size_t) {
   global_rows_ = m;
   if (sharded()) {
     // every rank must come to the same verdict before anybody throws (the next call is collective)
-    const bool ok_local = problem_->scaling_type() != Problem::kScalingAlpha;
-    double v[3] = {ok_local ? 0.0 : 1.0, static_cast<double>(m), static_cast<double>(n)};
+    const bool alpha = problem_->scaling_type() == Problem::kScalingAlpha;
+    double v[3] = {alpha ? 1.0 : 0.0, static_cast<double>(m), static_cast<double>(n)};
     comm_->allreduce_sum_host(v, 3);
-    if (v[0] != 0.0)
-      fail(PB_ERR_UNSUPPORTED, "row-sharded ADMM: the alpha preconditioners need column sums over all ranks' rows; "
-                               "use identity or custom scaling");
+    if (v[0] != 0.0 && v[0] != comm_->world())
+      fail(PB_ERR_INVALID, "row-sharded ADMM: ranks disagree on the scaling type");
     if (v[2] != static_cast<double>(n) * comm_->world())
       fail(PB_ERR_INVALID, "row-sharded ADMM: ranks disagree on the number of columns");
     global_rows_ = static_cast<unsigned long long>(v[1]);
+    // alpha scaling: the preconditioners of the whole operator replace the rank-local ones
+    if (alpha) problem_->shard_alpha_scaling(*comm_);
     comm_->ensure_halo(4);             // maps every rank's control block (reduction slots)
     if (!comm_->reduce_p2p())
       fail(PB_ERR_UNSUPPORTED, "row-sharded ADMM needs peer-to-peer access between the GPUs (CUDA IPC)");

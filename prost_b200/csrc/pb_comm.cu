@@ -440,6 +440,28 @@ void Comm::allreduce_sum_host(double* h_buf, size_t n) {
   PB_CUDA(cudaStreamSynchronize(ctx_->stream));
 }
 
+void Comm::exchange_edge_column(const float* d_src, size_t ny, size_t nx, size_t L, bool to_left, float* d_recv) {
+  if (world_ == 1) return;
+  ctx_->bind();
+  cudaStream_t s = ctx_->stream;
+  const size_t col = ny * L;
+  const int dst = to_left ? rank_ - 1 : rank_ + 1;
+  const int src = to_left ? rank_ + 1 : rank_ - 1;
+  const bool sends = to_left ? has_left() : has_right();
+  const bool receives = to_left ? has_right() : has_left();
+  if (sends) {
+    // gather the strided column: L rows of ny floats, nx*ny floats apart
+    if (edge_send_.size() < col) edge_send_.resize(col);
+    const size_t x = to_left ? 0 : nx - 1;
+    PB_CUDA(cudaMemcpy2DAsync(edge_send_.data(), ny * sizeof(float), d_src + x * ny, nx * ny * sizeof(float),
+                              ny * sizeof(float), L, cudaMemcpyDeviceToDevice, s));
+  }
+  PB_NCCL(nccl().GroupStart());
+  if (sends) PB_NCCL(nccl().Send(edge_send_.data(), col, ncclFloat, dst, as_comm(nccl_), s));
+  if (receives) PB_NCCL(nccl().Recv(d_recv, col, ncclFloat, src, as_comm(nccl_), s));
+  PB_NCCL(nccl().GroupEnd());
+}
+
 void Comm::barrier() {
   double one[1] = {1.0};
   allreduce_sum_host(one, 1);

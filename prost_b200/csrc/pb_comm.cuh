@@ -107,6 +107,15 @@ class Comm {
   void allreduce_sum_host(double* h_buf, size_t n);
   void barrier();
 
+  // collective, for code outside the PDHG passes (the power iteration of the step-size rescaling): one edge
+  // column of the planar array d_src (ny x nx x L, idx = y + x*ny + l*nx*ny) moves to a neighbour with grouped
+  // ncclSend / ncclRecv on the context stream.  to_left: every rank sends its column 0 to the left neighbour and
+  // receives the right neighbour's column 0; otherwise it sends column nx-1 to the right and receives the left
+  // neighbour's column nx-1.  d_recv gets ny*L floats laid out y + l*ny (SlabHalo::in_a) and is left untouched on
+  // a rank without that neighbour.  Independent of the halo blocks: no sequence number, flag or slot changes, and
+  // ensure_halo() need not have run.  All ranks must pass the same ny * L.
+  void exchange_edge_column(const float* d_src, size_t ny, size_t nx, size_t L, bool to_left, float* d_recv);
+
   // --- halo descriptors of the PDHG passes on a slab (pb_pdhg.cu).  All ranks run the same passes, so the pass
   // sequence numbers behind them are identical on every rank.  A two-pass iteration calls primal_halo() before its
   // primal pass, dual_halo() between the passes and end_two_pass_iteration() after the dual pass; a one-pass
@@ -168,6 +177,7 @@ class Comm {
   void* right_block_ = nullptr;
   std::vector<void*> peer_blocks_;     // every rank's block (own: block_), p2p only
   DeviceBuffer<float> stage_x_, stage_y_;   // staging mode
+  DeviceBuffer<float> edge_send_;           // exchange_edge_column: the packed outgoing column
   DeviceBuffer<double> scratch_;
 };
 

@@ -10,6 +10,7 @@
 //               problems) and as an A/B check of the fused passes.
 #include <algorithm>
 #include <cmath>
+#include <cstdlib>
 #include <iostream>
 
 #include "pb_backend.cuh"
@@ -227,6 +228,7 @@ class BackendPDHG : public Backend {
   DeviceBuffer<unsigned> fin_ticket_;        // RingFinish: CTAs of the running residual-refresh launch that are done
   RingFinish ring_finish();
   void slab_apply(float* d_res, const float* d_rhs, const float* d_halo, bool adjoint);
+  float slab_normest();
   Comm* comm_ = nullptr;
   bool is_check_iteration() const {
     // size_t % int of the reference: a negative residual_iter wraps to a huge modulus, i.e.
@@ -356,20 +358,6 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
     prox_fstar_ = problem_->prox_fstar();
   }
 
-  if (opts_.scale_steps_operator && comm_)
-    fail(PB_ERR_UNSUPPORTED, "slab decomposition: scale_steps_operator (normest) is not distributed; "
-                             "set scale_steps_operator = false");
-  if (opts_.scale_steps_operator) {                      // :274-286
-    const float norm = problem_->normest(1e-6f, 100, opts_.normest_x0);
-    if (std::abs(norm - 1) > 0.1) {
-      st.tau /= norm;
-      st.sigma /= norm;
-      if (sopts_.verbose)
-        std::cout << "|K|=" << norm << " => Rescaled tau=" << st.tau << ", sigma=" << st.sigma << "."
-                  << std::endl;
-    }
-  }
-
   // Slabs: a rank-local failure must not leave the peers blocked in the next collective, so every rank-local
   // verdict between two collectives is voted on (sum of failure flags) before any rank throws.
   auto vote = [&](bool ok_local, int status, const std::string& msg) {
@@ -417,6 +405,18 @@ void BackendPDHG::initialize(const float* h_x0, size_t nx0, const float* h_y0, s
     double no_tile[1] = {(tile_ok_ && (comm_->p2p() || comm_->world() == 1)) ? 0.0 : 1.0};
     comm_->allreduce_sum_host(no_tile, 1);
     tile_ok_ = no_tile[0] == 0.0;
+  }
+  // step sizes over the operator norm (:274-286); on slabs after the verdict above, so that every rank has planned
+  // its stencil and agreed that the problem shards
+  if (opts_.scale_steps_operator) {
+    const float norm = comm_ ? slab_normest() : problem_->normest(1e-6f, 100, opts_.normest_x0);
+    if (std::abs(norm - 1) > 0.1) {
+      st.tau /= norm;
+      st.sigma /= norm;
+      if (sopts_.verbose && (!comm_ || comm_->rank() == 0))
+        std::cout << "|K|=" << norm << " => Rescaled tau=" << st.tau << ", sigma=" << st.sigma << "."
+                  << std::endl;
+    }
   }
   {
     PB_TRACE_SCOPE("  allocate iterates");
@@ -600,7 +600,59 @@ RingFinish BackendPDHG::ring_finish() {
   return f;
 }
 
-// K u / K^T p on the local slab including the neighbours' columns (current_solution only)
+// Power iteration of Problem::normest on the global operator, each rank holding its slab of the vectors: K and K^T
+// through slab_apply with the neighbours' edge columns, the sums of squares added over the ranks.  The start
+// vector is the single-GPU one restricted to the slab: the std::rand() sequence over all global columns, of
+// which each rank keeps its own entries (or the rank's slice of normest_x0).
+float BackendPDHG::slab_normest() {
+  PB_TRACE_SCOPE("  slab normest");
+  const GradGeom& g = stencil_.geom;
+  const size_t nx = g.nx, ny = g.ny, L = g.L;
+  const size_t m = problem_->nrows(), n = problem_->ncols();
+  const int world = comm_->world(), rank = comm_->rank();
+  // the ranks' widths in rank order, and ny, L with their squares (all ranks agree iff the variance is zero)
+  std::vector<double> v(world + 4, 0.0);
+  v[rank] = static_cast<double>(nx);
+  v[world] = static_cast<double>(ny);
+  v[world + 1] = static_cast<double>(ny) * ny;
+  v[world + 2] = static_cast<double>(L);
+  v[world + 3] = static_cast<double>(L) * L;
+  comm_->allreduce_sum_host(v.data(), v.size());
+  if (v[world + 1] * world != v[world] * v[world] || v[world + 3] * world != v[world + 2] * v[world + 2])
+    fail(PB_ERR_INVALID, "slab decomposition: ranks disagree on ny or L of the gradient operator");
+  size_t x_begin = 0, nx_global = 0;
+  for (int r = 0; r < world; ++r) {
+    if (r < rank) x_begin += static_cast<size_t>(v[r]);
+    nx_global += static_cast<size_t>(v[r]);
+  }
+  std::vector<float> x0;
+  if (!opts_.normest_x0) {
+    x0.resize(n);
+    std::srand(0);                     // as Problem::normest: global index y + x*ny + l*nx*ny in sequence order
+    for (size_t l = 0; l < L; ++l)
+      for (size_t x = 0; x < nx_global; ++x)
+        for (size_t y = 0; y < ny; ++y) {
+          const float r = (float)std::rand() / (float)RAND_MAX;
+          if (x >= x_begin && x < x_begin + nx) x0[y + (x - x_begin) * ny + l * nx * ny] = r;
+        }
+  }
+  // rows of K that slab_apply writes; any beyond see K = 0 as in Problem::apply_K
+  const size_t covered = g.has_id ? (size_t)g.id_row + g.plane : (stencil_.three_d ? 3 : 2) * (size_t)g.plane;
+  DeviceBuffer<float> halo(ny * L);
+  halo.zero(ctx_->stream);
+  NormestOps ops;
+  ops.apply = [&](float* res, const float* rhs, bool adjoint) {
+    // K u needs the right neighbour's column 0 of u, K^T p the left neighbour's last column of p's x-component
+    comm_->exchange_edge_column(rhs, ny, nx, L, /*to_left=*/!adjoint, halo.data());
+    slab_apply(res, rhs, halo.data(), adjoint);
+    if (!adjoint && m > covered)
+      PB_CUDA(cudaMemsetAsync(res + covered, 0, (m - covered) * sizeof(float), ctx_->stream));
+  };
+  ops.sum = [&](double* h, size_t k) { comm_->allreduce_sum_host(h, k); };
+  return problem_->normest(1e-6f, 100, opts_.normest_x0 ? opts_.normest_x0 : x0.data(), ops);
+}
+
+// K u / K^T p on the local slab including the neighbours' columns (current_solution, slab_normest)
 void BackendPDHG::slab_apply(float* d_res, const float* d_rhs, const float* d_halo, bool adjoint) {
   GradGeom g = stencil_.geom;
   g.q = g.ny;

@@ -5,12 +5,11 @@
 #include "pb_problem.cuh"
 
 #include <algorithm>
-
-#include <algorithm>
 #include <cmath>
 #include <cstdlib>
 #include <iostream>
 
+#include "pb_comm.cuh"
 #include "pb_reduce.cuh"
 
 namespace pb {
@@ -378,6 +377,56 @@ void Problem::initialize() {
   initialized_ = true;
 }
 
+// The element-wise alpha scaling of initialize() for the whole row-sharded operator.  Row sums are complete on
+// the rank that owns the row; column sums are this rank's partial sums, added over the ranks in double and
+// rounded once.  The carry of the reference (one variable through all rows, then all columns) crosses the ranks:
+// rank r's first empty rows take the value of the last non-empty row of ranks < r, and column 0's carry is the
+// value of the globally last non-empty row (1 where there is none).
+void Problem::shard_alpha_scaling(Comm& comm) {
+  ctx_->bind();
+  PB_TRACE_SCOPE("Problem::shard_alpha_scaling");
+  const int world = comm.world(), rank = comm.rank();
+  std::vector<float> rs, cs;
+  linop_->row_sums(scaling_alpha_, rs);
+  linop_->col_sums(static_cast<float>(2. - scaling_alpha_), cs);
+  auto row_sum = [&](size_t r) { return r < rs.size() ? rs[r] : 0.f; };
+
+  // (has a non-empty row, value of the last one) of every rank, in rank order
+  std::vector<double> last(2 * (size_t)world + ncols_, 0.0);
+  for (size_t r = nrows_; r-- > 0;) {
+    const float s = row_sum(r);
+    if (s > 0) {
+      last[2 * rank] = 1.0;
+      last[2 * rank + 1] = static_cast<float>(1. / s);
+      break;
+    }
+  }
+  double* col = last.data() + 2 * world;
+  for (size_t c = 0; c < cs.size() && c < ncols_; ++c) col[c] = cs[c];
+  comm.allreduce_sum_host(last.data(), last.size());
+
+  float value = 1;
+  for (int k = 0; k < rank; ++k)
+    if (last[2 * k] != 0.0) value = static_cast<float>(last[2 * k + 1]);
+  std::vector<float> left_host(nrows_), right_host(ncols_);
+  for (size_t r = 0; r < nrows_; ++r) {
+    const float s = row_sum(r);
+    if (s > 0) value = static_cast<float>(1. / s);
+    left_host[r] = value;
+  }
+  for (int k = rank + 1; k < world; ++k)
+    if (last[2 * k] != 0.0) value = static_cast<float>(last[2 * k + 1]);
+  for (size_t c = 0; c < ncols_; ++c) {
+    const float s = static_cast<float>(col[c]);
+    if (s > 0) value = static_cast<float>(1. / s);
+    right_host[c] = value;
+  }
+  average_preconditioners(right_host, prox_g_.empty() ? prox_gstar_ : prox_g_);
+  average_preconditioners(left_host, prox_f_.empty() ? prox_fstar_ : prox_f_);
+  left_.set_host(std::move(left_host));
+  right_.set_host(std::move(right_host));
+}
+
 // AveragePreconditioners (problem.cu:502-536): float running sum in group order, then divide.
 void Problem::average_preconditioners(std::vector<float>& precond, const ProxList& prox) {
   std::vector<std::tuple<size_t, size_t, size_t>> groups;
@@ -442,8 +491,10 @@ size_t Problem::gpu_mem_amount() const {
   return mem;
 }
 
-// Power iteration on Sigma^1/2 K T^1/2 (problem.cu:428-500).
-float Problem::normest(float tol, int max_iters, const float* h_x0) {
+// Power iteration on Sigma^1/2 K T^1/2 (problem.cu:428-500).  `ops` supplies K / K^T and the sum over ranks of
+// the two sums of squares of every step (slabs, pb_pdhg.cu); by default the problem's own operator on one GPU.
+// The norms are taken from the summed doubles, so every rank sees the same values and stops at the same step.
+float Problem::normest(float tol, int max_iters, const float* h_x0, const NormestOps& ops) {
   ctx_->bind();
   const size_t n = ncols_, m = nrows_;
   DeviceBuffer<float> x(n), Ax(m), x_temp(n), Ax_temp(m);
@@ -457,20 +508,28 @@ float Problem::normest(float tol, int max_iters, const float* h_x0) {
   }
   x.upload(x_host.data(), n, ctx_->stream);
   auto sgrid = [&](size_t k) { return (unsigned)std::min<size_t>(grid_for(k), (size_t)ctx_->num_sms * 32); };
+  auto apply = [&](float* res, const float* rhs, bool adjoint) {
+    if (ops.apply) ops.apply(res, rhs, adjoint);
+    else apply_K(res, rhs, adjoint);
+  };
 
   float norm = 0, norm_prev;
   for (int i = 0; i < max_iters; ++i) {
     norm_prev = norm;
+    double sq[2];
     mul_sqrt_kernel<<<sgrid(n), kBlock, 0, ctx_->stream>>>(x_temp.data(), scaling_right(), x.data(), n);
-    apply_K(Ax_temp.data(), x_temp.data(), false);
+    apply(Ax_temp.data(), x_temp.data(), false);
     mul_sqrt_kernel<<<sgrid(m), kBlock, 0, ctx_->stream>>>(Ax.data(), scaling_left(), Ax_temp.data(), m);
-    const float norm_Ax = std::sqrt(static_cast<float>(device_sumsq(ctx_, Ax.data(), m, scratch)));
+    sq[0] = device_sumsq(ctx_, Ax.data(), m, scratch);
     mul_sqrt_kernel<<<sgrid(m), kBlock, 0, ctx_->stream>>>(Ax_temp.data(), scaling_left(), Ax.data(), m);
-    apply_K(x_temp.data(), Ax_temp.data(), true);
+    apply(x_temp.data(), Ax_temp.data(), true);
     mul_sqrt_kernel<<<sgrid(n), kBlock, 0, ctx_->stream>>>(x.data(), scaling_right(), x_temp.data(), n);
     PB_CHECK_LAUNCH();
     ctx_->launches += 4;
-    const float norm_x = std::sqrt(static_cast<float>(device_sumsq(ctx_, x.data(), n, scratch)));
+    sq[1] = device_sumsq(ctx_, x.data(), n, scratch);
+    if (ops.sum) ops.sum(sq, 2);
+    const float norm_Ax = std::sqrt(static_cast<float>(sq[0]));
+    const float norm_x = std::sqrt(static_cast<float>(sq[1]));
     norm = norm_x / norm_Ax;
     if (std::abs(norm_prev - norm) < tol * norm) break;
     divide_kernel<<<sgrid(n), kBlock, 0, ctx_->stream>>>(x.data(), n, norm_x);

@@ -2,6 +2,7 @@
 // src/problem.cu.
 #pragma once
 
+#include <functional>
 #include <memory>
 #include <string>
 #include <vector>
@@ -45,6 +46,15 @@ class ScaleVec {
   mutable bool dev_valid_ = false;
 };
 
+class Comm;
+
+// K / K^T and the sum over ranks of the power iteration (Problem::normest); empty members: the problem's own
+// operator (apply_K) on one GPU
+struct NormestOps {
+  std::function<void(float* d_res, const float* d_rhs, bool adjoint)> apply;
+  std::function<void(double* h_buf, size_t n)> sum;
+};
+
 class Problem {
  public:
   enum Scaling { kScalingIdentity, kScalingAlpha, kScalingCustom };
@@ -63,8 +73,13 @@ class Problem {
   void set_scaling_custom(const float* left, size_t nl, const float* right, size_t nr);
 
   void initialize();
+  // Row shards (BackendADMM): after initialize() on this rank's rows, replace the alpha preconditioners by those
+  // of the whole operator -- T from the column sums over all ranks' rows, and Sigma and T with the empty-row /
+  // empty-column carry running across the ranks in rank order.  Collective.
+  void shard_alpha_scaling(Comm& comm);
   void dualize();
-  float normest(float tol, int max_iters, const float* h_x0);
+  // on a slab (rank-local problem) only with `ops` that apply the global operator; h_x0: ncols floats or NULL
+  float normest(float tol, int max_iters, const float* h_x0, const NormestOps& ops = NormestOps());
 
   size_t nrows() const { return nrows_; }
   size_t ncols() const { return ncols_; }

@@ -152,8 +152,8 @@ def shard_rows(desc, part, rank):
 
     Blocks are cut at the rank's row range (sparse / dense / zero blocks: a row slice of the matrix; diagonal
     identity-pattern blocks become sparse slices).  f-side proxes must be element-wise (1d family, dim 1): their
-    index range and per-element coefficients are sliced.  Scaling: identity, or custom with the left vector sliced
-    (the alpha preconditioners need column sums over all ranks' rows and are rejected by the backend)."""
+    index range and per-element coefficients are sliced.  Scaling: alpha (kept; the backend's Initialize computes the
+    preconditioners of the whole operator from all ranks' rows), identity, or custom with the left vector sliced."""
     import scipy.sparse as sp
     if part.nrows != int(desc["nrows"]):
         raise ValueError("partition and description disagree on nrows")
