@@ -73,9 +73,13 @@ def norm2_ball(P):
     return np.where(nrm > 1, P / np.maximum(nrm, 1e-300), P)
 
 
-def prox_1d_closed(fun, x0, tau):
-    """Closed-form prox_{tau f} for the simple Function1D members (function_1d.hpp)."""
+def prox_1d_closed(fun, x0, tau, alpha=0.0):
+    """Closed-form prox_{tau f} for the simple Function1D members (function_1d.hpp); alpha is the
+    Huber threshold."""
     x0 = np.asarray(x0, dtype=np.float64)
+    if fun == "huber":
+        r = (x0 / tau) / (1 + alpha / tau)
+        return x0 - tau * r / np.maximum(1.0, np.abs(r))
     if fun == "zero":
         return x0
     if fun == "abs":
@@ -97,13 +101,13 @@ def prox_1d_closed(fun, x0, tau):
     raise ValueError(fun)
 
 
-def prox_general_1d(fun, arg, tau, a, b, c, d, e):
+def prox_general_1d(fun, arg, tau, a, b, c, d, e, alpha=0.0):
     """prox of h(x) = c f(ax - b) + dx + (e/2)x^2 through the shift/scale rules
     (elem_operation_1d.hpp:36-59), in float64."""
     arg = np.asarray(arg, dtype=np.float64)
     p = (a * (arg - d * tau)) / (1 + tau * e) - b
     s = (c * a * a * tau) / (1 + tau * e)
-    return (prox_1d_closed(fun, p, s) + b) / a
+    return (prox_1d_closed(fun, p, s, alpha) + b) / a
 
 
 def brute_force_epi_quad(x0, y0, a, iters=200):

@@ -78,7 +78,7 @@ def test_prox_simplex(d, interleaved):
 
 
 @pytest.mark.parametrize("fun", ["zero", "abs", "square", "ind_leq0", "ind_geq0", "ind_eq0", "ind_box01",
-                                 "max_pos0", "l0"])
+                                 "max_pos0", "l0", "huber"])
 def test_prox_1d_general_form(fun):
     """test_prox_transform.m / conj_trans: h(x) = c f(ax - b) + dx + (e/2)x^2 with random a..e, tau, Tau."""
     N = 4000
@@ -88,10 +88,12 @@ def test_prox_1d_general_form(fun):
     arg = (3 * r.standard_normal(N)).astype(np.float32)
     Tau = r.uniform(0.5, 1.5, N).astype(np.float32)
     tau = 0.7
-    desc = ("elem_operation:1d:" + fun, 0, N, True, [N, 1, False, cases.coeffs(a, b, c, d, e)])
+    alpha = 0.3                                   # the Huber threshold; the other members ignore it
+    desc = ("elem_operation:1d:" + fun, 0, N, True, [N, 1, False, cases.coeffs(a, b, c, d, e, alpha)])
     res = oracle_prox_eval(desc, arg, Tau, tau)
     f32 = lambda v: np.asarray(v, dtype=np.float32).astype(np.float64)
-    want = refmath.prox_general_1d(fun, arg, tau * Tau.astype(np.float64), f32(a), f32(b), f32(c), f32(d), f32(e))
+    want = refmath.prox_general_1d(fun, arg, tau * Tau.astype(np.float64), f32(a), f32(b), f32(c), f32(d), f32(e),
+                                   f32(alpha))
     if fun == "l0":     # hard threshold: ignore points within rounding of the jump
         p = (f32(a) * (arg - f32(d) * tau * Tau)) / (1 + tau * Tau * f32(e)) - f32(b)
         s = (f32(c) * f32(a) ** 2 * tau * Tau) / (1 + tau * Tau * f32(e))
