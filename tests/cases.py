@@ -88,6 +88,10 @@ def linop_matrix(blocks):
             K = sp.csr_matrix(data[0]).astype(np.float64)
         elif name == "zero":
             K = sp.csr_matrix((data[0], data[1]))
+        elif name in ("dense_kron_id", "id_kron_dense", "sparse_kron_id", "id_kron_sparse"):
+            F = sp.csr_matrix(data[0]).astype(np.float64)
+            I = sp.identity(int(data[1]), dtype=np.float64, format="csr")
+            K = sp.kron(I, F) if name.startswith("id_") else sp.kron(F, I)
         mats.append((row, col, K.tocoo()))
         m, n = max(m, row + K.shape[0]), max(n, col + K.shape[1])
     rows = np.concatenate([k.row + r for r, c, k in mats])

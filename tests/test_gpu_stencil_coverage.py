@@ -25,6 +25,7 @@ import numpy as np
 import pytest
 
 from prost_b200 import synthetic as syn
+from launch_log import _template_args, launch_log
 from pdhg_f64 import run_f64
 from pdhg_util import assert_parity, rel_err, run_oracle
 
@@ -408,46 +409,6 @@ def test_f64_reference_matches_oracle(name):
 # ---- launch log ----------------------------------------------------------------------------------------------
 KERNELS = ("grad_primal_kernel", "grad_primal_simplex_staged_kernel", "grad_dual_norm2_kernel",
            "grad_dual_norm2_staged_kernel", "prox_pass_kernel", "prox_pass_pairs4_kernel")
-
-
-def _template_args(name, kernel):
-    """top-level template arguments of `kernel<...>` in a demangled name, whitespace and namespaces removed"""
-    m = re.search(r"\b" + kernel + "<", name)
-    if not m:
-        return None
-    i, depth, cur, args = m.end(), 1, "", []
-    while depth:
-        ch = name[i]
-        i += 1
-        if ch == "<":
-            depth += 1
-        elif ch == ">":
-            depth -= 1
-            if depth == 0:
-                break
-        if ch == "," and depth == 1:
-            args.append(cur)
-            cur = ""
-        else:
-            cur += ch
-    args.append(cur)
-    norm = []
-    for a in args:
-        a = re.sub(r"\s+|pb::|\(int\)", "", a)
-        norm.append({"(bool)1": "true", "(bool)0": "false"}.get(a, a))
-    return tuple(norm)
-
-
-def launch_log(run):
-    """Demangled names of every CUDA kernel `run()` launches, and run()'s result."""
-    import torch
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        out = run()
-        torch.cuda.synchronize()
-    names = {e.name for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA}
-    return names, out
 
 
 def instantiations(names):
